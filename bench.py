@@ -42,7 +42,7 @@ PREHEAT = 64  # untimed launches before every timed region, whatever --warmup sa
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=2000, help="timed steps of the headline workload (a fused run's last launch takes the remainder)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--envs", type=int, default=65536, help="envs per GPU")
@@ -60,7 +60,13 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-legs", action="store_true")
     ap.add_argument("--seed", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed headline step returned as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 def workload_name(a):
@@ -210,6 +216,25 @@ def latest_profile(pattern):
     return files[-1] if files else None
 
 
+DUMP_BYTES = 60 << 20  # --dump-outputs stays below 64 MB, .npy headers included
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every [B, ...] device tensor of `arrays` as out_dir/<name>.npy in float32.  Above DUMP_BYTES in all, the
+    same fixed, seeded sample of envs is taken from every array and its env indices go to env_index.npy (float64)."""
+    import numpy as np
+    arrays = {k: v.float().cpu().numpy() for k, v in arrays.items()}
+    B = len(next(iter(arrays.values())))
+    per_env = sum(v[0].nbytes for v in arrays.values())
+    if B * per_env > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // (per_env + 8), replace=False))
+        arrays = {k: v[idx] for k, v in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def main():
     a = parse()
     if a.impl == "reference":
@@ -302,9 +327,10 @@ def main():
         torch.cuda.synchronize()
         return ring
 
-    def plain_legs(net, sets, ring, n_steps, fuse, obs=0, flushed=False):
+    def plain_legs(net, sets, ring, n_steps, fuse, obs=0, flushed=False, keep_last=False):
         """Fused (`fuse` plain steps per launch) and one-launch-per-step timings of alternating defender / attacker turns
-        over the rotating env sets.  Returns dict(ms_fused, steps_fused, launches, ms_single, steps_single)."""
+        over the rotating env sets, n_steps steps each.  Returns dict(ms_fused, steps_fused, launches, ms_single, steps_single);
+        keep_last adds `last`: copies of what the last step of the first timed region (fused if fuse > 1) returned."""
         nB, n_sets, n_ring = sets[0].B, len(sets), len(ring[0])
 
         def one_step(i):
@@ -316,7 +342,9 @@ def main():
         out = {}
         F = max(1, fuse) if not obs else 1
         if F > 1:
-            Kf = ((n_steps + F - 1) // F) * F
+            n_launch = (n_steps + F - 1) // F  # the last launch of a timed region fuses the remaining n_steps - (n_launch - 1) * F
+            w_f = (Wm + F - 1) // F
+            p0 = max(w_f, PREHEAT)  # index of the first timed launch: timed() and timed_flushed() pre-heat with launches 0 .. p0 - 1
             fused = []
             for s_i in range(n_sets):
                 per_set = []
@@ -329,17 +357,26 @@ def main():
                      torch.empty(F, nB, dtype=torch.int32, device=dev)) for _ in range(n_sets)]
             torch.cuda.synchronize()
 
-            def one_launch(j):
+            def one_launch(j, T=F):
                 s_i = j % n_sets
                 h_, m_ = fused[s_i][(j // n_sets) & 1]
-                sets[s_i].step_many(h_, m_, out=outs[s_i])
+                o_ = outs[s_i]
+                if T < F:
+                    h_, m_, o_ = h_[:T], m_[:T], tuple(x[:T] for x in o_)
+                sets[s_i].step_many(h_, m_, out=o_)
+
+            def timed_launch(j):
+                one_launch(j, min(F, n_steps - (j - p0) * F))
 
             if flushed:
-                out["ms_fused"], out["launches"] = timed_flushed(one_launch, Kf // F, (Wm + F - 1) // F), Kf // F
+                out["ms_fused"], out["launches"] = timed_flushed(timed_launch, n_launch, w_f), n_launch
             else:
-                out["ms_fused"], out["launches"] = timed(one_launch, Kf // F, (Wm + F - 1) // F, sets)
-            out["steps_fused"] = Kf
-        K1 = min(n_steps, 600)
+                out["ms_fused"], out["launches"] = timed(timed_launch, n_launch, w_f, sets)
+            out["steps_fused"] = n_steps
+            if keep_last:
+                T_last = n_steps - (n_launch - 1) * F
+                out["last"] = [x[T_last - 1].clone() for x in outs[(p0 + n_launch - 1) % n_sets]]
+        K1 = n_steps
         if flushed:
             out["ms_single"] = timed_flushed(one_step, K1, Wm)
         else:
@@ -347,6 +384,12 @@ def main():
             if F == 1:
                 out["launches"] = l1
         out["steps_single"] = K1
+        if keep_last and F == 1:
+            i = max(Wm, PREHEAT) + K1 - 1  # the last timed step (see one_step)
+            env = sets[i % n_sets]
+            out["last"] = [x.clone() for x in (env.raw, env.shaped, env.done)]
+            if obs:
+                out["last"].append(env.last_obs(1 + ((i // n_sets) & 1)).clone())
         if not flushed and not obs and n_sets > 1:
             # the same one-launch-per-step workload with every env set on its OWN stream (each set still steps in order:
             # closed loop per set): a launch's CTAs move onto SMs as the previous launch's CTAs leave them, so the
@@ -375,19 +418,19 @@ def main():
             barrier()
             out["ms_single_streams"] = e0.elapsed_time(e1)
             if F > 1:  # and the fused launches the same way (each set's launches in order on its own stream)
-                def run_f(n):
+                def run_f(n, total=None):  # n launches; with `total`, exactly `total` steps
                     for j in range(n):
                         s_i = j % n_sets
                         if j < n_sets:
                             streams[s_i].wait_stream(cur)
                         with torch.cuda.stream(streams[s_i]):
-                            one_launch(j)
+                            one_launch(j, F if total is None else min(F, total - j * F))
                     for st_ in streams:
                         cur.wait_stream(st_)
-                run_f(max((Wm + F - 1) // F, PREHEAT))
+                run_f(p0)
                 barrier()
                 e0.record()
-                run_f(Kf // F)
+                run_f(n_launch, n_steps)
                 e1.record()
                 barrier()
                 out["ms_fused_streams"] = e0.elapsed_time(e1)
@@ -426,8 +469,10 @@ def main():
     F = max(1, a.fuse) if not a.obs else 1
     sampler = ClockSampler(local)
     sampler.start()
-    head = plain_legs(net, sets, ring, K, F, obs=a.obs)
+    head = plain_legs(net, sets, ring, K, F, obs=a.obs, keep_last=bool(a.dump_outputs))
     clocks = sampler.stop()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, dict(zip(("raw_reward", "shaped_reward", "done", "obs"), head.pop("last"))))
     if F > 1:
         ms, Kh, launches = head["ms_fused"], head["steps_fused"], head["launches"]
     else:
@@ -674,7 +719,7 @@ def main():
             return None, None
         traffic, traffic_src = traffic_of("step_kernel_traffic.json", envs_per_launch=B, device_slots=a.devices)
         traffic_f, traffic_f_src = traffic_of("step_kernel_fused_traffic.json", envs_per_launch=B, device_slots=a.devices, steps_per_launch=F)
-        launch_s = ms * 1e-3 / (Kh // F)      # average duration of one launch (F steps)
+        launch_s = ms * 1e-3 * F / Kh         # average duration of F steps (one launch)
         achieved = alg * B * F / launch_s / 1e9
         value = world * B * Kh / (ms * 1e-3)
         line = {

@@ -79,6 +79,80 @@ class CudaImpl:
         return o.cpu().numpy()[0]
 
 
+def gym_action(hdr, mask, order, M, order_form):
+    """A recorded action row (include/cygym_b200.h packing) as the reference's (type, exploits, devices, app) tuple."""
+    at = int(np.int8(hdr[0] & 0xFF))
+    if (int(hdr[0]) & 0xFF) == 0x80:
+        return None
+    n_ex = (int(hdr[0]) >> 16) & 0xFF
+    ex = [int(np.int8((int(hdr[1]) >> (8 * i)) & 0xFF)) for i in range(n_ex)]
+    n = int(hdr[2]) & 0xFFFF
+    devs = [int(x) for x in order[:n]] if order_form else [d for d in range(M) if (int(mask[d >> 5]) >> (d & 31)) & 1]
+    return (at, ex, devs, int(np.int32(hdr[3])))
+
+
+def replay_golden_on_gym(env, g):
+    """Feed golden trajectory `g` (recorded from the reference) to the drop-in Volt_Typhoon_CyberDefenseEnv `env` as the
+    reference's action tuples, and compare after every op: the 6-tuple, observations, counters, the canonical state and,
+    where the recording keeps it, the hop log.  Where the reference trained its detector, numpy's stream was seeded
+    with `train_seed`; the drop-in gets the same seed and must fit (and later consult) the detector on its own."""
+    from oracle import trajectory as TR
+    meta = json.loads(str(g["meta"]))
+    M = meta["M"]
+    for t in range(len(g["kind"])):
+        kind = int(g["kind"][t])
+        if kind == TR.OP_RANDOMIZE:
+            env.randomize_compromise_and_ownership()
+        elif kind == TR.OP_BASELINE:
+            env.base_line = TR.BASELINES[int(g["baseline"][t])]
+        else:
+            G = int(g["n_groups"][t])
+            env.mode = "attacker" if int(g["mode"][t]) else "defender"
+            acts = [gym_action(g["hdr"][t][k], g["mask"][t][k], g["order"][t][k], M, meta["order_form"]) for k in range(G)]
+            # the reference drew every non-None action with sample_action(): one draw epoch each
+            env._venv.scalars[:, 1] += sum(1 for a in acts if a is not None)
+            env._host = None
+            seed = int(g["train_seed"][t]) if "train_seed" in g else -1
+            env.detector_fit_seed = seed if seed >= 0 else None
+            out = env.step(acts if kind == TR.OP_GROUPED else acts[0])
+            assert len(out) == 6
+            state, raw, shaped, done, info, logs = out
+            tol = 1e-5 * max(1.0, abs(float(g["raw"][t])))
+            assert abs(raw - float(g["raw"][t])) <= tol and abs(shaped - float(g["shaped"][t])) <= tol, f"op {t}"
+            assert done == bool(g["done"][t])
+            assert state.shape == (6 * M,) and state.dtype == np.float64
+            s6 = state.reshape(M, 6)
+            for row, col in enumerate((2, 4, 5)):
+                exp = np.array([(int(g["pre"][t][row, d >> 5]) >> (d & 31)) & 1 for d in range(M)], np.float64)
+                assert np.array_equal(s6[:, col], exp), f"op {t}: returned state column {col}"
+            assert np.array_equal(env._get_defender_state().astype(np.float32), g["obs_def"][t]), f"op {t}"
+            a_obs = env._get_attacker_state()
+            assert a_obs.dtype == np.float32 and a_obs.shape == (4 * M + 6,) and np.array_equal(a_obs, g["obs_att"][t])
+            sc = g["scal"][t]
+            assert env.step_num == int(sc[0]) and env.work_done == int(sc[8]) and env.scan_cnt == int(sc[11])
+            assert env.compromised_devices_cnt == int(sc[7]) and env.edges_blocked == int(sc[14])
+            assert info["Compromised_devices"] == int(sc[7]) and info["mode"] == env.mode
+            # info is built before step_num moves in step(), after it in step_grouped() (volt:1272-1285 / :746-755)
+            assert info["step_count"] == (int(sc[0]) if kind == TR.OP_GROUPED else int(sc[0]) - 1), f"op {t}"
+            assert len(logs) == int(sc[6])
+            nya = np.array([(int(g["dev"][t][d]) >> 2) & 1 for d in range(M)])
+            assert [int(d.Not_yet_added) for d in env._get_ordered_devices()] == nya.tolist()
+        st = env._snap()
+        for k in ("dev", "ckpt", "blocked"):
+            assert np.array_equal(st[k], g[k][t]), f"op {t}: {k}"
+        a, r = np.array(st["scal"], np.uint32), np.array(g["scal"][t], np.uint32)
+        assert np.allclose(a[9:11].view(np.float32), r[9:11].view(np.float32), rtol=1e-5, atol=1e-6), f"op {t}: cost counters"
+        a[9:11] = r[9:11] = 0
+        assert np.array_equal(a, r), f"op {t}: scalars {a} != {r}"  # includes the detector's trained / pending flags
+        nx = int(g["n_extra"][t])
+        assert sorted(int(x) & 0x1FFFFFF for x in st["extra"][:nx]) == sorted(int(x) for x in g["extra"][t][:nx]), f"op {t}: extra edges"
+        if meta.get("log_cap", 0):
+            tail = np.zeros(TR.LOG_TAIL, np.uint32)
+            recs = [l for l in env.simulator.logger.get_logs()[-TR.LOG_TAIL:] if l is not None]
+            tail[TR.LOG_TAIL - len(recs):] = [l["from_device"] | (l["to_device"] << 16) for l in recs]
+            assert np.array_equal(tail, g["logs_tail"][t]), f"op {t}: hop-log records"
+
+
 def oracle_for(net, seed, xcap, env_id0=0, base_line="Nash"):
     from oracle import cyg_oracle as O
     cfg = O.make_config(net.cfg, net.E, seed=seed, xcap=xcap, base_line=base_line)

@@ -12,7 +12,7 @@ import pytest
 
 from oracle import ref_harness as H
 
-pytestmark = pytest.mark.skipif(not H.available(), reason="reference checkout not present")
+needs_reference = pytest.mark.skipif(not H.available(), reason="reference checkout not present")
 
 
 class ReplayedRef:
@@ -53,6 +53,7 @@ def _pair(numOfDevice, M, seed, draw_seed=77, env_id=5):
     return ReplayedRef(ref), ours
 
 
+@needs_reference
 @pytest.mark.parametrize("numOfDevice,M,seed", [(10, 20, 21), (40, 50, 22)])
 def test_unmodified_double_oracle_runs_on_the_dropin(numOfDevice, M, seed):
     warnings.filterwarnings("ignore")
@@ -153,6 +154,24 @@ def test_dropin_pickles_and_info_counters():
         env.simulator.subnet.net[0].isCompromised = True
 
 
+@pytest.mark.parametrize("name", ["c2_m50_detector", "c1_m30_detector_busy_log"])
+def test_dropin_replays_the_references_detector_trajectories(name):
+    """The reference's recorded detector trajectories (defender 10 fits the IsolationForest on the hop log, scans consult
+    it) fed to the drop-in on the host compile of the device source: the drop-in must fit where the reference did, with
+    numpy's stream seeded alike, and reach the same 6-tuples, device state and hop log after every step."""
+    from cygym_b200 import network_from_golden
+    from cygym_b200.volt_typhoon_env import Volt_Typhoon_CyberDefenseEnv
+    from tests.common import GOLDEN, load_golden, replay_golden_on_gym
+    from tests.emu.emu_venv import EmuVectorEnv
+    warnings.filterwarnings("ignore")
+    g = load_golden([p for p in GOLDEN if name in p][0])
+    net, meta = network_from_golden(g)
+    env = Volt_Typhoon_CyberDefenseEnv(net, seed=meta["draw_seed"], env_id=meta["env_id"], xcap=meta["xcap"], venv_cls=EmuVectorEnv)
+    replay_golden_on_gym(env, g)
+    assert env.simulator.detector.trained and int((g["train_seed"] >= 0).sum()) >= 10
+
+
+@needs_reference
 def test_dropin_trains_and_consults_the_detector_like_the_reference():
     """Defender action 10 fits the IsolationForest on the hop log (scikit-learn, on the host, from the ring the kernels
     keep) and later scans (action 5) consult it on the device (volt:945-962, :1020-1069): same 6-tuples, same device

@@ -1,28 +1,15 @@
 """The drop-in Gym surface (Volt_Typhoon_CyberDefenseEnv.reset()/step()) against golden trajectories of the
 reference: same action tuples in, same rewards / done / observations / counters out."""
-import json
-
 import numpy as np
 import pytest
 
-from oracle import trajectory as TR
-from tests.common import GOLDEN, load_golden
+from tests.common import GOLDEN, load_golden, replay_golden_on_gym
 
 pytestmark = pytest.mark.gpu
 
 
-def _decode(hdr, mask, order, M, order_form):
-    at = int(np.int8(hdr[0] & 0xFF))
-    if (int(hdr[0]) & 0xFF) == 0x80:
-        return None
-    n_ex = (int(hdr[0]) >> 16) & 0xFF
-    ex = [int(np.int8((int(hdr[1]) >> (8 * i)) & 0xFF)) for i in range(n_ex)]
-    n = int(hdr[2]) & 0xFFFF
-    devs = [int(x) for x in order[:n]] if order_form else [d for d in range(M) if (int(mask[d >> 5]) >> (d & 31)) & 1]
-    return (at, ex, devs, int(np.int32(hdr[3])))
-
-
-@pytest.mark.parametrize("name", ["c1_m20_plain", "c1_m20_order", "c1_m20_baselines", "c2_m50_plain"])
+@pytest.mark.parametrize("name", ["c1_m20_plain", "c1_m20_order", "c1_m20_baselines", "c2_m50_plain",
+                                  "c2_m50_detector", "c1_m30_detector_busy_log"])
 def test_gym_surface_replays_golden(name):
     from cygym_b200 import network_from_golden
     from cygym_b200.volt_typhoon_env import Volt_Typhoon_CyberDefenseEnv
@@ -31,44 +18,7 @@ def test_gym_surface_replays_golden(name):
     env = Volt_Typhoon_CyberDefenseEnv(net, seed=meta["draw_seed"], env_id=meta["env_id"], xcap=meta["xcap"])
     assert env.get_num_action_types("defender") == 14 and env.get_num_action_types("attacker") == 3
     assert env.Max_network_size == meta["M"] and env.MaxExploits == 6
-    M = meta["M"]
-    for t in range(len(g["kind"])):
-        kind = int(g["kind"][t])
-        if kind == TR.OP_RANDOMIZE:
-            env.randomize_compromise_and_ownership()
-            continue
-        if kind == TR.OP_BASELINE:
-            env.base_line = TR.BASELINES[int(g["baseline"][t])]
-            continue
-        G = int(g["n_groups"][t])
-        env.mode = "attacker" if int(g["mode"][t]) else "defender"
-        acts = [_decode(g["hdr"][t][k], g["mask"][t][k], g["order"][t][k], M, meta["order_form"]) for k in range(G)]
-        # the reference drew every non-None action with sample_action(): one draw epoch each
-        env._venv.scalars[:, 1] += sum(1 for a in acts if a is not None)
-        env._host = None
-        out = env.step(acts if kind == TR.OP_GROUPED else acts[0])
-        assert len(out) == 6
-        state, raw, shaped, done, info, logs = out
-        tol = 1e-5 * max(1.0, abs(float(g["raw"][t])))
-        assert abs(raw - float(g["raw"][t])) <= tol and abs(shaped - float(g["shaped"][t])) <= tol, f"op {t}"
-        assert done == bool(g["done"][t])
-        assert state.shape == (6 * M,) and state.dtype == np.float64
-        s6 = state.reshape(M, 6)
-        for row, col in enumerate((2, 4, 5)):
-            exp = np.array([(int(g["pre"][t][row, d >> 5]) >> (d & 31)) & 1 for d in range(M)], np.float64)
-            assert np.array_equal(s6[:, col], exp), f"op {t}: returned state column {col}"
-        assert np.array_equal(env._get_defender_state().astype(np.float32), g["obs_def"][t]), f"op {t}"
-        a_obs = env._get_attacker_state()
-        assert a_obs.dtype == np.float32 and a_obs.shape == (4 * M + 6,) and np.array_equal(a_obs, g["obs_att"][t])
-        sc = g["scal"][t]
-        assert env.step_num == int(sc[0]) and env.work_done == int(sc[8]) and env.scan_cnt == int(sc[11])
-        assert env.compromised_devices_cnt == int(sc[7]) and env.edges_blocked == int(sc[14])
-        assert info["Compromised_devices"] == int(sc[7]) and info["mode"] == env.mode
-        # info is built before step_num moves in step(), after it in step_grouped() (volt:1272-1285 / :746-755)
-        assert info["step_count"] == (int(sc[0]) if kind == TR.OP_GROUPED else int(sc[0]) - 1), f"op {t}"
-        assert len(logs) == int(sc[6])
-        nya = np.array([(int(g["dev"][t][d]) >> 2) & 1 for d in range(M)])
-        assert [int(d.Not_yet_added) for d in env._get_ordered_devices()] == nya.tolist()
+    replay_golden_on_gym(env, g)
 
 
 def test_gym_surface_errors_and_counters():

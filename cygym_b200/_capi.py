@@ -19,19 +19,64 @@ _DEPS = [_SRC, os.path.join(_HERE, "csrc", "cyg_core.cuh"), os.path.join(_HERE, 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 PLANE_WIDTHS = (1, 2, 3, 4, 64)  # one translation unit of cyg_kernels.cu per plane width W (+ one for the C-ABI)
 
+# The constants of include/cygym_b200.h, named as there without the CYG_ prefix (tests/test_abi_formats.py checks them).
+ABI_VERSION = 2
 NSCAL = 16
 ATYPE_NONE = 0x80
 MODE_DEFENDER, MODE_ATTACKER = 0, 1
 STEP_GROUPED, STEP_SKIP_WORK = 1, 2
-BASE_LINES = {"Nash": 0, "No Defense": 1, "Preset": 2, "No Attack": 3}
+BL_NASH, BL_NO_DEFENSE, BL_PRESET, BL_NO_ATTACK, BL_OTHER = range(5)
+BASE_LINES = {"Nash": BL_NASH, "No Defense": BL_NO_DEFENSE, "Preset": BL_PRESET, "No Attack": BL_NO_ATTACK}
 E_INVAL, E_NOMEM, E_CUDA, E_STATE = -22, -12, -5, -71
+
+# canonical per-device word dev[B][M] (CYG_DEV_*)
+DEV_COMP, DEV_KNOWN, DEV_NYA, DEV_OWNED = 1 << 0, 1 << 1, 1 << 2, 1 << 3
+DEV_REMOVED, DEV_HASWL, DEV_BUSYSET, DEV_ACTSET = 1 << 4, 1 << 5, 1 << 6, 1 << 7
+DEV_PT_SHIFT, DEV_BUSY_SHIFT, DEV_CBY_SHIFT = 8, 12, 20
+DEV_PT_MASK, DEV_BUSY_MASK, DEV_CBY_MASK = 0x7, 0xFF, 0x3F
+# per-device checkpoint word ckpt[B][M] (CYG_CK_*); processing time, busy time and compromised_by use the DEV_* fields
+CK_COMP, CK_KNOWN, CK_NYA, CK_REACH, CK_HASWL, CK_VALID = 1 << 0, 1 << 1, 1 << 2, 1 << 3, 1 << 5, 1 << 31
+# static per-device word dev_static[M] (CYG_ST_*)
+ST_DC, ST_SERVER, ST_REACH = 1 << 0, 1 << 1, 1 << 2
+ST_NAPPS_SHIFT, ST_VULN_SHIFT = 8, 16
 
 # scalar slots (CYG_S_*)
 (S_STEP, S_EPOCH, S_FLAGS, S_PREV_X, S_DEF_STEP, S_ATT_STEP, S_LOGS, S_COMPCNT, S_WORK, S_DEFCOST,
  S_CLEANCOST, S_SCAN, S_REVERT, S_CKPT, S_EBLK, S_EADD) = range(16)
-FL_ERR_MASK = 0xF0
-FL_DET_TRAINED, FL_DET_PENDING = 0x4, 0x8
-DET_WORDS = 6160
+# flag bits of scal[S_FLAGS] (CYG_FL_*); bit FL_DISC_SHIFT + e: exploits[e].discovered
+FL_HAS_CKPT, FL_SETS_INIT, FL_DET_TRAINED, FL_DET_PENDING = 0x1, 0x2, 0x4, 0x8
+FL_ERR_BUSY, FL_ERR_XCAP, FL_ERR_DETECTOR, FL_ERR_MASK = 0x10, 0x20, 0x40, 0xF0
+FL_DISC_SHIFT = 8
+
+# The reference env's counters held in scalar slots: (attribute name, info-dict key, slot, slot holds float32 bits),
+# in the key order of VectorCyberDefenseEnv.info() and of the reference's info dict (volt_typhoon_env.py:1272-1285).
+COUNTERS = (
+    ("step_num", "step_count", S_STEP, False), ("revert_count", "revert_count", S_REVERT, False),
+    ("checkpoint_count", "checkpoint_count", S_CKPT, False), ("defensive_cost", "defensive_cost", S_DEFCOST, True),
+    ("clearning_cost", "clearning_cost", S_CLEANCOST, True), ("scan_cnt", "Scan_count", S_SCAN, False),
+    ("work_done", "work_done", S_WORK, False), ("compromised_devices_cnt", "Compromised_devices", S_COMPCNT, False),
+    ("edges_blocked", "Edges Blocked", S_EBLK, False), ("edges_added", "Edges Added", S_EADD, False),
+    ("defender_step", "defender_step", S_DEF_STEP, False), ("attacker_step", "attacker_step", S_ATT_STEP, False),
+)
+
+# extra (per-env) edge word extra[B][xcap] (CYG_X_*)
+X_V_SHIFT, X_BLOCKED, X_IDMASK = 12, 1 << 24, 0xFFF
+
+# trained-detector slot (CYG_DET_*)
+DET_WORDS, DET_TREE0, DET_TREE_STRIDE, DET_TABLE = 6160, 4, 2048, 4100
+
+
+def extra_edges(words):
+    """Extra-edge words -> [(from_device, to_device, blocked)]."""
+    return [(int(w) & X_IDMASK, (int(w) >> X_V_SHIFT) & X_IDMASK, bool(int(w) & X_BLOCKED)) for w in words]
+
+
+def log_records(ring, n, k):
+    """The last k of the n records of an env's hop-log ring (record i at i % len(ring), from_device | to_device << 16),
+    in log order: int64 array [k, 2] of (from_device, to_device)."""
+    import numpy as np
+    r = np.asarray(ring, np.uint32)[np.arange(n - k, n) % max(1, len(ring))]
+    return np.stack([r & 0xFFFF, r >> 16], axis=1).astype(np.int64)
 
 
 class CygConfig(C.Structure):
@@ -219,7 +264,7 @@ def make_config(cfg, E, seed=0, xcap=16, base_line="Nash", tri_mode=2, tri_high=
     c.zero_day_mask = cfg["zero_day_mask"]
     c.att_space_n, c.def_space_n, c.default_high = cfg["att_space_n"], cfg["def_space_n"], cfg["default_high"]
     c.n_app_ids = cfg.get("n_app_ids", 0)
-    c.base_line = BASE_LINES.get(base_line, 4)
+    c.base_line = BASE_LINES.get(base_line, BL_OTHER)
     c.tri_high = tri_high
     c.log_cap = int(log_cap)
     c.work_scale, c.comp_scale, c.def_scale, c.gamma = cfg["work_scale"], cfg["comp_scale"], cfg["def_scale"], cfg["gamma"]

@@ -10,7 +10,8 @@ decision_function, predict of sklearn/ensemble/_iforest.py, 1.9) -- so the devic
 """
 import numpy as np
 
-DET_WORDS, DET_TREE0, DET_TREE_STRIDE, DET_TABLE = 6160, 4, 2048, 4100  # include/cygym_b200.h CYG_DET_*
+from ._capi import DET_TABLE, DET_TREE0, DET_TREE_STRIDE, DET_WORDS
+
 MAX_NODES = 512
 
 

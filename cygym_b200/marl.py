@@ -4,7 +4,7 @@ envs at once, as torch ops on the env's own device buffers.  The grouped step it
 VectorCyberDefenseEnv.step_grouped (volt_typhoon_env.py:694-779)."""
 import torch
 
-from .vector_env import ActionBatch, VectorCyberDefenseEnv
+from .vector_env import ActionBatch, VectorCyberDefenseEnv, header_rows, pack_device_mask
 
 P_COMP, P_KNOWN, P_NYA, P_OWNED = 0, 1, 2, 3   # bit-plane ids of the internal record (cyg_core.cuh)
 REC_PLANES = 16
@@ -73,17 +73,6 @@ def grouped_actions(env: VectorCyberDefenseEnv, per_dev_types, role, exp_idx, ap
     return out
 
 
-def _pack_mask(m, W):
-    """bool [B, M] -> int32 [B, W] device masks."""
-    B, M = m.shape
-    pad = W * 32 - M
-    if pad:
-        m = torch.nn.functional.pad(m, (0, pad))
-    weights = (1 << torch.arange(32, device=m.device, dtype=torch.int64))
-    words = (m.view(B, W, 32).to(torch.int64) * weights).sum(-1)
-    return torch.where(words >= 2 ** 31, words - 2 ** 32, words).to(torch.int32)
-
-
 def grouped_actions_from_types(env: VectorCyberDefenseEnv, per_dev_types, visible, exp_idx, app_idx, mode, n_types, noop,
                                single_choice=None):
     """per_dev_types: int [B, M] sampled action type per device; visible: [B, M] (>0.5 = counts);
@@ -110,6 +99,5 @@ def grouped_actions_from_types(env: VectorCyberDefenseEnv, per_dev_types, visibl
                 sel = sel & first
         n_dev = sel.sum(1).to(torch.int32)
         atype = torch.where(n_dev > 0, torch.full_like(n_dev, t), torch.full_like(n_dev, noop))
-        hdr = torch.stack([(atype & 0xFF) | (m << 8) | (1 << 16), exp_idx.to(torch.int32) & 0xFF, n_dev, app_idx.to(torch.int32)], dim=1)
-        groups.append(ActionBatch(hdr.contiguous(), _pack_mask(sel, W).contiguous()))
+        groups.append(ActionBatch(header_rows(atype, m, exp_idx, n_dev, app_idx), pack_device_mask(sel, W).contiguous()))
     return groups

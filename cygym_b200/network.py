@@ -21,13 +21,8 @@ import math
 import numpy as np
 
 from . import cve as CVE
-
-DEV_COMP, DEV_KNOWN, DEV_NYA, DEV_OWNED = 1 << 0, 1 << 1, 1 << 2, 1 << 3
-DEV_REMOVED, DEV_HASWL, DEV_BUSYSET, DEV_ACTSET = 1 << 4, 1 << 5, 1 << 6, 1 << 7
-DEV_PT_SHIFT, DEV_BUSY_SHIFT, DEV_CBY_SHIFT = 8, 12, 20
-ST_DC, ST_SERVER, ST_REACH = 1 << 0, 1 << 1, 1 << 2
-ST_NAPPS_SHIFT, ST_VULN_SHIFT = 8, 16
-NSCAL = 16
+from ._capi import (DEV_COMP, DEV_HASWL, DEV_KNOWN, DEV_NYA, DEV_OWNED, DEV_PT_SHIFT, NSCAL, S_PREV_X, ST_DC, ST_NAPPS_SHIFT,
+                    ST_REACH, ST_SERVER, ST_VULN_SHIFT)
 
 DEFAULT_CFG = dict(
     X=6, n_exploits=2, Min_network_size=2, work_scale=1.0, comp_scale=30.0, def_scale=1.0, gamma=0.99,
@@ -58,7 +53,7 @@ class Network:
 
     def blank_template(self, xcap=16):
         scal = np.zeros(NSCAL, np.uint32)
-        scal[3] = 0xFFFF  # _prev_att_potential is None
+        scal[S_PREV_X] = 0xFFFF  # _prev_att_potential is None
         return dict(dev=np.zeros(self.M, np.uint32), ckpt=np.zeros(self.M, np.uint32),
                     blocked=np.zeros(self.EW, np.uint32), extra=np.zeros(0, np.uint32), scal=scal)
 
@@ -244,7 +239,7 @@ def synthetic_network(M=100, num_of_device=None, n_subnets=8, seed=0, n_cve_rows
             pt = min(5, max(1, pt))
             dev[int(d)] |= DEV_HASWL | (pt << DEV_PT_SHIFT)
     scal = np.zeros(NSCAL, np.uint32)
-    scal[3] = 0xFFFF
+    scal[S_PREV_X] = 0xFFFF
     E = len(col)
     template = dict(dev=dev, ckpt=np.zeros(M, np.uint32), blocked=np.zeros(max(1, (E + 31) // 32), np.uint32),
                     extra=np.zeros(0, np.uint32), scal=scal)

@@ -11,8 +11,19 @@ evaluation.  The 10 columns are simulate_game's return tuple (do_agent.py:2078-2
 """
 import numpy as np
 
+from . import _capi as K
+
 COLUMNS = ("defender_return", "attacker_return", "compromised_fraction", "jobs_completed", "scan_count",
            "defensive_cost", "checkpoint_count", "revert_count", "edges_blocked", "edges_added")
+_INFO_OF_COLUMN = ("Compromised_devices", "work_done", "Scan_count", "defensive_cost", "checkpoint_count", "revert_count",
+                   "Edges Blocked", "Edges Added")  # env.info() keys of COLUMNS[2:]
+# the counters the reference zeroes before a rollout (do_agent.py:2038-2045)
+_ROLLOUT_RESET = (K.S_STEP, K.S_DEF_STEP, K.S_ATT_STEP, K.S_WORK, K.S_CKPT, K.S_DEFCOST, K.S_CLEANCOST, K.S_REVERT, K.S_SCAN)
+
+
+def _columns(def_r, att_r, info):
+    """The 10 COLUMNS of every env as float64 [B] tensors: the defender / attacker returns and env.info() counters."""
+    return [def_r, att_r] + [info[k].double() for k in _INFO_OF_COLUMN]
 
 
 class Strategy:
@@ -60,7 +71,6 @@ def evaluate_payoff_matrix(network, def_strategies, att_strategies, n_rollouts, 
     """Returns a float64 tensor [n_def, n_att, 10] (averages) on `device`."""
     import torch
     from .vector_env import ActionBatch, VectorCyberDefenseEnv
-    from . import _capi as K
     lo, hi = shard_range(n_rollouts, rank, world)
     nloc = hi - lo
     nd, na = len(def_strategies), len(att_strategies)
@@ -73,11 +83,8 @@ def evaluate_payoff_matrix(network, def_strategies, att_strategies, n_rollouts, 
                 env = VectorCyberDefenseEnv(network, nloc, device=device, seed=seed,
                                             env_id0=(i * na + j) * n_rollouts + lo, xcap=xcap)
                 env.randomize_compromise_and_ownership()
-                # counters the reference zeroes before a rollout (do_agent.py:2038-2045)
-                s = env.scalars
-                for slot in (K.S_STEP, K.S_DEF_STEP, K.S_ATT_STEP, K.S_WORK, K.S_CKPT, K.S_DEFCOST, K.S_CLEANCOST,
-                             K.S_REVERT, K.S_SCAN):
-                    s[:, slot] = 0
+                for slot in _ROLLOUT_RESET:
+                    env.scalars[:, slot] = 0
                 def_r = torch.zeros(nloc, dtype=torch.float64, device=device)
                 att_r = torch.zeros(nloc, dtype=torch.float64, device=device)
                 for t in range(steps_per_episode):
@@ -94,11 +101,7 @@ def evaluate_payoff_matrix(network, def_strategies, att_strategies, n_rollouts, 
                         def_r += raw.double()
                     else:
                         att_r += raw.double()
-                info = env.info()
-                cols = [def_r, att_r, info["Compromised_devices"].double(), info["work_done"].double(),
-                        info["Scan_count"].double(), info["defensive_cost"].double(), info["checkpoint_count"].double(),
-                        info["revert_count"].double(), info["Edges Blocked"].double(), info["Edges Added"].double()]
-                sums[i, j] = torch.stack([c.sum() for c in cols])
+                sums[i, j] = torch.stack([c.sum() for c in _columns(def_r, att_r, env.info())])
                 env.close()
     if not reduce:
         return sums
@@ -110,14 +113,13 @@ def decode_actions(raw, mode, n_types, M, X, n_app, W):
     raw [N, n_types + M + X + n_app] on the device -> (hdr [N, 4], mask [N, W]) int32.  action_type = argmax of the type
     slice, device_indices = where(slice > 0) (ascending: the set form), exploit and app index = argmax of their slices."""
     import torch
-    from .marl import _pack_mask
+    from .vector_env import header_rows, pack_device_mask
     m = 1 if mode in (1, "attacker") else 0
     at = raw[:, :n_types].argmax(1).to(torch.int32)
     dev = raw[:, n_types:n_types + M] > 0
     ex = raw[:, n_types + M:n_types + M + X].argmax(1).to(torch.int32)
     app = raw[:, n_types + M + X:n_types + M + X + n_app].argmax(1).to(torch.int32) if n_app > 0 else torch.zeros_like(at)
-    hdr = torch.stack([(at & 0xFF) | (m << 8) | (1 << 16), ex & 0xFF, dev.sum(1).to(torch.int32), app], dim=1)
-    return hdr.contiguous(), _pack_mask(dev, W).contiguous()
+    return header_rows(at, m, ex, dev.sum(1), app), pack_device_mask(dev, W).contiguous()
 
 
 def _strategy_rows(def_strategies, att_strategies, T, M):
@@ -125,7 +127,6 @@ def _strategy_rows(def_strategies, att_strategies, T, M):
     turn: per side (hdr rows [R, 4], mask rows [R, W], row index [T, S], base_line code [S] (255 = the strategy does not
     touch env.base_line)).  A fixed sequence of L actions is L rows indexed by t % L."""
     from .vector_env import ActionBatch
-    from . import _capi as K
     out = []
     for mode, sts in ((0, def_strategies), (1, att_strategies)):
         hs, ms, first, length, bls, n_rows = [], [], [], [], [], 0
@@ -136,7 +137,7 @@ def _strategy_rows(def_strategies, att_strategies, T, M):
                 if st.actor is not None:
                     acts, bl = [None], 255
                 elif st.baseline_name is not None:
-                    acts, bl = [None], K.BASE_LINES.get(st.baseline_name, 4)
+                    acts, bl = [None], K.BASE_LINES.get(st.baseline_name, K.BL_OTHER)
                 elif st.actions:
                     acts, bl = list(st.actions), 255
                 else:
@@ -188,11 +189,12 @@ def _block_order(env, sides, i_of_pair, j_of_pair, pair_of_env, T):
     unblock actions over 40 devices against the no-op), so the launch used to end with whichever expensive blocks
     started last.  The estimate needs no measurement: action types and list lengths of the strategies' rows."""
     import torch
-    from . import _capi as K
+    from .vector_env import decode_header
     cost_side = []
     for mode, (h, _, ridx, bls) in enumerate(sides):
-        t = (h[:, 0] & 0xFF).astype(np.int64)
-        n = (h[:, 2] & 0xFFFF).astype(np.float64)
+        f = decode_header(h)
+        t = (f.atype & 0xFF).astype(np.int64)
+        n = f.n_dev.astype(np.float64)
         if mode == 0:
             c = _TURN_BASE + np.array([_DEF_PER_DEVICE.get(int(x), 0.0) for x in t]) * n
         else:
@@ -230,7 +232,6 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
     here (use the per-pair evaluator)."""
     import torch
     from .vector_env import ActionBatch, VectorCyberDefenseEnv
-    from . import _capi as K
     nd, na = len(def_strategies), len(att_strategies)
     P, T = nd * na, int(steps_per_episode)
     M, W = network.M, network.W
@@ -253,9 +254,8 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
         i_of_pair = np.arange(P) // na
         j_of_pair = np.arange(P) % na
         env.randomize_compromise_and_ownership()
-        s = env.scalars
-        for slot in (K.S_STEP, K.S_DEF_STEP, K.S_ATT_STEP, K.S_WORK, K.S_CKPT, K.S_DEFCOST, K.S_CLEANCOST, K.S_REVERT, K.S_SCAN):
-            s[:, slot] = 0
+        for slot in _ROLLOUT_RESET:
+            env.scalars[:, slot] = 0
         # per-pair tables, assembled on the device from the strategies' packed rows: the moving side's row of every turn,
         # and the base_line each pair's env carries on that turn (a strategy that sets no base_line leaves it as the
         # other player's last baseline left it, do_agent.py:716-719)
@@ -311,11 +311,7 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
                 env.set_base_line_per_env(bl_d[t][pair_of_env])
                 raw, _, _ = env.step(ActionBatch(hdr_e, mask_e))
                 ret[mode] += raw.double()
-        info = env.info()
-        cols = torch.stack([ret[0], ret[1], info["Compromised_devices"].double(), info["work_done"].double(),
-                            info["Scan_count"].double(), info["defensive_cost"].double(), info["checkpoint_count"].double(),
-                            info["revert_count"].double(), info["Edges Blocked"].double(), info["Edges Added"].double()], dim=1)
-        sums.index_add_(0, pair_of_env, cols)
+        sums.index_add_(0, pair_of_env, torch.stack(_columns(ret[0], ret[1], env.info()), dim=1))
     sums = sums.view(nd, na, len(COLUMNS))
     if not reduce:
         return sums

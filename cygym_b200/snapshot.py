@@ -13,11 +13,11 @@ import json
 
 import numpy as np
 
-from .network import (DEV_ACTSET, DEV_BUSY_SHIFT, DEV_BUSYSET, DEV_CBY_SHIFT, DEV_COMP, DEV_HASWL, DEV_KNOWN, DEV_NYA,
-                      DEV_OWNED, DEV_PT_SHIFT, DEV_REMOVED, NSCAL, ST_DC, ST_NAPPS_SHIFT, ST_REACH, ST_SERVER,
-                      ST_VULN_SHIFT, Network)
-
-CK_COMP, CK_KNOWN, CK_NYA, CK_REACH, CK_HASWL, CK_VALID = 1 << 0, 1 << 1, 1 << 2, 1 << 3, 1 << 5, 1 << 31
+from . import _capi as K
+from ._capi import (CK_COMP, CK_HASWL, CK_KNOWN, CK_NYA, CK_REACH, CK_VALID, DEV_ACTSET, DEV_BUSY_MASK, DEV_BUSY_SHIFT,
+                    DEV_BUSYSET, DEV_CBY_MASK, DEV_CBY_SHIFT, DEV_COMP, DEV_HASWL, DEV_KNOWN, DEV_NYA, DEV_OWNED, DEV_PT_MASK,
+                    DEV_PT_SHIFT, DEV_REMOVED, NSCAL, ST_DC, ST_NAPPS_SHIFT, ST_REACH, ST_SERVER, ST_VULN_SHIFT)
+from .network import Network
 
 
 def save_npz(path, net: Network):
@@ -125,23 +125,23 @@ def from_reference_env(env):
         if e is not None:
             blocked[e >> 5] |= np.uint32(1 << (e & 31))
     scal = np.zeros(NSCAL, np.uint32)
-    scal[0] = env.step_num
-    fl = (1 if env.checkpoint is not None else 0) | (2 if has_sets else 0)
+    scal[K.S_STEP] = env.step_num
+    fl = (K.FL_HAS_CKPT if env.checkpoint is not None else 0) | (K.FL_SETS_INIT if has_sets else 0)
     if getattr(env.simulator.detector, "trained", False):
-        fl |= 4  # CYG_FL_DET_TRAINED
+        fl |= K.FL_DET_TRAINED
     for i, exp in enumerate(exploits):
         if exp.discovered:
-            fl |= 1 << (8 + i)
-    scal[2] = fl
+            fl |= 1 << (K.FL_DISC_SHIFT + i)
+    scal[K.S_FLAGS] = fl
     prev = getattr(env, "_prev_att_potential", None)
-    scal[3] = 0xFFFF if prev is None else int(round(prev * M / env.γ))
-    scal[4], scal[5] = env.defender_step, env.attacker_step
-    scal[6] = len(env.simulator.logger.logs)
-    scal[7], scal[8] = env.compromised_devices_cnt, env.work_done
+    scal[K.S_PREV_X] = 0xFFFF if prev is None else int(round(prev * M / env.γ))
+    scal[K.S_DEF_STEP], scal[K.S_ATT_STEP] = env.defender_step, env.attacker_step
+    scal[K.S_LOGS] = len(env.simulator.logger.logs)
+    scal[K.S_COMPCNT], scal[K.S_WORK] = env.compromised_devices_cnt, env.work_done
     f32 = np.array([env.defensive_cost, env.clearning_cost], np.float32).view(np.uint32)
-    scal[9], scal[10] = f32[0], f32[1]
-    scal[11], scal[12], scal[13] = env.scan_cnt, env.revert_count, env.checkpoint_count
-    scal[14], scal[15] = env.edges_blocked, env.edges_added
+    scal[K.S_DEFCOST], scal[K.S_CLEANCOST] = f32[0], f32[1]
+    scal[K.S_SCAN], scal[K.S_REVERT], scal[K.S_CKPT] = env.scan_cnt, env.revert_count, env.checkpoint_count
+    scal[K.S_EBLK], scal[K.S_EADD] = env.edges_blocked, env.edges_added
     zd = 0
     if env.zero_day:
         for i in (set(env.common_exploit_indices) | set(env.private_exploit_indices)):
@@ -198,32 +198,32 @@ def apply_state_to_reference_env(env, net, state):
         d.Not_yet_added = bool(w & DEV_NYA)
         d.attacker_owned = bool(w & DEV_OWNED)
         d.removed_before = 1 if w & DEV_REMOVED else 0
-        d.busy_time = float((w >> DEV_BUSY_SHIFT) & 0xFF)
+        d.busy_time = float((w >> DEV_BUSY_SHIFT) & DEV_BUSY_MASK)
         if w & DEV_HASWL:
             wl = Workload()
-            wl.processing_time = (w >> DEV_PT_SHIFT) & 7
+            wl.processing_time = (w >> DEV_PT_SHIFT) & DEV_PT_MASK
             wl.adversarial, wl.assigned, wl.wtype = False, True, d.wtype
             d.workload = wl
         else:
             d.workload = None
-        cb = (w >> DEV_CBY_SHIFT) & 0x3F
+        cb = (w >> DEV_CBY_SHIFT) & DEV_CBY_MASK
         d.compromised_by = type(d.compromised_by)(exploits[e].id for e in range(len(exploits)) if (cb >> e) & 1)
     env._device_ckpts = {}
     for i in range(M):
         k = int(ck[i])
         if k & CK_VALID:
-            cb = (k >> DEV_CBY_SHIFT) & 0x3F
+            cb = (k >> DEV_CBY_SHIFT) & DEV_CBY_MASK
             env._device_ckpts[i] = dict(
                 isCompromised=bool(k & CK_COMP), Known_to_attacker=bool(k & CK_KNOWN), Not_yet_added=bool(k & CK_NYA),
                 reachable_by_attacker=bool(k & CK_REACH),
-                workload=({"processing_time": (k >> DEV_PT_SHIFT) & 7, "adversarial": False} if k & CK_HASWL else None),
-                busy_time=float((k >> DEV_BUSY_SHIFT) & 0xFF),
+                workload=({"processing_time": (k >> DEV_PT_SHIFT) & DEV_PT_MASK, "adversarial": False} if k & CK_HASWL else None),
+                busy_time=float((k >> DEV_BUSY_SHIFT) & DEV_BUSY_MASK),
                 compromised_by=[exploits[e].id for e in range(len(exploits)) if (cb >> e) & 1])
     # extra (hub-star) edges go into the graph; the cache rebuild makes them visible and forgets the blocks (volt:476) ...
     g = sim.subnet.graph
-    n_extra = int(sc[3]) >> 16
+    n_extra = int(sc[K.S_PREV_X]) >> 16
     have = set(g.get_edgelist())
-    new_edges = [(int(x & 0xFFF), int((x >> 12) & 0xFFF)) for x in np.asarray(state["extra"], np.uint32)[:n_extra]]
+    new_edges = [(u, v) for u, v, _ in K.extra_edges(np.asarray(state["extra"], np.uint32)[:n_extra])]
     add = [e for e in new_edges if e not in have]
     if add:
         g.add_edges(add)
@@ -235,32 +235,32 @@ def apply_state_to_reference_env(env, net, state):
         for e in range(int(net.row_ptr[u]), int(net.row_ptr[u + 1])):
             if (int(bl[e >> 5]) >> (e & 31)) & 1:
                 blocked.add((u, int(net.col[e])))
-    for x in np.asarray(state["extra"], np.uint32)[:n_extra]:
-        if int(x) & (1 << 24):
-            blocked.add((int(x & 0xFFF), int((x >> 12) & 0xFFF)))
+    for u, v, is_blocked in K.extra_edges(np.asarray(state["extra"], np.uint32)[:n_extra]):
+        if is_blocked:
+            blocked.add((u, v))
     env._blocked = blocked
     env._busy_devices = {devs[i] for i in range(M) if int(dev[i]) & DEV_BUSYSET}
-    if int(sc[2]) & 2:  # CYG_FL_SETS_INIT
+    if int(sc[K.S_FLAGS]) & K.FL_SETS_INIT:
         env._active_ids = {i for i in range(M) if int(dev[i]) & DEV_ACTSET}
         env._inactive_ids = {i for i in range(M) if not int(dev[i]) & DEV_ACTSET}
     else:
         for a in ("_active_ids", "_inactive_ids"):
             if hasattr(env, a):
                 delattr(env, a)
-    env.checkpoint = {"simulator": sim, "state": env.state} if int(sc[2]) & 1 else None  # an alias, as checkpoint_variables stores it
+    env.checkpoint = {"simulator": sim, "state": env.state} if int(sc[K.S_FLAGS]) & K.FL_HAS_CKPT else None  # an alias, as checkpoint_variables stores it
     for e, exp in enumerate(exploits):
-        exp.discovered = bool((int(sc[2]) >> (8 + e)) & 1)
-    pn = int(sc[3]) & 0xFFFF
+        exp.discovered = bool((int(sc[K.S_FLAGS]) >> (K.FL_DISC_SHIFT + e)) & 1)
+    pn = int(sc[K.S_PREV_X]) & 0xFFFF
     env._prev_att_potential = None if pn == 0xFFFF else env.γ * (pn / M)
-    env.step_num, env.defender_step, env.attacker_step = int(sc[0]), int(sc[4]), int(sc[5])
-    env.compromised_devices_cnt, env.work_done = int(sc[7]), int(sc[8])
-    env.defensive_cost = float(sc[9:10].view(np.float32)[0])
-    env.clearning_cost = float(sc[10:11].view(np.float32)[0])
-    env.scan_cnt, env.revert_count, env.checkpoint_count = int(sc[11]), int(sc[12]), int(sc[13])
-    env.edges_blocked, env.edges_added = int(sc[14]), int(sc[15])
+    env.step_num, env.defender_step, env.attacker_step = int(sc[K.S_STEP]), int(sc[K.S_DEF_STEP]), int(sc[K.S_ATT_STEP])
+    env.compromised_devices_cnt, env.work_done = int(sc[K.S_COMPCNT]), int(sc[K.S_WORK])
+    env.defensive_cost = float(sc[K.S_DEFCOST:K.S_DEFCOST + 1].view(np.float32)[0])
+    env.clearning_cost = float(sc[K.S_CLEANCOST:K.S_CLEANCOST + 1].view(np.float32)[0])
+    env.scan_cnt, env.revert_count, env.checkpoint_count = int(sc[K.S_SCAN]), int(sc[K.S_REVERT]), int(sc[K.S_CKPT])
+    env.edges_blocked, env.edges_added = int(sc[K.S_EBLK]), int(sc[K.S_EADD])
     # the hop log: the kernels keep its length; records beyond what is known are neutral placeholders
     logs = sim.logger.logs
-    n = int(sc[6])
+    n = int(sc[K.S_LOGS])
     if len(logs) > n:
         del logs[n:]
     while len(logs) < n:

@@ -6,6 +6,7 @@ device memory and streams only; every state transition is a kernel of libcygym_b
 through the C-ABI of include/cygym_b200.h.  There is no CPU path.
 """
 import ctypes as C
+from collections import namedtuple
 
 import numpy as np
 import torch
@@ -58,6 +59,47 @@ class ActionBatch:
                 raise ValueError("mask form needs an ascending duplicate-free device list; use order_form=True")
         return hdr, mask, order
 
+    @staticmethod
+    def unpack(hdr, mask, order=None):
+        """The inverse of pack: hdr [B, 4] + mask [B, W] (+ order [B, >= n_dev] for the order form) -> the list of B
+        reference-style action tuples, None where the header holds ATYPE_NONE."""
+        f = decode_header(hdr)
+        bits = np.unpackbits(np.ascontiguousarray(mask).view(np.uint8).reshape(len(f.atype), -1), axis=1, bitorder="little")
+        devs = lambda b: [int(d) for d in order[b][:f.n_dev[b]]] if order is not None else np.nonzero(bits[b])[0].tolist()
+        return [None if (f.atype[b] & 0xFF) == K.ATYPE_NONE else (int(f.atype[b]), f.ex[b, :f.n_ex[b]].tolist(), devs(b), int(f.app[b]))
+                for b in range(len(f.atype))]
+
+
+ActionHeader = namedtuple("ActionHeader", "atype mode n_ex ex n_dev first app")
+
+
+def decode_header(hdr):
+    """Action headers [B, 4] (numpy or CPU torch; include/cygym_b200.h) -> ActionHeader of [B] arrays: atype (the
+    signed type byte; ATYPE_NONE reads as -128), mode, n_ex, ex [B, 4] (signed exploit bytes), n_dev, first
+    (device_indices[0], -1 when not given) and app."""
+    h = np.ascontiguousarray(hdr.numpy() if hasattr(hdr, "numpy") else hdr).view(np.uint32).reshape(-1, 4)
+    i8 = lambda a: (a & 0xFF).astype(np.uint8).view(np.int8).astype(np.int32)
+    return ActionHeader(atype=i8(h[:, 0]), mode=(h[:, 0] >> 8) & 1, n_ex=(h[:, 0] >> 16) & 0xFF,
+                        ex=i8(h[:, 1][:, None] >> (8 * np.arange(4, dtype=np.uint32))), n_dev=h[:, 2] & 0xFFFF,
+                        first=(h[:, 2] >> 16).astype(np.int64) - 1, app=h[:, 3].view(np.int32))
+
+
+def header_rows(atype, mode, exploit, n_dev, app):
+    """torch: single-exploit action headers [N, 4] int32 from int [N] tensors (mode: 0 defender, 1 attacker)."""
+    i32 = lambda t: t.to(torch.int32)
+    return torch.stack([(i32(atype) & 0xFF) | (mode << 8) | (1 << 16), i32(exploit) & 0xFF, i32(n_dev), i32(app)], dim=1)
+
+
+def pack_device_mask(m, W):
+    """torch: bool [B, M] -> int32 [B, W] device masks."""
+    B, M = m.shape
+    pad = W * 32 - M
+    if pad:
+        m = torch.nn.functional.pad(m, (0, pad))
+    weights = (1 << torch.arange(32, device=m.device, dtype=torch.int64))
+    words = (m.view(B, W, 32).to(torch.int64) * weights).sum(-1)
+    return torch.where(words >= 2 ** 31, words - 2 ** 32, words).to(torch.int32)
+
 
 def compact_action_rows(hdr, mask):
     """hdr [B, 4] + mask [B, W] (numpy or CPU torch, the arrays of ActionBatch.pack) -> compact rows [B, 2 + W] int32
@@ -65,10 +107,8 @@ def compact_action_rows(hdr, mask):
     action does not fit the compact ranges (exploit indices -8..7, app_index -32768..32767, device_indices[0] < 255)."""
     h = np.ascontiguousarray(hdr.numpy() if hasattr(hdr, "numpy") else hdr).view(np.uint32)
     m = np.ascontiguousarray(mask.numpy() if hasattr(mask, "numpy") else mask).view(np.uint32)
-    n_ex = (h[:, 0] >> 16) & 0xFF
-    n_dev, first1 = h[:, 2] & 0xFFFF, h[:, 2] >> 16
-    app = h[:, 3].view(np.int32)
-    ex = ((h[:, 1][:, None] >> (8 * np.arange(4, dtype=np.uint32))) & 0xFF).astype(np.uint8).view(np.int8).astype(np.int32)
+    f = decode_header(h)
+    n_ex, n_dev, first1, app, ex = f.n_ex, f.n_dev, (f.first + 1).astype(np.uint32), f.app, f.ex
     if (h[:, 0] >> 24).any() or ((h[:, 0] >> 9) & 0x7F).any() or (n_ex > 4).any() or (n_dev > 4095).any() or (first1 > 255).any() \
             or (app < -32768).any() or (app > 32767).any() or (ex < -8).any() or (ex > 7).any():
         raise ValueError("action outside the compact row ranges: use the full hdr / mask arrays")
@@ -181,7 +221,7 @@ class VectorCyberDefenseEnv:
     def set_base_line(self, name):
         self.base_line = name
         self._drop_graphs()
-        K.check(self.L.cyg_set_base_line(self.h, K.BASE_LINES.get(name, 4)))
+        K.check(self.L.cyg_set_base_line(self.h, K.BASE_LINES.get(name, K.BL_OTHER)))
 
     def set_base_line_per_env(self, codes):
         """codes: uint8 device tensor [B] of CYG_BL_* (see _capi.BASE_LINES), or [T, B] with one row per step of the
@@ -483,9 +523,7 @@ class VectorCyberDefenseEnv:
         if k > self.log_cap:
             raise ValueError(f"the hop-log ring keeps {self.log_cap} records per env, {k} are needed (log_cap=)")
         base = self.B * (self.S + self.M + self.xcap)
-        ring = self._state[base + b * self.log_cap: base + (b + 1) * self.log_cap].cpu().numpy().view(np.uint32)
-        r = ring[(np.arange(n - k, n) % max(1, self.log_cap)).astype(np.int64)]
-        return np.stack([r & 0xFFFF, r >> 16], axis=1).astype(np.int64)
+        return K.log_records(self._state[base + b * self.log_cap: base + (b + 1) * self.log_cap].cpu().numpy(), n, k)
 
     def pending_detectors(self):
         """Envs whose defender trained the detector (action 10 on a non-empty log) since the last service."""
@@ -543,13 +581,8 @@ class VectorCyberDefenseEnv:
     # ---- counters (the `info` dict of volt:1272-1285, per env) ----
     def info(self):
         s = self.scalars
-        f = lambda i: s[:, i].contiguous().view(torch.float32)
-        return {
-            "step_count": s[:, K.S_STEP], "revert_count": s[:, K.S_REVERT], "checkpoint_count": s[:, K.S_CKPT],
-            "defensive_cost": f(K.S_DEFCOST), "clearning_cost": f(K.S_CLEANCOST), "Scan_count": s[:, K.S_SCAN],
-            "work_done": s[:, K.S_WORK], "Compromised_devices": s[:, K.S_COMPCNT], "Edges Blocked": s[:, K.S_EBLK],
-            "Edges Added": s[:, K.S_EADD], "defender_step": s[:, K.S_DEF_STEP], "attacker_step": s[:, K.S_ATT_STEP],
-        }
+        return {key: s[:, slot].contiguous().view(torch.float32) if is_float else s[:, slot]
+                for _, key, slot, is_float in K.COUNTERS}
 
     def error_flags(self):
         """Sticky per-env CYG_FL_ERR_* bits (0 everywhere on a healthy run)."""

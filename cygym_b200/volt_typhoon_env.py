@@ -15,16 +15,17 @@ import numpy as np
 import torch
 
 from . import _capi as K
-from .network import (DEV_BUSY_SHIFT, DEV_CBY_SHIFT, DEV_COMP, DEV_HASWL, DEV_KNOWN, DEV_NYA, DEV_OWNED, DEV_PT_SHIFT,
-                      DEV_REMOVED, ST_DC, ST_NAPPS_SHIFT, ST_REACH, ST_SERVER, Network, synthetic_network)
-from .vector_env import ActionBatch, VectorCyberDefenseEnv
+from ._capi import (DEV_BUSY_MASK, DEV_BUSY_SHIFT, DEV_CBY_MASK, DEV_CBY_SHIFT, DEV_COMP, DEV_HASWL, DEV_KNOWN, DEV_NYA,
+                    DEV_OWNED, DEV_PT_MASK, DEV_PT_SHIFT, DEV_REMOVED, ST_DC, ST_NAPPS_SHIFT, ST_REACH, ST_SERVER)
+from .network import Network, synthetic_network
+from .vector_env import ActionBatch, VectorCyberDefenseEnv, decode_header
 
-_COUNTERS = {
-    "step_num": K.S_STEP, "defender_step": K.S_DEF_STEP, "attacker_step": K.S_ATT_STEP, "work_done": K.S_WORK,
-    "checkpoint_count": K.S_CKPT, "revert_count": K.S_REVERT, "scan_cnt": K.S_SCAN,
-    "compromised_devices_cnt": K.S_COMPCNT, "edges_blocked": K.S_EBLK, "edges_added": K.S_EADD,
-}
-_FLOAT_COUNTERS = {"defensive_cost": K.S_DEFCOST, "clearning_cost": K.S_CLEANCOST}
+_COUNTER_SLOTS = {attr: (slot, is_float) for attr, _, slot, is_float in K.COUNTERS}
+
+
+def _counter(scal, slot, is_float):
+    """One counter from a host copy of an env's scalars."""
+    return float(scal[slot: slot + 1].view(np.float32)[0]) if is_float else int(scal[slot])
 
 
 # ---- read-only views of the object graph (CDSimulatorComponents.py:18-26, :219-242, :491-499; CDSimulator.py:663-679) ----
@@ -56,7 +57,7 @@ class DeviceView:
     attacker_owned = property(lambda s: bool(s._w() & DEV_OWNED))
     removed_before = property(lambda s: 1 if s._w() & DEV_REMOVED else 0)
     reachable_by_attacker = property(lambda s: bool(s._st() & ST_REACH))
-    busy_time = property(lambda s: (s._w() >> DEV_BUSY_SHIFT) & 0xFF)
+    busy_time = property(lambda s: (s._w() >> DEV_BUSY_SHIFT) & DEV_BUSY_MASK)
     anomaly_score = 0.0  # stays 0 under fast_scan (volt_typhoon_env.py:46)
     device_type = property(lambda s: "DomainController" if s._st() & ST_DC else "Workstation")
     wtype = property(lambda s: "server" if s._st() & ST_SERVER else "client")
@@ -67,11 +68,11 @@ class DeviceView:
     @property
     def workload(self):
         w = self._w()
-        return _Workload((w >> DEV_PT_SHIFT) & 7, self.wtype) if w & DEV_HASWL else None
+        return _Workload((w >> DEV_PT_SHIFT) & DEV_PT_MASK, self.wtype) if w & DEV_HASWL else None
 
     @property
     def compromised_by(self):
-        m = (self._w() >> DEV_CBY_SHIFT) & 0x3F
+        m = (self._w() >> DEV_CBY_SHIFT) & DEV_CBY_MASK
         return {self._env.simulator.exploits[e].id for e in range(len(self._env.simulator.exploits)) if (m >> e) & 1}
 
     def __setattr__(self, name, value):
@@ -96,8 +97,7 @@ class _GraphView:
         for u in range(n.M):
             for e in range(int(n.row_ptr[u]), int(n.row_ptr[u + 1])):
                 out.extend([(u, int(n.col[e]))] * int(n.mult[e]))
-        x = self._env._snap()["extra"]
-        out.extend((int(w & 0xFFF), int((w >> 12) & 0xFFF)) for w in x[: self._env._n_extra()])
+        out.extend((u, v) for u, v, _ in K.extra_edges(self._env._snap()["extra"][: self._env._n_extra()]))
         return out
 
     def vcount(self):
@@ -123,7 +123,7 @@ class _ExploitView:
 
     @property
     def discovered(self):
-        return bool((int(self._env._snap()["scal"][K.S_FLAGS]) >> (8 + self._e)) & 1)
+        return bool((int(self._env._snap()["scal"][K.S_FLAGS]) >> (K.FL_DISC_SHIFT + self._e)) & 1)
 
 
 class _LoggerView:
@@ -143,11 +143,9 @@ class _LoggerView:
         ring = self._env._snap().get("logs")
         if ring is None or len(ring) == 0:
             return [None] * n
-        cap = len(ring)
-        k = min(n, cap)
-        tail = [{"time_step": None, "from_device": int(r & 0xFFFF), "to_device": int(r >> 16), "kind": "A"}
-                for r in ring[(np.arange(n - k, n) % cap).astype(np.int64)]]
-        return [None] * (n - k) + tail
+        k = min(n, len(ring))
+        return [None] * (n - k) + [{"time_step": None, "from_device": int(a), "to_device": int(b), "kind": "A"}
+                                   for a, b in K.log_records(ring, n, k)]
 
     logs = property(lambda s: s.get_logs())
 
@@ -159,7 +157,7 @@ class _DetectorView:
     def __init__(self, env):
         self._env = env
 
-    trained = property(lambda s: bool(int(s._env._snap()["scal"][K.S_FLAGS]) & 4))
+    trained = property(lambda s: bool(int(s._env._snap()["scal"][K.S_FLAGS]) & K.FL_DET_TRAINED))
     random_detection = False
 
 
@@ -332,27 +330,22 @@ class Volt_Typhoon_CyberDefenseEnv:
 
     # ---- counters: views of the env's scalars; callers zero them between rollouts (do_agent.py:192-196) ----
     def __getattr__(self, name):
-        if name in _COUNTERS or name in _FLOAT_COUNTERS:
+        if name in _COUNTER_SLOTS:
             d = self.__dict__
             if d.get("_venv") is None:
                 if name in d.get("_pending", {}):
                     return d["_pending"][name]
                 raise AttributeError(name)
-            s = self._snap()["scal"]
-            if name in _COUNTERS:
-                return int(s[_COUNTERS[name]])
-            return float(s[_FLOAT_COUNTERS[name]: _FLOAT_COUNTERS[name] + 1].view(np.float32)[0])
+            return _counter(self._snap()["scal"], *_COUNTER_SLOTS[name])
         raise AttributeError(name)
 
     def __setattr__(self, name, value):
-        if name in _COUNTERS or name in _FLOAT_COUNTERS:
+        if name in _COUNTER_SLOTS:
             if self.__dict__.get("_venv") is None:
                 self._pending[name] = value  # replayed into the scalars by _build()
                 return
-            if name in _COUNTERS:
-                self._venv.scalars[0, _COUNTERS[name]] = int(value)
-            else:
-                self._venv.scalars[0, _FLOAT_COUNTERS[name]] = int(np.float32(value).view(np.int32))
+            slot, is_float = _COUNTER_SLOTS[name]
+            self._venv.scalars[0, slot] = int(np.float32(value).view(np.int32)) if is_float else int(value)
             self.__dict__["_host"] = None
         else:
             object.__setattr__(self, name, value)
@@ -384,11 +377,10 @@ class Volt_Typhoon_CyberDefenseEnv:
         """(action_type, exploit_indices, device_indices, app_index) with device_indices in random.sample's draw order
         (CyberDefenseEnv.py:555-578)."""
         ab = self._venv.sample_actions(self._mode_id(), want_order=True)
-        hdr = ab.hdr[0].cpu().numpy().view(np.uint32)
-        n = int(hdr[2]) & 0xFFFF
-        devs = [int(x) for x in ab.order[0, :n].cpu().numpy().view(np.uint16)]
+        f = decode_header(ab.hdr.cpu())
+        devs = [int(x) for x in ab.order[0, :int(f.n_dev[0])].cpu().numpy().view(np.uint16)]
         self._host = None  # the draw epoch moved
-        return (int(np.int8(hdr[0] & 0xFF)), np.array([int(np.int8(hdr[1] & 0xFF))], dtype=int), devs, int(np.int32(hdr[3])))
+        return (int(f.atype[0]), np.array([int(f.ex[0, 0])], dtype=int), devs, int(f.app[0]))
 
     def randomize_compromise_and_ownership(self):
         self._venv.randomize_compromise_and_ownership()
@@ -431,16 +423,12 @@ class Volt_Typhoon_CyberDefenseEnv:
         st[:, 2], st[:, 4], st[:, 5] = bits(0), bits(1), bits(2)
         self.state = st.reshape(-1)
         s = self._snap()["scal"]
-        f32 = lambda i: float(s[i: i + 1].view(np.float32)[0])
-        step_num = int(s[K.S_STEP])
-        info = {
-            # step() builds info BEFORE step_num increments (volt:1272-1285), step_grouped() after (volt:746-755)
-            "mode": self.mode, "step_count": step_num - 1 if (executed and not grouped) else step_num,
-            "revert_count": int(s[K.S_REVERT]), "checkpoint_count": int(s[K.S_CKPT]),
-            "defensive_cost": f32(K.S_DEFCOST), "clearning_cost": f32(K.S_CLEANCOST), "Scan_count": int(s[K.S_SCAN]),
-            "action_taken": action, "work_done": int(s[K.S_WORK]), "Compromised_devices": int(s[K.S_COMPCNT]),
-            "Edges Blocked": int(s[K.S_EBLK]), "Edges Added": int(s[K.S_EADD]),
-        }
+        c = [(key, _counter(s, slot, is_float)) for _, key, slot, is_float in K.COUNTERS]
+        # the reference's info dict: its first six counters, action_taken, four more; no defender_step / attacker_step
+        info = dict([("mode", self.mode)] + c[:6] + [("action_taken", action)] + c[6:10])
+        # step() builds info BEFORE step_num increments (volt:1272-1285), step_grouped() after (volt:746-755)
+        if executed and not grouped:
+            info["step_count"] -= 1
         return (self.state, float(out[0:1].view(np.float32)[0]), float(out[1:2].view(np.float32)[0]), bool(out[2]), info,
                 self._sim.logger.get_logs())
 

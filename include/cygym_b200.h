@@ -232,7 +232,7 @@ int cyg_set_base_line_per_env(cyg_handle h, const uint8_t* base_line);
 int cyg_set_base_line_per_env_steps(cyg_handle h, const uint8_t* base_line, int32_t n_rows);
 
 /* uint32 words PER ENV the caller must allocate for the kernels' internal state.  The buffer holds, in this
- * order: B records of S words (16 scalars + bit-planes + the blocked-edge bitset in out- and in-list order;
+ * order: B records of S words (16 scalars + bit-planes + the blocked-edge bitset in incidence-unit order;
  * what a CTA bulk-copies into shared memory), then B*M per-device checkpoint words (actions 11/12,
  * volt_typhoon_env.py:419-453), then B*xcap extra-edge words, then B*log_cap hop-log ring words.
  * words_per_env = S + M + xcap + log_cap. */

@@ -79,24 +79,13 @@ class CudaImpl:
         return o.cpu().numpy()[0]
 
 
-def gym_action(hdr, mask, order, M, order_form):
-    """A recorded action row (include/cygym_b200.h packing) as the reference's (type, exploits, devices, app) tuple."""
-    at = int(np.int8(hdr[0] & 0xFF))
-    if (int(hdr[0]) & 0xFF) == 0x80:
-        return None
-    n_ex = (int(hdr[0]) >> 16) & 0xFF
-    ex = [int(np.int8((int(hdr[1]) >> (8 * i)) & 0xFF)) for i in range(n_ex)]
-    n = int(hdr[2]) & 0xFFFF
-    devs = [int(x) for x in order[:n]] if order_form else [d for d in range(M) if (int(mask[d >> 5]) >> (d & 31)) & 1]
-    return (at, ex, devs, int(np.int32(hdr[3])))
-
-
 def replay_golden_on_gym(env, g):
     """Feed golden trajectory `g` (recorded from the reference) to the drop-in Volt_Typhoon_CyberDefenseEnv `env` as the
     reference's action tuples, and compare after every op: the 6-tuple, observations, counters, the canonical state and,
     where the recording keeps it, the hop log.  Where the reference trained its detector, numpy's stream was seeded
     with `train_seed`; the drop-in gets the same seed and must fit (and later consult) the detector on its own."""
     from oracle import trajectory as TR
+    from cygym_b200.vector_env import ActionBatch
     meta = json.loads(str(g["meta"]))
     M = meta["M"]
     for t in range(len(g["kind"])):
@@ -108,7 +97,7 @@ def replay_golden_on_gym(env, g):
         else:
             G = int(g["n_groups"][t])
             env.mode = "attacker" if int(g["mode"][t]) else "defender"
-            acts = [gym_action(g["hdr"][t][k], g["mask"][t][k], g["order"][t][k], M, meta["order_form"]) for k in range(G)]
+            acts = ActionBatch.unpack(g["hdr"][t][:G], g["mask"][t][:G], g["order"][t][:G] if meta["order_form"] else None)
             # the reference drew every non-None action with sample_action(): one draw epoch each
             env._venv.scalars[:, 1] += sum(1 for a in acts if a is not None)
             env._host = None

@@ -25,13 +25,6 @@ def test_draw_tables_match_the_oracle_contract():
     assert abs(t[0] / 2**32 - 0.1) < 1e-9 and abs(t[1] / 2**32 - 0.4) < 1e-9 and abs(t[3] / 2**32 - 14 / 15) < 1e-9
 
 
-def test_config_struct_mirrors_agree():
-    from cygym_b200 import _capi as K
-    from oracle import cyg_oracle as O
-    assert [f[0] for f in K.CygConfig._fields_] == [f[0] for f in O.CygConfig._fields_]
-    assert C.sizeof(K.CygConfig) == C.sizeof(O.CygConfig)
-
-
 def test_action_pack_roundtrip_and_errors():
     from cygym_b200.vector_env import ActionBatch
     hdr, mask, order = ActionBatch.pack([(6, [1], [3, 40, 99], 7), None, (1, [0, 2], [], 0)], ["defender", "attacker", "attacker"], 100)
@@ -45,6 +38,11 @@ def test_action_pack_roundtrip_and_errors():
         ActionBatch.pack([(1, [0], [100], 0)], 0, 100)
     h, m, o = ActionBatch.pack([(1, [0], [5, 2, 5], 0)], 0, 100, order_form=True)
     assert list(o[0, :3]) == [5, 2, 5] and h[0, 2] == 3
+    # unpack is the inverse of pack, in set form and in order form
+    acts = [(6, [1], [3, 40, 99], 7), None, (1, [0, 2], [], 0), (-3, [-8, 7, 0, 5], list(range(0, 100, 7)), -500)]
+    assert ActionBatch.unpack(*ActionBatch.pack(acts, 0, 100)[:2]) == acts
+    acts[0] = (6, [1], [99, 3, 40, 3], 7)
+    assert ActionBatch.unpack(*ActionBatch.pack(acts, 1, 100, order_form=True)) == acts
 
 
 def test_compact_action_rows_roundtrip_and_ranges():
@@ -75,7 +73,7 @@ def test_compact_action_rows_roundtrip_and_ranges():
 @pytest.mark.parametrize("M,subnets", [(20, 1), (50, 3), (100, 8), (2000, 64)])
 def test_synthetic_network_invariants(M, subnets):
     from cygym_b200 import synthetic_network
-    from cygym_b200.network import DEV_COMP, DEV_NYA, DEV_OWNED, ST_DC, ST_SERVER
+    from cygym_b200._capi import DEV_COMP, DEV_NYA, DEV_OWNED, ST_DC, ST_SERVER
     net = synthetic_network(M, n_subnets=subnets, seed=3)
     assert net.row_ptr[0] == 0 and net.row_ptr[-1] == net.E == len(net.col)
     for u in range(M):
@@ -125,7 +123,7 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(lib, name), f"{name} declared in the header but not exported"
     assert sorted(K.EXPORTS) == declared
     lib.cyg_version.restype = C.c_int
-    assert lib.cyg_version() == 2
+    assert lib.cyg_version() == K.ABI_VERSION
 
 
 def test_product_package_never_imports_the_oracle():

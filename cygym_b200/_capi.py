@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CYGYM_B200_LIB") or os.path.join(_HERE, "libcygym_b200.so")  # override: profiling builds only
 _SRC = os.path.join(_HERE, "csrc", "cyg_kernels.cu")
 _DEPS = [_SRC, os.path.join(_HERE, "csrc", "cyg_core.cuh"), os.path.join(_HERE, "csrc", "cyg_coop.cuh"),
-         os.path.join(_HERE, "csrc", "cyg_tables.h"),
+         os.path.join(_HERE, "csrc", "cyg_tables.h"), os.path.join(_HERE, "csrc", "cyg_iforest.cuh"),
          os.path.join(os.path.dirname(_HERE), "include", "cygym_b200.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
@@ -63,7 +63,7 @@ COUNTERS = (
 X_V_SHIFT, X_BLOCKED, X_IDMASK = 12, 1 << 24, 0xFFF
 
 # trained-detector slot (CYG_DET_*)
-DET_WORDS, DET_TREE0, DET_TREE_STRIDE, DET_TABLE = 6160, 4, 2048, 4100
+DET_WORDS, DET_TREE0, DET_TREE_STRIDE, DET_TABLE, DET_WINDOW = 6160, 4, 2048, 4100, 2000
 
 
 def extra_edges(words):
@@ -128,7 +128,7 @@ class CygRolloutArgs(C.Structure):
 
 
 EXPORTS = ["cyg_version", "cyg_last_error", "cyg_create", "cyg_destroy", "cyg_set_base_line", "cyg_set_base_line_per_env", "cyg_set_base_line_per_env_steps", "cyg_internal_words",
-           "cyg_bind", "cyg_set_detectors", "cyg_import_state", "cyg_export_state", "cyg_step", "cyg_step_multi", "cyg_rollout", "cyg_unpack_actions", "cyg_pack_done", "cyg_block_envs", "cyg_set_env_id_stride", "cyg_randomize", "cyg_rebuild_graph_cache", "cyg_sample_actions", "cyg_sample_actions_ordered",
+           "cyg_bind", "cyg_set_detectors", "cyg_fit_detectors", "cyg_import_state", "cyg_export_state", "cyg_step", "cyg_step_multi", "cyg_rollout", "cyg_unpack_actions", "cyg_pack_done", "cyg_block_envs", "cyg_set_env_id_stride", "cyg_randomize", "cyg_rebuild_graph_cache", "cyg_sample_actions", "cyg_sample_actions_ordered",
            "cyg_observe", "cyg_group_actions", "cyg_launch_count", "cyg_set_debug_cycles"]
 
 
@@ -225,6 +225,7 @@ def lib():
         L.cyg_internal_words.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
         L.cyg_bind.argtypes = [C.c_void_p, C.c_void_p]
         L.cyg_set_detectors.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]
+        L.cyg_fit_detectors.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.cyg_import_state.argtypes = [C.c_void_p, C.POINTER(CygState), C.c_void_p]
         L.cyg_export_state.argtypes = [C.c_void_p, C.POINTER(CygState), C.c_void_p]
         L.cyg_step.argtypes = [C.c_void_p, C.POINTER(CygActions), C.c_uint32, C.POINTER(CygStepOut), C.c_void_p]

@@ -15,6 +15,8 @@
  *                                           defender / 3+X attacker branches do not serialise
  *     3. epilogue  thread t -> env t      : work, arrivals, reward, counters, evolve_network,
  *                                           coalesced outputs, optional fused observation rows
+ * cyg_fit_assign_kernel + cyg_fit_kernel: the detector fit of defender action 10 (cyg_iforest.cuh), one warp per
+ *   pending env.
  * No tensor cores: the path has no dense contraction.  No CPU fallback anywhere in this file.
  */
 #include <cuda_runtime.h>
@@ -27,6 +29,7 @@
 
 #include "cyg_coop.cuh"
 #include "cyg_core.cuh"
+#include "cyg_iforest.cuh"
 #include "cyg_tables.h"
 
 using namespace cyg;
@@ -925,6 +928,108 @@ extern "C" void cyg_pack_done_launch(int blocks, int threads, cudaStream_t st, c
 }
 #endif
 
+/* ---- detector fits (cyg_fit_detectors; cyg_iforest.cuh) ---- */
+struct FitParams {
+  uint32_t* recs;          /* internal records [B][S] (the scalars lead each) */
+  const uint32_t* logs;    /* internal hop-log rings [B][log_cap], NULL when log_cap == 0 */
+  uint32_t* slots;         /* detector slots [n_slots][CYG_DET_WORDS] */
+  int32_t* det_of_env;     /* [B] */
+  const uint32_t* seeds;   /* [B] */
+  int32_t* next_slot;      /* first free slot */
+  int32_t* work;           /* [2 + B]: envs to fit, the fit kernel's cursor, their list */
+  int S, B, log_cap, n_slots;
+};
+#define CYG_FIT_WARPS 4 /* fitting warps per CTA (cyg_iforest::Scratch each, in shared memory) */
+#if defined(CYG_TU_W) && CYG_TU_W == 4
+/* Block-wide exclusive count of `v` over the threads below this one; *total = count over the block. */
+__device__ __forceinline__ int block_rank(bool v, int* warp_tot, int* total) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = (blockDim.x + 31) >> 5;
+  const uint32_t m = __ballot_sync(0xFFFFFFFFu, v);
+  if (lane == 0) warp_tot[warp] = __popc(m);
+  __syncthreads();
+  int before = 0, all = 0;
+  for (int w = 0; w < nwarps; w++) {
+    before += w < warp ? warp_tot[w] : 0;
+    all += warp_tot[w];
+  }
+  __syncthreads();
+  *total = all;
+  return before + __popc(m & ((1u << lane) - 1u));
+}
+/* One CTA walks the envs in order: slots go to pending envs without one in env order (deterministic, and the same
+ * order service_detectors() uses); the envs that can be fitted are listed for cyg_fit_kernel. */
+__global__ void __launch_bounds__(1024) cyg_fit_assign_kernel(const __grid_constant__ FitParams p) {
+  __shared__ int warp_tot[32];
+  const int first = *p.next_slot;
+  int taken = 0, listed = 0;
+  for (int c = 0; c < p.B; c += blockDim.x) {
+    const int b = c + (int)threadIdx.x;
+    bool pend = false, fits_ring = false;
+    int cur = -1;
+    uint32_t flags = 0;
+    if (b < p.B) {
+      const uint32_t* sc = p.recs + (size_t)b * p.S;
+      flags = sc[CYG_S_FLAGS];
+      pend = (flags & CYG_FL_DET_PENDING) != 0;
+      if (pend) {
+        const uint32_t nl = sc[CYG_S_LOGS];
+        const uint32_t win = nl < (uint32_t)CYG_DET_WINDOW ? nl : (uint32_t)CYG_DET_WINDOW;
+        fits_ring = p.logs != nullptr && win >= 1u && win <= (uint32_t)p.log_cap;
+        cur = p.det_of_env[b];
+      }
+    }
+    const bool need = pend && fits_ring && cur < 0;
+    int n_need, n_ok;
+    const int slot = first + taken + block_rank(need, warp_tot, &n_need);
+    const bool ok = pend && fits_ring && (cur >= 0 || slot < p.n_slots);
+    const int at = listed + block_rank(ok, warp_tot, &n_ok);
+    if (need && slot < p.n_slots) p.det_of_env[b] = slot;
+    if (pend && !ok) p.recs[(size_t)b * p.S + CYG_S_FLAGS] = flags | CYG_FL_ERR_DETECTOR;
+    if (ok) p.work[2 + at] = b;
+    taken += n_need;
+    listed += n_ok;
+  }
+  if (threadIdx.x == 0) {
+    const int next = first + taken;
+    *p.next_slot = next <= p.n_slots ? next : (first > p.n_slots ? first : p.n_slots);
+    p.work[0] = listed;
+    p.work[1] = 0;
+  }
+}
+/* Persistent warps take the listed envs one by one: lane 0 runs the serial fit (streams, row sampling, tree builds)
+ * in shared memory, all lanes zero the slot and fill the verdict table. */
+__global__ void __launch_bounds__(32 * CYG_FIT_WARPS) cyg_fit_kernel(const __grid_constant__ FitParams p) {
+  extern __shared__ __align__(16) unsigned char fit_smem[];
+  iforest::Scratch& s = reinterpret_cast<iforest::Scratch*>(fit_smem)[threadIdx.x >> 5];
+  const int lane = threadIdx.x & 31;
+  const int n = p.work[0];
+  for (;;) {
+    int i = 0;
+    if (lane == 0) i = atomicAdd(&p.work[1], 1);
+    i = __shfl_sync(0xFFFFFFFFu, i, 0);
+    if (i >= n) break;
+    const int b = p.work[2 + i];
+    uint32_t* slot = p.slots + (size_t)p.det_of_env[b] * CYG_DET_WORDS;
+    uint32_t* sc = p.recs + (size_t)b * p.S;
+    for (int w = lane; w < CYG_DET_WORDS; w += 32) slot[w] = 0u;
+    __syncwarp();
+    if (lane == 0) iforest::fit_serial(s, p.logs + (size_t)b * p.log_cap, (uint32_t)p.log_cap, sc[CYG_S_LOGS], p.seeds[b], slot);
+    __syncwarp();
+    iforest::verdict_words(s, slot, lane, 32);
+    if (lane == 0) sc[CYG_S_FLAGS] &= ~CYG_FL_DET_PENDING;
+    __syncwarp();
+  }
+}
+extern "C" int cyg_fit_launch(int n_sms, cudaStream_t st, const FitParams& p) {
+  const size_t smem = sizeof(iforest::Scratch) * CYG_FIT_WARPS;
+  cudaError_t e = cudaFuncSetAttribute(cyg_fit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return (int)e;
+  cyg_fit_assign_kernel<<<1, 1024, 0, st>>>(p);
+  cyg_fit_kernel<<<3 * n_sms, 32 * CYG_FIT_WARPS, smem, st>>>(p); /* 3 CTAs of 4 Scratch each fit one SM's shared memory */
+  return (int)cudaGetLastError();
+}
+#endif
+
 struct ObsParams {
   Net net;
   const uint32_t* recs;
@@ -1005,6 +1110,7 @@ extern "C" {
 void cyg_group_launch(int blocks, int threads, cudaStream_t st, const GroupParams& p);
 void cyg_unpack_launch(int blocks, int threads, cudaStream_t st, const UnpackParams& p);
 void cyg_pack_done_launch(int blocks, int threads, cudaStream_t st, const int32_t* done, uint32_t* bits, int B);
+int cyg_fit_launch(int n_sms, cudaStream_t st, const FitParams& p);
 const WOps* cyg_wops_4(void);
 #ifndef CYG_FAST_BUILD /* profiling builds link the W = 4 unit only (config C3) */
 const WOps* cyg_wops_1(void);
@@ -1039,6 +1145,8 @@ struct cyg_env_s {
   unsigned long long* dbg_cycles;
   const uint32_t* det_slots; /* uploaded detectors (device memory of the caller) */
   const int32_t* det_of_env;
+  int n_det_slots;
+  int32_t* fit_work; /* [2 + B] device words of cyg_fit_detectors (allocated with the detector slots) */
   const uint8_t* bl_env;
   int bl_rows;       /* rows of [B] codes behind bl_env (cyg_set_base_line_per_env_steps; 1 otherwise) */
   int id_run, id_stride; /* cyg_set_env_id_stride (0: env id = env_id0 + slot) */
@@ -1125,7 +1233,7 @@ int cyg_create(cyg_handle* out, const cyg_config* cfg, const cyg_network* host_n
   std::string err = build_tables(*cfg, *host_net, h->blob);
   if (!err.empty()) { delete h; return fail(CYG_E_INVAL, err); }
   h->B = B; h->env_id0 = env_id0; h->device = device; h->state = nullptr; h->launches = 0; h->dbg_cycles = nullptr; h->bl_env = nullptr; h->bl_rows = 1; h->id_run = 0; h->id_stride = 0;
-  h->det_slots = nullptr; h->det_of_env = nullptr;
+  h->det_slots = nullptr; h->det_of_env = nullptr; h->n_det_slots = 0; h->fit_work = nullptr;
   h->W = h->blob.net.W;
   DeviceGuard g(device);
   if (!g.ok) { delete h; return fail(CYG_E_CUDA, "cudaSetDevice failed"); }
@@ -1151,6 +1259,7 @@ int cyg_destroy(cyg_handle h) {
   if (!h) return CYG_OK;
   DeviceGuard g(h->device);
   cudaFree(h->d_blob);
+  if (h->fit_work) cudaFree(h->fit_work);
   delete h;
   return CYG_OK;
 }
@@ -1191,11 +1300,34 @@ int cyg_set_base_line_per_env_steps(cyg_handle h, const uint8_t* base_line, int3
   return CYG_OK;
 }
 
+static uint32_t* logs_of(cyg_handle h);
 int cyg_set_detectors(cyg_handle h, const uint32_t* slots, int32_t n_slots, const int32_t* det_of_env) {
   if (!h) return fail(CYG_E_INVAL, "null handle");
   if ((slots == nullptr) != (det_of_env == nullptr) || (slots && n_slots < 1)) return fail(CYG_E_INVAL, "slots and det_of_env go together");
+  if (slots && !h->fit_work) {
+    DeviceGuard g(h->device);
+    CU(cudaMalloc((void**)&h->fit_work, sizeof(int32_t) * (2 + (size_t)h->B)));
+  }
   h->det_slots = slots;
   h->det_of_env = det_of_env;
+  h->n_det_slots = slots ? n_slots : 0;
+  return CYG_OK;
+}
+
+/* Detector.train of every pending env on the device (CDSimulator.py:687-695; cyg_iforest.cuh restates scikit-learn's
+ * ensemble/_iforest.py, ensemble/_bagging.py, utils/_random.pyx, tree/_splitter.pyx, _partitioner.pyx, _criterion.pyx,
+ * _tree.pyx and numpy's legacy MT19937). */
+int cyg_fit_detectors(cyg_handle h, const uint32_t* seeds, int32_t* next_slot, void* stream) {
+  if (!h) return fail(CYG_E_INVAL, "null handle");
+  if (!h->det_slots) return fail(CYG_E_INVAL, "cyg_fit_detectors: the handle has no detector slots (cyg_set_detectors)");
+  if (!seeds || !next_slot) return fail(CYG_E_INVAL, "null argument");
+  if (!h->state) return fail(CYG_E_INVAL, "cyg_bind() first");
+  DeviceGuard g(h->device);
+  FitParams p = {h->state, logs_of(h), const_cast<uint32_t*>(h->det_slots), const_cast<int32_t*>(h->det_of_env), seeds, next_slot,
+                 h->fit_work, (int)h->net.S, h->B, h->net.cfg.log_cap, h->n_det_slots};
+  const int e = cyg_fit_launch(h->n_sms, (cudaStream_t)stream, p);
+  h->launches += 2;
+  if (e != 0) return cuda_fail((cudaError_t)e, "cyg_fit_detectors");
   return CYG_OK;
 }
 

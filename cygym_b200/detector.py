@@ -2,9 +2,10 @@
 CDSimulator.py:681-723).
 
 The reference's Detector is scikit-learn's IsolationForest(n_estimators=2, max_samples=256) fitted on the (from, to)
-pairs of the last <= 2000 hop-log records.  The FIT stays scikit-learn's (its arithmetic and its use of numpy's global
-random stream are not ours to restate); what the kernels need is PREDICT, and that is two tree walks plus a threshold on
-a function of the two leaves reached.  `pack_detector` ships exactly that: the trees, and the forest's verdict for every
+pairs of the last <= 2000 hop-log records.  Here the FIT is scikit-learn's, drawing from numpy's global random stream;
+with a seed per env the same fit also runs on the device (VectorCyberDefenseEnv.fit_detectors, csrc/cyg_iforest.cuh),
+into the same slot format, word for word.  What the step kernels need is PREDICT, and that is two tree walks plus a
+threshold on a function of the two leaves reached.  `pack_detector` ships exactly that: the trees, and the forest's verdict for every
 PAIR of leaves, computed here with the same numpy expressions scikit-learn evaluates (_compute_score_samples,
 decision_function, predict of sklearn/ensemble/_iforest.py, 1.9) -- so the device never evaluates 2 ** x.
 """

@@ -142,7 +142,8 @@ class VectorCyberDefenseEnv:
                  stream=None, log_cap=0, detector_slots=0):
         """log_cap: records of every env's hop log kept in a ring (simulator.logger.logs, CDSimulator.py:663-679): 0 = only
         its length; >= 30 serves scans with a trained detector, 2000 what detector training reads.  detector_slots: how
-        many envs can hold a trained detector (IsolationForest fitted on the host by service_detectors())."""
+        many envs can hold a trained detector (IsolationForest fitted by fit_detectors() on the device or by
+        service_detectors() on the host)."""
         if not torch.cuda.is_available():
             raise RuntimeError("VectorCyberDefenseEnv needs a CUDA device (no CPU fallback)")
         self.L = K.lib()
@@ -183,11 +184,12 @@ class VectorCyberDefenseEnv:
         self._stream = stream
         self._obs = {}
         self._pre = None
-        self._det_slots = self._det_of_env = None
-        self._n_det = 0
+        self._det_slots = self._det_of_env = self._next_slot = None
         if detector_slots:
             self._det_slots = torch.zeros(int(detector_slots), K.DET_WORDS, dtype=torch.int32, device=self.device)
             self._det_of_env = torch.full((self.B,), -1, dtype=torch.int32, device=self.device)
+            # the first free slot: both fit paths take slots from this one device counter
+            self._next_slot = torch.zeros(1, dtype=torch.int32, device=self.device)
             K.check(self.L.cyg_set_detectors(self.h, _ptr(self._det_slots), int(detector_slots), _ptr(self._det_of_env)))
         self.reset()
 
@@ -515,7 +517,7 @@ class VectorCyberDefenseEnv:
             self._hold_mask = env_mask
         K.check(self.L.cyg_randomize(self.h, _ptr(env_mask), self._s()))
 
-    # ---- trained detectors (defender actions 10 / 5; the fit is scikit-learn's, on the host) ----
+    # ---- trained detectors (defender actions 10 / 5; fitted on the device from per-env seeds, or by scikit-learn) ----
     def log_records(self, b, last=2000):
         """The last `last` hop-log records of env b in log order: int array [n, 2] of (from_device, to_device)."""
         n = int(self.scalars[b, K.S_LOGS].item())
@@ -533,7 +535,9 @@ class VectorCyberDefenseEnv:
         """Fit (scikit-learn IsolationForest on the env's last <= 2000 hop-log records: Detector.train,
         CDSimulator.py:687-695) and upload the detector of every pending env; the next scan of that env consults it.
         Call after a step that may have trained (the Gym drop-in does it itself).  seed_of_env(b) -> seed for numpy's
-        global stream before env b's fit (the reference's forest has random_state=None), or None."""
+        global stream before env b's fit (the reference's forest has random_state=None), or None: the fit then draws
+        from numpy's stream as it stands, which only this host path can do.  With a seed per env, fit_detectors() does
+        the same fits on the device in one launch."""
         from . import detector as DET
         pend = self.pending_detectors()
         for b in pend:
@@ -541,14 +545,30 @@ class VectorCyberDefenseEnv:
                 raise RuntimeError("no detector slots: construct the env with detector_slots=")
             slot = int(self._det_of_env[b].item())
             if slot < 0:
-                if self._n_det >= self._det_slots.shape[0]:
+                slot = int(self._next_slot.item())
+                if slot >= self._det_slots.shape[0]:
                     raise RuntimeError(f"all {self._det_slots.shape[0]} detector slots are taken (detector_slots=)")
-                slot, self._n_det = self._n_det, self._n_det + 1
+                self._next_slot.fill_(slot + 1)
                 self._det_of_env[b] = slot
             model = DET.fit_detector(self.log_records(b), None if seed_of_env is None else seed_of_env(b))
             self._det_slots[slot] = torch.from_numpy(DET.pack_detector(model).view(np.int32)).to(self.device)
             self.scalars[b, K.S_FLAGS] &= ~K.FL_DET_PENDING
         return len(pend)
+
+    def fit_detectors(self, seeds):
+        """Fit the detector of every pending env on the device, in one launch and without a host synchronisation
+        (cyg_fit_detectors): env b's slot becomes exactly what service_detectors(lambda b: seeds[b]) uploads, i.e.
+        numpy's global stream seeded with seeds[b], then scikit-learn's IsolationForest on the env's last <= 2000 hop-log
+        records.  seeds: integer tensor [B] with values in [0, 2**32).  An env that cannot be fitted (every slot taken,
+        or a hop-log ring shorter than the records the fit reads) stays pending and gets CYG_FL_ERR_DETECTOR
+        (error_flags()).  Envs without a slot take the next free ones in env order, from the counter service_detectors()
+        uses as well."""
+        s = torch.as_tensor(seeds).to(self.device, torch.int64, non_blocking=True).reshape(-1)
+        assert s.numel() == self.B, "one seed per env"
+        s = s & 0xFFFFFFFF
+        s = torch.where(s >= 2 ** 31, s - 2 ** 32, s).to(torch.int32).contiguous()
+        self._hold_seeds = s
+        K.check(self.L.cyg_fit_detectors(self.h, _ptr(s), _ptr(self._next_slot), self._s()))
 
     def rebuild_graph_cache(self, env_mask=None):
         """_rebuild_graph_cache() from outside a step (volt_typhoon_env.py:456-483): every blocked edge is forgotten (:476)."""

@@ -90,14 +90,17 @@ enum {
 #define CYG_FL_HAS_CKPT 0x00000001u     /* env.checkpoint is not None */
 #define CYG_FL_SETS_INIT 0x00000002u    /* env._active_ids exists */
 #define CYG_FL_DET_TRAINED 0x00000004u  /* action 10 ran with a non-empty log: simulator.detector.trained (CDSimulator.py:693-694) */
-#define CYG_FL_DET_PENDING 0x00000008u  /* ... and the host has not yet fitted / uploaded that model (cyg_set_detectors): the
-                                           IsolationForest FIT is scikit-learn's, done on the host from the env's hop log;
-                                           the kernels only PREDICT (tree walks).  A scan that finds it set raises
-                                           CYG_FL_ERR_DETECTOR.  Never part of a reference-side state: cleared by the host. */
+#define CYG_FL_DET_PENDING 0x00000008u  /* ... and that model is not yet fitted into the env's detector slot: either the host
+                                           fits it with scikit-learn and uploads it (cyg_set_detectors), or cyg_fit_detectors
+                                           fits every pending env on the device; the step kernels only PREDICT (tree walks).
+                                           A scan that finds it set raises CYG_FL_ERR_DETECTOR.  Never part of a
+                                           reference-side state: cleared by whichever fit ran. */
 #define CYG_FL_ERR_BUSY 0x00000010u     /* busy_time exceeded CYG_BUSY_MAX (kernel saturated it) */
 #define CYG_FL_ERR_XCAP 0x00000020u     /* more attacker-star edges than xcap */
 #define CYG_FL_ERR_DETECTOR 0x00000040u /* a scan needed the trained detector and the env had none uploaded (no slot, model
-                                           pending, or a hop-log ring shorter than the 30-record scan window) */
+                                           pending, or a hop-log ring shorter than the 30-record scan window); or
+                                           cyg_fit_detectors could not fit a pending env (no free slot, or a ring shorter
+                                           than the CYG_DET_WINDOW records the fit reads): the env stays pending */
 #define CYG_FL_ERR_MASK 0x000000F0u
 #define CYG_FL_DISC_SHIFT 8             /* bit e: exploits[e].discovered */
 
@@ -321,7 +324,8 @@ int cyg_rebuild_graph_cache(cyg_handle h, const uint8_t* env_mask, void* stream)
 
 /* ---- trained detector (defender action 5 after action 10; volt_typhoon_env.py:1020-1069, CDSimulator.py:681-723) -----
  * Detector = IsolationForest(n_estimators=2, max_samples=256).  The host fits it (scikit-learn, from the env's hop log)
- * and uploads the two trees plus the forest's verdict for every pair of leaves; the kernels walk the trees.  One slot =
+ * and uploads the two trees plus the forest's verdict for every pair of leaves, or cyg_fit_detectors fits it on the
+ * device into the same format; the kernels walk the trees.  One slot =
  * CYG_DET_WORDS uint32:
  *   [0]            L1 = leaves of tree 1 (row length of the verdict table)
  *   [4 + t*2048 + 4*n .. +4), t = 0, 1, node n < 512:  threshold (float64, lo / hi word), left | right << 16,
@@ -332,7 +336,19 @@ int cyg_rebuild_graph_cache(cyg_handle h, const uint8_t* env_mask, void* stream)
 #define CYG_DET_TREE0 4
 #define CYG_DET_TREE_STRIDE 2048
 #define CYG_DET_TABLE 4100
+#define CYG_DET_WINDOW 2000 /* records a fit reads: the last min(CYG_S_LOGS, 2000) of the log (CDSimulator.py:691-692) */
 int cyg_set_detectors(cyg_handle h, const uint32_t* slots, int32_t n_slots, const int32_t* det_of_env);
+/* Detector.train (CDSimulator.py:687-695) of every env with CYG_FL_DET_PENDING, on the device: numpy's global stream
+ * seeded with seeds[b] (uint32), then IsolationForest(n_estimators=2, max_samples=256).fit on the env's last
+ * min(CYG_S_LOGS, CYG_DET_WINDOW) hop-log records, read from the internal ring.  The slot written is bit-identical to what
+ * the host uploads after that seeded scikit-learn 1.9 fit (cygym_b200/csrc/cyg_iforest.cuh restates ensemble/_iforest.py,
+ * ensemble/_bagging.py, utils/_random.pyx and tree/_splitter.pyx, _partitioner.pyx, _criterion.pyx, _tree.pyx).
+ * An env without a slot (det_of_env[b] < 0) takes slot *next_slot, in env order, and *next_slot advances: next_slot is a
+ * device int32 owned by the caller and shared with whatever assigns slots on the host.  A fitted env keeps
+ * CYG_FL_DET_TRAINED and loses CYG_FL_DET_PENDING.  An env that cannot be fitted -- no slot left, or
+ * min(CYG_S_LOGS, CYG_DET_WINDOW) > log_cap -- stays pending and gets CYG_FL_ERR_DETECTOR.  Two launches on `stream` (slot
+ * assignment, then the fits), no host synchronisation.  CYG_E_INVAL when the handle has no detector slots. */
+int cyg_fit_detectors(cyg_handle h, const uint32_t* seeds, int32_t* next_slot, void* stream);
 
 /* Replaces sample_action() (CyberDefenseEnv.py:555-578) for every env; writes hdr[B][4], mask[B][W]. */
 int cyg_sample_actions(cyg_handle h, int32_t mode, uint32_t* hdr, uint32_t* mask, void* stream);

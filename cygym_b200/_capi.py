@@ -138,11 +138,14 @@ class CygError(RuntimeError):
         self.code = code
 
 
-SPILL_LIMIT = 256   # bytes of spill stores tolerated in the config-C3 step kernel (cyg_step_kernel<4, true>)
+SPILL_LIMIT = 256   # bytes of spill stores tolerated in the config-C3 step kernel (cyg_step_kernel<4, false, false>)
 THREAD_CAPS = (640, 512)  # threads per CTA -> 93 / 127 registers per thread at one CTA per SM (640 measured fastest)
 
 
-def _step_kernel_spill(ptxas_log, mangled="_Z15cyg_step_kernelILi4ELb1ELb0ELb0EEv10StepParams"):
+STEP_KERNEL = "_Z15cyg_step_kernelILi4ELb0ELb0EEv10StepParams"  # cyg_step_kernel<4, false, false>: plain steps, no ROLL, no LOG
+
+
+def _step_kernel_spill(ptxas_log, mangled=STEP_KERNEL):
     """Bytes of spill stores ptxas reports for the plain-step W = 4 kernel (None when the log has no such entry)."""
     import re
     m = re.search(r"Function properties for " + re.escape(mangled) + r"\s+\d+ bytes stack frame, (\d+) bytes spill stores", ptxas_log)
@@ -194,9 +197,11 @@ def build(force=False, verbose=False):
     log = ""
     for cap in THREAD_CAPS:
         w4 = compile_units(LIB_PATH, extra=[f"-DCYG_MAX_BLOCK_THREADS={cap}"], verbose=verbose)
-        spill = _step_kernel_spill(w4)
-        log += f"[cygym_b200 build] {cap} threads per CTA: cyg_step_kernel<4, plain> spills {spill} bytes\n"
-        if spill is None or spill <= SPILL_LIMIT:
+        spill = _step_kernel_spill(w4, STEP_KERNEL)
+        if spill is None:
+            raise RuntimeError(f"the W = 4 ptxas log has no entry for {STEP_KERNEL}: the spill check would check nothing")
+        log += f"[cygym_b200 build] {cap} threads per CTA: cyg_step_kernel<4, false, false> spills {spill} bytes\n"
+        if spill <= SPILL_LIMIT:
             break
     with open(LIB_PATH + ".buildlog", "w") as f:
         f.write(log)

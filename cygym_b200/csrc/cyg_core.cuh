@@ -1612,15 +1612,9 @@ struct Env {
   }
   /* ... plus block / unblock.  (Measured: the owning thread walking the list itself -- flip_walk, ~135 instructions per
    * listed device, branch-free -- is a ~90k-cycle dependent chain for a 46-device list; the warp-per-env windows of
-   * cyg_coop.cuh take ~11k.  -DCYG_FLIP_THREAD keeps that experiment for envs without extra edges.) */
+   * cyg_coop.cuh take ~11k.  profiles/NOTES_r02.md.) */
   CYG_HD bool deferred_type(int mode, int atype) {
-    if (mode == CYG_MODE_DEFENDER && (atype == 6 || atype == 9)) {
-#ifdef CYG_FLIP_THREAD
-      return n_extra() > 0;
-#else
-      return true;
-#endif
-    }
+    if (mode == CYG_MODE_DEFENDER && (atype == 6 || atype == 9)) return true;
     return coop_type(mode, atype);
   }
   /* LIGHT: a plain (ungrouped, set-form) step whose cooperative types are handled elsewhere -- they return at once

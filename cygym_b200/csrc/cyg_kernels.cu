@@ -1,20 +1,17 @@
 /*
  * cyg_kernels.cu -- sm_100a kernels + the C-ABI of include/cygym_b200.h.
  *
- * cyg_step_kernel<W, PLAIN>: ONE launch per env step (volt_typhoon_env.py:818-1333 / :694-779).
- *   A CTA owns a block of NB consecutive envs.  Their internal records (cyg_core.cuh) are one
- *   contiguous span of HBM, so the CTA moves them with a single TMA bulk copy into shared
- *   memory (cp.async.bulk + mbarrier), steps them there, and writes them back with a single
- *   bulk store: HBM sees exactly one full-sector read and one write of the state per step.
- *   The hot network tables (adjacency bit rows, device masks, CSR) ride in on the same mbarrier.
- *   Work mapping is thread-per-env over bit-planes (32 devices per integer op), in three phases
- *   separated by __syncthreads():
- *     1. prologue  thread t -> env t      : epoch, executed action type, busy tick
- *     2. action    thread t -> env perm[t]: envs are counting-sorted by (mode, action type) inside
- *                                           the CTA so that a warp runs one action type and the 14
- *                                           defender / 3+X attacker branches do not serialise
- *     3. epilogue  thread t -> env t      : work, arrivals, reward, counters, evolve_network,
- *                                           coalesced outputs, optional fused observation rows
+ * The env step (volt_typhoon_env.py:818-1333 / :694-779).  A CTA owns a block of NB consecutive envs.  Their internal
+ *   records (cyg_core.cuh) are one contiguous span of HBM, so the CTA moves them with a single TMA bulk copy into shared
+ *   memory (cp.async.bulk + mbarrier) and steps them there; the hot network tables (adjacency bit rows, device masks,
+ *   CSR) ride in on the same mbarrier.  Envs are counting-sorted by (mode, executed action type) inside the CTA so that
+ *   a warp runs one action type and the 14 defender / 3+X attacker branches do not serialise.  Work is thread-per-env
+ *   over bit-planes (32 devices per integer op).
+ * cyg_step_kernel<W, ROLL, LOG>: plain steps (one set-form action per env), T fused per launch: phase A thread per
+ *   env, phase B warp per env for the draw-heavy actions, phase C thread per env; each warp sends its finished records
+ *   home by warp-wide copies.
+ * cyg_step_seq_kernel<W>: grouped steps and explicit order lists, one thread-per-env pass, one bulk store of the block.
+ * cyg_step_generic_kernel<W>: networks beyond 128 device slots (tables too large for shared memory).
  * cyg_fit_assign_kernel + cyg_fit_kernel: the detector fit of defender action 10 (cyg_iforest.cuh), one warp per
  *   pending env.
  * No tensor cores: the path has no dense contraction.  No CPU fallback anywhere in this file.
@@ -106,8 +103,6 @@ struct StepParams {
 #define CYG_NKEYS 48 /* sort keys: (mode, executed action type) in 0..31; 32..47 = block / unblock envs of a plain step
                         bucketed by listed-device count, longest first (the warp-per-env tasks of phase B run in that order) */
 #define CYG_KEY_FLIP0 32
-#define CYG_TMA_STORE 1 /* records go back with one bulk store; plain coalesced stores measured the same (the
-                          write-back is bound by the per-SM path to L2: ~16k cycles for 210 KB either way) */
 #define CYG_MAX_BLOCK_ENVS 512   /* envs per CTA */
 #ifndef CYG_MAX_BLOCK_THREADS
 #define CYG_MAX_BLOCK_THREADS 640 /* threads per CTA at one CTA per SM: 20 warps with up to 93 registers each.  Phases A / C
@@ -200,6 +195,77 @@ __device__ __forceinline__ void observe_rows(const Net& n, const uint32_t* recs,
   else observe_rows_f<W, 6>(n, recs, S, n_envs, obs_mode, out, warp, nwarps, lane);
 }
 
+/* ---- the CTA prologue of the two shared-memory step kernels ----
+ * 1. thread 0 arms the mbarrier and starts the TMA bulk loads of the hot tables and -- when the block's record span is
+ *    16-byte sized and aligned (the return value, bulk_ok) -- of the nb records */
+__device__ __forceinline__ bool load_block_start(const Net& net, uint32_t* s_tab, uint32_t* s_rec, const uint32_t* g_rec, int nb,
+                                                 int S, uint64_t* bar, int tid) {
+  const uint32_t rec_bytes = (uint32_t)nb * S * 4u;
+  const uint32_t tab_bytes = net.hot_words * 4u;
+  const bool bulk_ok = (rec_bytes & 15u) == 0 && ((((size_t)g_rec) & 15) == 0);
+  if (tid == 0) {
+    mbar_init(bar, 1);
+    mbar_expect_tx(bar, tab_bytes + (bulk_ok ? rec_bytes : 0u));
+    bulk_g2s(s_tab, net.blob, tab_bytes, bar);
+    if (bulk_ok) bulk_g2s(s_rec, g_rec, rec_bytes, bar);
+  }
+  return bulk_ok;
+}
+/* 2. the records by word copies when they could not ride the bulk load, then wait for the tables (and records) */
+__device__ __forceinline__ void load_block_finish(bool bulk_ok, uint32_t* s_rec, const uint32_t* g_rec, int n_words, uint64_t* bar,
+                                                  int tid, int NT) {
+  if (!bulk_ok) {
+    for (int i = tid; i < n_words; i += NT) s_rec[i] = g_rec[i];
+  }
+  mbar_wait(bar, 0);
+}
+/* 3. sort the block's envs by the action type they will execute (needs only the action headers, so it overlaps the bulk
+ *    copies): a warp then runs ONE branch of the 14 defender / 3+X attacker actions.  s_perm[pos] = the env (0..nb-1)
+ *    thread pos steps; s_cnt[k + 1] ends as the end of key k's run.  keyed == false: every env has key 0 (grouped steps).
+ *    FLIP_KEYS: block / unblock envs go to keys 32..47 by listed-device count, longest first (phase B of the plain kernel
+ *    runs them in that order).  row_of(env) = the env's row of hdr_t / bl_t.  s_cnt[0..CYG_NKEYS] must be zero. */
+template <int W, bool FLIP_KEYS, class RowOf>
+__device__ __forceinline__ void sort_block(const Net& net, const uint32_t* hdr_t, const uint8_t* bl_t, bool keyed, RowOf row_of,
+                                           int env0, int nb, uint32_t* s_cnt, uint16_t* s_perm, int tid) {
+  int key = 0;
+  if (tid < nb) {
+    if (keyed) {
+      const size_t r0 = row_of(env0 + tid);
+      const uint4 hv = *reinterpret_cast<const uint4*>(hdr_t + r0 * 4);
+      const uint32_t h0 = hv.x;
+      const int blk = bl_t ? (int)bl_t[r0] : net.cfg.base_line;
+      const int xt = Env<W, 1>::exec_type(net.cfg, h0, blk) & 15;
+      key = (int)(((h0 >> 8) & 1u) << 4) | xt;
+      if (FLIP_KEYS && (key == 6 || key == 9)) { /* longest-processing-time first: 8 buckets of 16 listed devices */
+        int nd = (int)(hv.z & 0xFFFFu);
+        nd = nd < 0 ? 0 : (nd > 127 ? 127 : nd);
+        key = CYG_KEY_FLIP0 + 2 * (7 - (nd >> 4)) + (key == 9 ? 1 : 0);
+      }
+    }
+    atomicAdd(&s_cnt[key + 1], 1u);
+  }
+  __syncthreads();
+  if (tid < 32) { /* exclusive prefix over the keys (count of key k sits in s_cnt[k + 1]): one warp, two keys per lane */
+    static_assert(CYG_NKEYS > 32 && CYG_NKEYS <= 64, "two keys per lane");
+    const uint32_t c0 = s_cnt[1 + tid];
+    const uint32_t c1 = tid < CYG_NKEYS - 32 ? s_cnt[33 + tid] : 0u;
+    uint32_t x0 = c0, x1 = c1;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const uint32_t y0 = __shfl_up_sync(0xFFFFFFFFu, x0, d), y1 = __shfl_up_sync(0xFFFFFFFFu, x1, d);
+      if (tid >= d) { x0 += y0; x1 += y1; }
+    }
+    const uint32_t total0 = __shfl_sync(0xFFFFFFFFu, x0, 31);
+    s_cnt[1 + tid] = x0 - c0;
+    if (tid < CYG_NKEYS - 32) s_cnt[33 + tid] = total0 + x1 - c1;
+  }
+  __syncthreads();
+  if (tid < nb) {
+    uint32_t pos = atomicAdd(&s_cnt[key + 1], 1u);
+    s_perm[pos] = (uint16_t)tid;
+  }
+}
+
 /* shared-memory carve-up for a CTA of NB envs (all offsets 16-byte aligned; tables first, at word 0) */
 struct SmemPlan {
   size_t off_tables, off_recs, off_out, off_perm, off_cnt, off_def, off_bar, total;
@@ -229,16 +295,16 @@ __host__ __device__ inline SmemPlan smem_plan(uint32_t hot_words, int S, int NB)
 #define CYG_WARP_MARK(i) do { } while (0)
 #endif
 
-/* PLAIN: one ungrouped action per env, device lists as sets (no order array) -- the hot form: thread-per-env phases
- * A / C plus the warp-per-env phase B.  !PLAIN: grouped steps and explicit order lists, everything thread-per-env
- * (the sequential forms of every action live only in this instantiation). */
+/* The plain step: one ungrouped action per env, device lists as sets (no order array) -- the hot form: thread-per-env
+ * phases A / C plus the warp-per-env phase B, T steps fused per launch.  Grouped steps and explicit order lists run in
+ * cyg_step_seq_kernel (the sequential forms of every action live only there). */
 /* ROLL: the cyg_rollout form of the plain kernel -- action rows shared by runs of envs, raw rewards summed per env.  A
  * separate instantiation: compiled into the step kernel proper, the row indexing and the accumulation cost it 4.5 us per
  * step (registers) although no step ever takes those branches. */
 /* LOG: the env keeps a hop-log ring and may hold a trained detector (cfg.log_cap > 0): the lateral-movement scan writes
  * its hops, scans consult the detector.  Also its own instantiation (the handles that keep only the log's length --
  * every throughput run -- take the kernel without that code: ~1 us per step). */
-template <int W, bool PLAIN, bool ROLL = false, bool LOG = true>
+template <int W, bool ROLL, bool LOG>
 __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(const __grid_constant__ StepParams p) {
   unsigned char* smem = reinterpret_cast<unsigned char*>(cyg_smem);
   const int NB = p.block_envs, NT = blockDim.x, tid = threadIdx.x; /* NB envs, NT >= NB threads */
@@ -256,25 +322,15 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
   uint32_t* s_cnt = (uint32_t*)(smem + sp.off_cnt);
   uint32_t* s_def = (uint32_t*)(smem + sp.off_def);
   uint64_t* bar = (uint64_t*)(smem + sp.off_bar);
-  const bool grouped = PLAIN ? false : (p.flags & CYG_STEP_GROUPED) != 0;
 
   uint32_t* g_rec = p.recs + (size_t)env0 * S;
-  const uint32_t rec_bytes = (uint32_t)nb * S * 4u;
-  const uint32_t tab_bytes = p.net.hot_words * 4u;
-  const bool bulk_ok = (rec_bytes & 15u) == 0 && ((((size_t)g_rec) & 15) == 0);
-
-  if (tid == 0) {
-    mbar_init(bar, 1);
-    mbar_expect_tx(bar, tab_bytes + (bulk_ok ? rec_bytes : 0u));
-    bulk_g2s(s_tab, p.net.blob, tab_bytes, bar);
-    if (bulk_ok) bulk_g2s(s_rec, g_rec, rec_bytes, bar);
-  }
-  const int T = PLAIN ? (p.T < 1 ? 1 : p.T) : 1;
+  const bool bulk_ok = load_block_start(p.net, s_tab, s_rec, g_rec, nb, S, bar, tid);
+  const int T = p.T < 1 ? 1 : p.T;
   const int lane = tid & 31;
   for (int t = 0; t < T; t++) { /* the steps fused into this launch; the records stay in shared memory */
   const bool last = t == T - 1;
-  const uint32_t* hdr_t = p.hdr + (size_t)t * (ROLL ? p.n_rows : p.B) * 4 * (PLAIN ? 1 : 0);
-  const uint32_t* mask_t = p.mask + (size_t)t * (ROLL ? p.n_rows : p.B) * W * (PLAIN ? 1 : 0);
+  const uint32_t* hdr_t = p.hdr + (size_t)t * (ROLL ? p.n_rows : p.B) * 4;
+  const uint32_t* mask_t = p.mask + (size_t)t * (ROLL ? p.n_rows : p.B) * W;
   float* raw_t = p.raw + (size_t)t * p.B;
   float* shaped_t = p.shaped + (size_t)t * p.B;
   int32_t* done_t = p.done + (size_t)t * p.B;
@@ -291,59 +347,15 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
     if constexpr (ROLL) return (size_t)(((uint32_t)p.row_base + idx_of(env_i)) / (uint32_t)p.envs_per_row);
     else return (size_t)env_i;
   };
-  if (PLAIN && !ROLL && !last && tid < nb) { /* the next step's action rows of this block: into L2 while this step runs */
+  if (!ROLL && !last && tid < nb) { /* the next step's action rows of this block: into L2 while this step runs */
     asm volatile("prefetch.global.L2 [%0];" ::"l"(hdr_t + ((size_t)p.B + env0 + tid) * 4));
     asm volatile("prefetch.global.L2 [%0];" ::"l"(mask_t + ((size_t)p.B + env0 + tid) * W));
   }
   for (int i = tid; i < CYG_NKEYS + 7; i += NT) s_cnt[i] = 0; /* ... + one "past pass 0" flag per owning warp */
   __syncthreads(); /* mbarrier initialised, counters zeroed (t > 0: the previous step is complete) */
   CYG_CTA_MARK(1);
-
-  /* ---- sort the block's envs by the action type they will execute (needs only the action headers, so it
-   *      overlaps the bulk copies): a warp then runs ONE branch of the 14 defender / 3+X attacker actions ---- */
-  int key = 0;
-  if (tid < nb) {
-    if (!grouped) {
-      const size_t r0 = arow(env0 + tid);
-      const uint4 hv = *reinterpret_cast<const uint4*>(hdr_t + r0 * 4);
-      const uint32_t h0 = hv.x;
-      const int blk = bl_t ? (int)bl_t[r0] : p.net.cfg.base_line;
-      const int xt = Env<W, 1>::exec_type(p.net.cfg, h0, blk) & 15;
-      key = (int)(((h0 >> 8) & 1u) << 4) | xt;
-      if (PLAIN && (key == 6 || key == 9)) { /* longest-processing-time first: 8 buckets of 16 listed devices */
-        int nd = (int)(hv.z & 0xFFFFu);
-        nd = nd < 0 ? 0 : (nd > 127 ? 127 : nd);
-        key = CYG_KEY_FLIP0 + 2 * (7 - (nd >> 4)) + (key == 9 ? 1 : 0);
-      }
-    }
-    atomicAdd(&s_cnt[key + 1], 1u);
-  }
-  __syncthreads();
-  if (tid < 32) { /* exclusive prefix over the keys (count of key k sits in s_cnt[k + 1]): one warp, two keys per lane */
-    static_assert(CYG_NKEYS > 32 && CYG_NKEYS <= 64, "two keys per lane");
-    const uint32_t c0 = s_cnt[1 + tid];
-    const uint32_t c1 = tid < CYG_NKEYS - 32 ? s_cnt[33 + tid] : 0u;
-    uint32_t x0 = c0, x1 = c1;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t y0 = __shfl_up_sync(0xFFFFFFFFu, x0, d), y1 = __shfl_up_sync(0xFFFFFFFFu, x1, d);
-      if (tid >= d) { x0 += y0; x1 += y1; }
-    }
-    const uint32_t total0 = __shfl_sync(0xFFFFFFFFu, x0, 31);
-    s_cnt[1 + tid] = x0 - c0;
-    if (tid < CYG_NKEYS - 32) s_cnt[33 + tid] = total0 + x1 - c1;
-  }
-  __syncthreads();
-  if (tid < nb) {
-    uint32_t pos = atomicAdd(&s_cnt[key + 1], 1u);
-    s_perm[pos] = (uint16_t)tid;
-  }
-  if (t == 0) {
-    if (!bulk_ok) {
-      for (int i = tid; i < nb * S; i += NT) s_rec[i] = g_rec[i];
-    }
-    mbar_wait(bar, 0);
-  }
+  sort_block<W, true>(p.net, hdr_t, bl_t, true, arow, env0, nb, s_cnt, s_perm, tid);
+  if (t == 0) load_block_finish(bulk_ok, s_rec, g_rec, nb * S, bar, tid, NT);
   __syncthreads();
   CYG_CTA_MARK(2);
 
@@ -354,7 +366,6 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
    *      pass 1  phase B, warp per env, then the rest of the step (step_post) of those envs by their own threads.
    *      After either pass a warp sends the records its threads finished home (one warp-wide copy per record), so the
    *      write-back of the ~2/3 of the block that phase A completes drains under phase B. ---- */
-  constexpr bool coop_ok = PLAIN;
   const bool lower = (tid & ~31) < nb; /* warps that own envs in the thread-per-env phases */
   bool deferred = false;
   const int el = tid < nb ? (int)s_perm[tid] : 0, env = env0 + el;
@@ -385,12 +396,11 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
     }
   };
 #pragma unroll /* two copies of the thread-per-env code: un-unrolled, ptxas spills inside the warp-per-env routines (measured slower) */
-  for (int pass = 0; pass < (PLAIN ? 2 : 1); pass++) {
+  for (int pass = 0; pass < 2; pass++) {
     double cost = 0.0;
     bool dirty = false, do_post = false;
     if (pass == 0) {
       uint32_t act[4 + W]; /* this env's action (group 0), in registers */
-      const uint16_t* ord = (!PLAIN && p.order) ? p.order + (size_t)env * p.order_stride : nullptr;
       int atype = 0;
       if (tid < nb) {
         uint4 hv = *reinterpret_cast<const uint4*>(hdr_t + my_row * 4);
@@ -401,107 +411,100 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
         mode = (int)((act[0] >> 8) & 1u);
         if (bl_t) e.bl = (int)bl_t[my_row];
         atype = e.step_pre(act, p.flags);
-        deferred = coop_ok && Coop<W>::is_heavy(e, mode, atype) && !(mode == CYG_MODE_ATTACKER && e.bl == CYG_BL_NO_ATTACK);
+        deferred = Coop<W>::is_heavy(e, mode, atype) && !(mode == CYG_MODE_ATTACKER && e.bl == CYG_BL_NO_ATTACK);
       }
-      if (coop_ok) {
-        /* once every env has its epoch open and its busy tick done (s_cnt[CYG_NKEYS + 6] counts the owning warps that
-         * got there) phase B may touch any deferred env: the warps that own no env start it right away, the owning
-         * warps join after their thread-per-env work -- and check the same counter, a warp whose envs are all deferred
-         * gets to phase B before the others are through step_pre */
-        const uint32_t dmask = __ballot_sync(0xFFFFFFFFu, deferred);
-        if (lower) {
-          __syncwarp();
-          if (lane == 0) { s_def[tid >> 5] = dmask; __threadfence_block(); atomicAdd(&s_cnt[CYG_NKEYS + 6], 1u); }
-        }
+      /* once every env has its epoch open and its busy tick done (s_cnt[CYG_NKEYS + 6] counts the owning warps that
+       * got there) phase B may touch any deferred env: the warps that own no env start it right away, the owning
+       * warps join after their thread-per-env work -- and check the same counter, a warp whose envs are all deferred
+       * gets to phase B before the others are through step_pre */
+      const uint32_t dmask = __ballot_sync(0xFFFFFFFFu, deferred);
+      if (lower) {
+        __syncwarp();
+        if (lane == 0) { s_def[tid >> 5] = dmask; __threadfence_block(); atomicAdd(&s_cnt[CYG_NKEYS + 6], 1u); }
       }
       if (tid < nb && !deferred) {
-        if (PLAIN) e.template step_act<true>(act, act + 4, nullptr, 0, 0, 0, 1, p.flags, atype, cost, dirty);
-        else if (!grouped) e.step_act(act, act + 4, ord, 0, 0, 0, 1, p.flags, atype, cost, dirty);
-        else e.step_act(hdr_t + (size_t)env * 4, mask_t + (size_t)env * W, ord, (size_t)p.B * 4, (size_t)p.B * W,
-                        (size_t)p.B * p.order_stride, p.G, p.flags, atype, cost, dirty);
+        e.template step_act<true>(act, act + 4, nullptr, 0, 0, 0, 1, p.flags, atype, cost, dirty);
         do_post = true;
       }
     } else {
-      if constexpr (PLAIN) {
   CYG_CTA_MARK(3);
-        if (lane == 0) while (atomicAdd(&s_cnt[CYG_NKEYS + 6], 0u) < (uint32_t)((nb + 31) >> 5)) __nanosleep(32);
-        __syncwarp();
-        auto load_action = [&](size_t row_b, uint32_t* act) {
-          const uint4 hv = __ldg(reinterpret_cast<const uint4*>(hdr_t + row_b * 4)); /* phase A read these lines: L1 */
-          act[0] = hv.x; act[1] = hv.y; act[2] = hv.z; act[3] = hv.w;
+      if (lane == 0) while (atomicAdd(&s_cnt[CYG_NKEYS + 6], 0u) < (uint32_t)((nb + 31) >> 5)) __nanosleep(32);
+      __syncwarp();
+      auto load_action = [&](size_t row_b, uint32_t* act) {
+        const uint4 hv = __ldg(reinterpret_cast<const uint4*>(hdr_t + row_b * 4)); /* phase A read these lines: L1 */
+        act[0] = hv.x; act[1] = hv.y; act[2] = hv.z; act[3] = hv.w;
 #pragma unroll
-          for (int w = 0; w < W; w++) act[4 + w] = __ldg(mask_t + row_b * W + w);
-        };
-        /* B1: block / unblock (keys 6, 9; the longest lists first), B2: attacker exploit + lateral movement (key 16|1),
-         * B3: clean / revert / upgrade (keys 1, 3, 4).  One env per warp; perm[] holds each kind as a contiguous run. */
+        for (int w = 0; w < W; w++) act[4 + w] = __ldg(mask_t + row_b * W + w);
+      };
+      /* B1: block / unblock (keys 6, 9; the longest lists first), B2: attacker exploit + lateral movement (key 16|1),
+       * B3: clean / revert / upgrade (keys 1, 3, 4).  One env per warp; perm[] holds each kind as a contiguous run. */
 #pragma unroll
-        for (int kind = 0; kind < 3; kind++) {
-          int lo0, n0, lo1 = 0, n1 = 0, lo2 = 0, n2 = 0;
-          if (kind == 0) { lo0 = (int)s_cnt[CYG_KEY_FLIP0]; n0 = (int)s_cnt[CYG_NKEYS] - lo0; }
-          else if (kind == 1) { lo0 = (int)s_cnt[17]; n0 = (int)s_cnt[18] - lo0; }
-          else {
-            lo0 = (int)s_cnt[1]; n0 = (int)s_cnt[2] - lo0; lo1 = (int)s_cnt[3]; n1 = (int)s_cnt[4] - lo1;
-            lo2 = (int)s_cnt[4]; n2 = (int)s_cnt[5] - lo2;
+      for (int kind = 0; kind < 3; kind++) {
+        int lo0, n0, lo1 = 0, n1 = 0, lo2 = 0, n2 = 0;
+        if (kind == 0) { lo0 = (int)s_cnt[CYG_KEY_FLIP0]; n0 = (int)s_cnt[CYG_NKEYS] - lo0; }
+        else if (kind == 1) { lo0 = (int)s_cnt[17]; n0 = (int)s_cnt[18] - lo0; }
+        else {
+          lo0 = (int)s_cnt[1]; n0 = (int)s_cnt[2] - lo0; lo1 = (int)s_cnt[3]; n1 = (int)s_cnt[4] - lo1;
+          lo2 = (int)s_cnt[4]; n2 = (int)s_cnt[5] - lo2;
+        }
+        const int ntasks = n0 + n1 + n2;
+        for (;;) {
+          int task = 0;
+          if (lane == 0) task = (int)atomicAdd(&s_cnt[CYG_NKEYS + 1 + kind], 1u);
+          task = __shfl_sync(0xFFFFFFFFu, task, 0);
+          if (task >= ntasks) break;
+          const int ppos = task < n0 ? lo0 + task : (task < n0 + n1 ? lo1 + task - n0 : lo2 + task - n0 - n1);
+          if (!((s_def[ppos >> 5] >> (ppos & 31)) & 1u)) continue; /* its own thread did it in phase A */
+          const int el_b = s_perm[ppos];
+          const int env_b = env0 + el_b;
+          Env<W, 1> eb(&p.net, nullptr, p.ckpt + (size_t)env_b * M, p.xtra + (size_t)env_b * p.net.cfg.xcap,
+                          (uint32_t)p.env_id0 + idx_of(env_b), (uint32_t)(sp.off_recs / 4) + (uint32_t)(el_b * S), (uint32_t)(sp.off_tables / 4));
+          const size_t row_b = arow(env_b);
+          eb.resume_epoch();
+          if (LOG && kind == 1) eb.logs = p.logs ? p.logs + (size_t)env_b * p.net.cfg.log_cap : nullptr; /* the attack logs its hops */
+          uint32_t act[4 + W];
+          load_action(row_b, act);
+          typename Env<W, 1>::Act a;
+          Env<W, 1>::decode(act, act + 4, nullptr, a);
+          double tcost = 0.0;
+          bool tdirty = false;
+          long long tb0 = p.dbg_cycles ? clock64() : 0;
+          if (lane == 0) eb.load_costs();
+          if (kind == 0) {
+            Coop<W>::template flip<32>(eb, a, (int)(act[0] & 0xFFu), tcost, tdirty); /* flip keys only hold executed types 6 / 9 == the header's */
+          } else if (kind == 1) {
+            Coop<W>::template attack<LOG>(eb, a);
+          } else {
+            const int atype_b = Env<W, 1>::exec_type(p.net.cfg, act[0], bl_t ? (int)bl_t[row_b] : p.net.cfg.base_line);
+            Coop<W>::defender(eb, a, atype_b, tcost, tdirty);
           }
-          const int ntasks = n0 + n1 + n2;
-          for (;;) {
-            int task = 0;
-            if (lane == 0) task = (int)atomicAdd(&s_cnt[CYG_NKEYS + 1 + kind], 1u);
-            task = __shfl_sync(0xFFFFFFFFu, task, 0);
-            if (task >= ntasks) break;
-            const int ppos = task < n0 ? lo0 + task : (task < n0 + n1 ? lo1 + task - n0 : lo2 + task - n0 - n1);
-            if (!((s_def[ppos >> 5] >> (ppos & 31)) & 1u)) continue; /* its own thread did it in phase A */
-            const int el_b = s_perm[ppos];
-            const int env_b = env0 + el_b;
-            Env<W, 1> eb(&p.net, nullptr, p.ckpt + (size_t)env_b * M, p.xtra + (size_t)env_b * p.net.cfg.xcap,
-                            (uint32_t)p.env_id0 + idx_of(env_b), (uint32_t)(sp.off_recs / 4) + (uint32_t)(el_b * S), (uint32_t)(sp.off_tables / 4));
-            const size_t row_b = arow(env_b);
-            eb.resume_epoch();
-            if (LOG && kind == 1) eb.logs = p.logs ? p.logs + (size_t)env_b * p.net.cfg.log_cap : nullptr; /* the attack logs its hops */
-            uint32_t act[4 + W];
-            load_action(row_b, act);
-            typename Env<W, 1>::Act a;
-            Env<W, 1>::decode(act, act + 4, nullptr, a);
-            double tcost = 0.0;
-            bool tdirty = false;
-            long long tb0 = p.dbg_cycles ? clock64() : 0;
-            if (lane == 0) eb.load_costs();
-            if (kind == 0) {
-              Coop<W>::template flip<32>(eb, a, (int)(act[0] & 0xFFu), tcost, tdirty); /* flip keys only hold executed types 6 / 9 == the header's */
-            } else if (kind == 1) {
-              Coop<W>::template attack<LOG>(eb, a);
-            } else {
-              const int atype_b = Env<W, 1>::exec_type(p.net.cfg, act[0], bl_t ? (int)bl_t[row_b] : p.net.cfg.base_line);
-              Coop<W>::defender(eb, a, atype_b, tcost, tdirty);
-            }
-            if (lane == 0) {
+          if (lane == 0) {
 #if !defined(CYG_PHASE_TIMING) && !defined(CYG_CTA_TIMING)
-              if (p.dbg_cycles) p.dbg_cycles[env_b] = (unsigned long long)(clock64() - tb0); /* heavy envs: phase-B cycles */
+            if (p.dbg_cycles) p.dbg_cycles[env_b] = (unsigned long long)(clock64() - tb0); /* heavy envs: phase-B cycles */
 #endif
 #ifdef CYG_COUNT_ROUNDS
-              if (p.dbg_cycles && kind == 0) p.dbg_cycles[env_b] = (unsigned long long)eb.dbg_rounds;
+            if (p.dbg_cycles && kind == 0) p.dbg_cycles[env_b] = (unsigned long long)eb.dbg_rounds;
 #endif
-              eb.store_costs();
-              s_out[el_b] = (float)tcost;
-              s_out[NB + el_b] = __int_as_float(tdirty ? 1 : 0);
-            }
-            __syncwarp();
+            eb.store_costs();
+            s_out[el_b] = (float)tcost;
+            s_out[NB + el_b] = __int_as_float(tdirty ? 1 : 0);
           }
-          CYG_WARP_MARK(kind);
+          __syncwarp();
         }
-        __syncthreads();
+        CYG_WARP_MARK(kind);
+      }
+      __syncthreads();
   CYG_CTA_MARK(4);
-        /* ---- phase C, thread per env again: the rest of the step for the envs phase B handled ---- */
-        if (deferred) {
-          e = Env<W, 1>(&p.net, nullptr, p.ckpt + (size_t)env * M, p.xtra + (size_t)env * p.net.cfg.xcap, (uint32_t)p.env_id0 + idx_of(env),
-                           (uint32_t)(sp.off_recs / 4) + (uint32_t)(el * S), (uint32_t)(sp.off_tables / 4)); /* nothing of it stays live across phase B */
-          if (bl_t) e.bl = (int)bl_t[my_row];
-          bind_aux(e, env);
-          e.resume_epoch();
-          cost = (double)s_out[el];
-          dirty = __float_as_int(s_out[NB + el]) != 0;
-          do_post = true;
-        }
+      /* ---- phase C, thread per env again: the rest of the step for the envs phase B handled ---- */
+      if (deferred) {
+        e = Env<W, 1>(&p.net, nullptr, p.ckpt + (size_t)env * M, p.xtra + (size_t)env * p.net.cfg.xcap, (uint32_t)p.env_id0 + idx_of(env),
+                      (uint32_t)(sp.off_recs / 4) + (uint32_t)(el * S), (uint32_t)(sp.off_tables / 4)); /* nothing of it stays live across phase B */
+        if (bl_t) e.bl = (int)bl_t[my_row];
+        bind_aux(e, env);
+        e.resume_epoch();
+        cost = (double)s_out[el];
+        dirty = __float_as_int(s_out[NB + el]) != 0;
+        do_post = true;
       }
     }
     if (do_post) {
@@ -518,7 +521,7 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
       if (p.dbg_cycles && !deferred) p.dbg_cycles[env] = (unsigned long long)(clock64() - t_begin);
 #endif
     }
-    if (PLAIN && last && lower) {
+    if (last && lower) {
       /* The records this warp's threads just finished go home by warp-wide copies, right away.  Measured alternatives:
        * 4 records after each phase-B task of the warp (38.3 / 50.5 us fused / single against 37.8 / 48.1), a shared
        * claim counter with 4 records per claim (37.8 / 49.5), ONE warp copying for the whole block (45.1 / 67.5: a
@@ -537,13 +540,91 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
     const int dim = p.obs_mode == 2 ? 4 * M + p.net.cfg.X : 6 * M;
     observe_rows<W>(p.net, s_rec, S, nb, p.obs_mode, p.obs + (size_t)env0 * dim, tid >> 5, NT >> 5, lane);
   }
+  CYG_CTA_MARK(6); /* every warp sent its records home already */
+}
 
-  /* ---- write the block's records back ---- */
-  if constexpr (PLAIN) { /* every warp sent its records home already */
-    CYG_CTA_MARK(6);
-  } else
-#ifdef CYG_TMA_STORE
-  if (bulk_ok) { /* one bulk store; every writer fences generic -> async proxy first */
+/* Grouped steps (CYG_STEP_GROUPED: G action groups per env) and explicit order lists: one step per launch, thread per env
+ * over the same staged records, sorted envs and shared-memory plan as cyg_step_kernel, then the block goes back with one
+ * bulk store. */
+template <int W>
+__global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_seq_kernel(const __grid_constant__ StepParams p) {
+  unsigned char* smem = reinterpret_cast<unsigned char*>(cyg_smem);
+  const int NB = p.block_envs, NT = blockDim.x, tid = threadIdx.x;
+  CYG_CTA_MARK(0);
+  const int S = p.net.S, M = p.net.M;
+  const int env0 = (int)blockIdx.x * NB;
+  const int nb = min(NB, p.B - env0);
+  const SmemPlan sp = smem_plan(p.net.hot_words, S, NB);
+  uint32_t* s_tab = (uint32_t*)(smem + sp.off_tables);
+  uint32_t* s_rec = (uint32_t*)(smem + sp.off_recs);
+  uint16_t* s_perm = (uint16_t*)(smem + sp.off_perm);
+  uint32_t* s_cnt = (uint32_t*)(smem + sp.off_cnt);
+  uint64_t* bar = (uint64_t*)(smem + sp.off_bar);
+  const bool grouped = (p.flags & CYG_STEP_GROUPED) != 0;
+
+  uint32_t* g_rec = p.recs + (size_t)env0 * S;
+  const uint32_t rec_bytes = (uint32_t)nb * S * 4u;
+  const bool bulk_ok = load_block_start(p.net, s_tab, s_rec, g_rec, nb, S, bar, tid);
+  const int lane = tid & 31;
+  for (int i = tid; i < CYG_NKEYS + 7; i += NT) s_cnt[i] = 0;
+  __syncthreads(); /* mbarrier initialised, counters zeroed */
+  CYG_CTA_MARK(1);
+  sort_block<W, false>(p.net, p.hdr, p.bl_env, !grouped, [](int env_i) { return (size_t)env_i; }, env0, nb, s_cnt, s_perm, tid);
+  load_block_finish(bulk_ok, s_rec, g_rec, nb * S, bar, tid, NT);
+  __syncthreads();
+  CYG_CTA_MARK(2);
+
+  const int el = tid < nb ? (int)s_perm[tid] : 0, env = env0 + el;
+  Env<W, 1> e(&p.net, nullptr, p.ckpt + (size_t)env * M, p.xtra + (size_t)env * p.net.cfg.xcap, (uint32_t)p.env_id0 + (uint32_t)env,
+              (uint32_t)(sp.off_recs / 4) + (uint32_t)(el * S), (uint32_t)(sp.off_tables / 4));
+  if (tid < nb) { /* the hop-log ring and the uploaded detector (both optional, global memory) */
+    e.logs = p.logs ? p.logs + (size_t)env * p.net.cfg.log_cap : nullptr;
+    e.det = (p.det_slots && p.det_of_env[env] >= 0) ? p.det_slots + (size_t)p.det_of_env[env] * CYG_DET_WORDS : nullptr;
+  }
+  long long t_begin = 0;
+#ifdef CYG_PHASE_TIMING
+  long long ph[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  e.phase_t = ph;
+#endif
+  double cost = 0.0;
+  bool dirty = false;
+  uint32_t act[4 + W]; /* this env's action (group 0), in registers */
+  const uint16_t* ord = p.order ? p.order + (size_t)env * p.order_stride : nullptr;
+  if (tid < nb) {
+    uint4 hv = *reinterpret_cast<const uint4*>(p.hdr + (size_t)env * 4);
+    act[0] = hv.x; act[1] = hv.y; act[2] = hv.z; act[3] = hv.w;
+#pragma unroll
+    for (int w = 0; w < W; w++) act[4 + w] = p.mask[(size_t)env * W + w];
+    t_begin = p.dbg_cycles ? clock64() : 0;
+    const int mode = (int)((act[0] >> 8) & 1u);
+    if (p.bl_env) e.bl = (int)p.bl_env[env];
+    const int atype = e.step_pre(act, p.flags);
+    if (!grouped) e.step_act(act, act + 4, ord, 0, 0, 0, 1, p.flags, atype, cost, dirty);
+    else e.step_act(p.hdr + (size_t)env * 4, p.mask + (size_t)env * W, ord, (size_t)p.B * 4, (size_t)p.B * W,
+                    (size_t)p.B * p.order_stride, p.G, p.flags, atype, cost, dirty);
+    float raw, shaped;
+    int32_t done;
+    e.step_post(mode, cost, dirty, p.flags, &raw, &shaped, &done, p.pre_masks ? p.pre_masks + (size_t)env * 3 * W : nullptr);
+    p.raw[env] = raw; p.shaped[env] = shaped; p.done[env] = done;
+#ifdef CYG_PHASE_TIMING
+    if (p.dbg_cycles) for (int i = 0; i < 8; i++) p.dbg_cycles[(size_t)env * 8 + i] = (unsigned long long)(ph[i] - t_begin);
+#elif !defined(CYG_CTA_TIMING)
+    if (p.dbg_cycles) p.dbg_cycles[env] = (unsigned long long)(clock64() - t_begin);
+#endif
+  }
+  __syncthreads();
+  CYG_CTA_MARK(5);
+
+  /* ---- optional fused observation rows (post-evolve view, CyberDefenseEnv.py:146-257) ---- */
+  if (p.obs && p.obs_mode) {
+    const int dim = p.obs_mode == 2 ? 4 * M + p.net.cfg.X : 6 * M;
+    observe_rows<W>(p.net, s_rec, S, nb, p.obs_mode, p.obs + (size_t)env0 * dim, tid >> 5, NT >> 5, lane);
+  }
+
+  /* ---- write the block's records back: one bulk store (every writer fences generic -> async proxy first; plain
+   *      coalesced stores measured the same, the write-back is bound by the per-SM path to L2), word stores for a tail
+   *      block whose span is not 16-byte sized / aligned ---- */
+  if (bulk_ok) {
     fence_proxy_async();
     __syncthreads();
     CYG_CTA_MARK(6);
@@ -551,25 +632,16 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
       bulk_s2g(g_rec, s_rec, rec_bytes);
       bulk_commit_wait_read();
     }
-  } else
-#endif
-  {
-    /* coalesced 16-byte stores by all warps (tail blocks whose span is not 16-byte sized / aligned) */
-    if (bulk_ok) {
-      const uint4* s4 = reinterpret_cast<const uint4*>(s_rec);
-      uint4* g4 = reinterpret_cast<uint4*>(g_rec);
-      const int n4 = (int)(rec_bytes >> 4);
-      for (int i = tid; i < n4; i += NT) g4[i] = s4[i];
-    } else {
-      for (int i = tid; i < nb * S; i += NT) g_rec[i] = s_rec[i];
-    }
+  } else {
+    for (int i = tid; i < nb * S; i += NT) g_rec[i] = s_rec[i];
     CYG_CTA_MARK(6);
   }
 }
 
 /* ---- large networks (128 < M <= 2048, BASELINE.json config C4): the adjacency bit matrix (M x 64 words) exceeds
- *      shared memory, so this first correct path steps one env per thread straight on the records in global
- *      memory with the tables read through L2.  Same transition code (cyg_core.cuh), no staging, no sort. ---- */
+ *      shared memory, so it stays in global memory and is read through L2; the records and the other hot tables are
+ *      staged in shared memory.  Same transition code (cyg_core.cuh), every step form, a warp-per-env phase B for
+ *      the heavy actions of plain steps, no sort. ---- */
 template <int W>
 __global__ void __launch_bounds__(256) cyg_step_generic_kernel(const __grid_constant__ StepParams p) {
   /* block_envs envs per CTA, spread over all SMs (B = 1024 -> 7 per CTA); their records (~6.4 KB each at M = 2000) are
@@ -1070,28 +1142,28 @@ template <int KW>
 struct WImpl {
   static cudaError_t set_smem_optin(int max_optin) {
     if constexpr (KW <= CYG_MAX_W) {
-      cudaError_t e = cudaFuncSetAttribute(cyg_step_kernel<KW, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
+      cudaError_t e = cudaFuncSetAttribute(cyg_step_kernel<KW, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
       if (e != cudaSuccess) return e;
-      e = cudaFuncSetAttribute(cyg_step_kernel<KW, true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
+      e = cudaFuncSetAttribute(cyg_step_kernel<KW, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
       if (e != cudaSuccess) return e;
-      e = cudaFuncSetAttribute(cyg_step_kernel<KW, true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
+      e = cudaFuncSetAttribute(cyg_step_kernel<KW, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
       if (e != cudaSuccess) return e;
-      return cudaFuncSetAttribute(cyg_step_kernel<KW, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
+      return cudaFuncSetAttribute(cyg_step_seq_kernel<KW>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
     } else {
       return cudaFuncSetAttribute(cyg_step_generic_kernel<KW>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
     }
   }
   static void step(bool plain, int blocks, int threads, size_t smem, cudaStream_t st, const StepParams& p) {
     if constexpr (KW <= CYG_MAX_W) {
-      if (plain && !p.logs) cyg_step_kernel<KW, true, false, false><<<blocks, threads, smem, st>>>(p);
-      else if (plain) cyg_step_kernel<KW, true><<<blocks, threads, smem, st>>>(p);
-      else cyg_step_kernel<KW, false><<<blocks, threads, smem, st>>>(p);
+      if (!plain) cyg_step_seq_kernel<KW><<<blocks, threads, smem, st>>>(p);
+      else if (!p.logs) cyg_step_kernel<KW, false, false><<<blocks, threads, smem, st>>>(p);
+      else cyg_step_kernel<KW, false, true><<<blocks, threads, smem, st>>>(p);
     } else {
       cyg_step_generic_kernel<KW><<<blocks, threads, smem, st>>>(p);
     }
   }
   static void rollout(int blocks, int threads, size_t smem, cudaStream_t st, const StepParams& p) {
-    if constexpr (KW <= CYG_MAX_W) cyg_step_kernel<KW, true, true, false><<<blocks, threads, smem, st>>>(p);
+    if constexpr (KW <= CYG_MAX_W) cyg_step_kernel<KW, true, false><<<blocks, threads, smem, st>>>(p);
   }
   static void import_state(int blocks, int threads, cudaStream_t st, const ConvParams& p) { cyg_import_kernel<KW><<<blocks, threads, 0, st>>>(p); }
   static void export_state(int blocks, int threads, cudaStream_t st, const ConvParams& p) { cyg_export_kernel<KW><<<blocks, threads, 0, st>>>(p); }
@@ -1372,6 +1444,29 @@ int cyg_export_state(cyg_handle h, const cyg_state* c, void* stream) {
   return CYG_OK;
 }
 
+/* the fields of a step launch that come from the handle alone; every other field is zero */
+static StepParams step_params(cyg_handle h) {
+  StepParams p{};
+  p.net = h->net;
+  p.recs = h->state; p.ckpt = ckpt_of(h); p.xtra = xtra_of(h); p.logs = logs_of(h);
+  p.det_slots = h->det_slots; p.det_of_env = h->det_of_env;
+  p.B = h->B; p.env_id0 = h->env_id0; p.block_envs = h->NB;
+  return p;
+}
+
+/* one CTA per block of NB envs; the shared-memory kernels run 2 threads per env up to CYG_MAX_BLOCK_THREADS (never fewer
+ * than one per env), the generic kernel 256 */
+struct StepGrid { int blocks, threads; };
+static StepGrid step_grid(cyg_handle h) {
+  StepGrid g;
+  g.blocks = (h->B + h->NB - 1) / h->NB;
+  if (h->W > CYG_MAX_W) { g.threads = 256; return g; }
+  g.threads = ((2 * h->NB + 31) / 32) * 32;
+  if (g.threads > CYG_MAX_BLOCK_THREADS) g.threads = CYG_MAX_BLOCK_THREADS;
+  if (g.threads < h->NB) g.threads = ((h->NB + 31) / 32) * 32;
+  return g;
+}
+
 static int step_impl(cyg_handle h, const cyg_actions* a, int n_steps, uint32_t step_flags, const cyg_step_out* out, void* stream);
 
 int cyg_step(cyg_handle h, const cyg_actions* a, uint32_t step_flags, const cyg_step_out* out, void* stream) {
@@ -1401,36 +1496,22 @@ static int step_impl(cyg_handle h, const cyg_actions* a, int n_steps, uint32_t s
   if (out->obs && (out->obs_mode < 1 || out->obs_mode > 3)) return fail(CYG_E_INVAL, "obs_mode must be 1..3 when obs is given");
   if (((uintptr_t)a->hdr) & 15) return fail(CYG_E_INVAL, "hdr must be 16-byte aligned");
   DeviceGuard g(h->device);
-  StepParams p;
-  p.net = h->net;
-  p.recs = h->state; p.ckpt = ckpt_of(h); p.xtra = xtra_of(h);
+  StepParams p = step_params(h);
   p.hdr = a->hdr; p.mask = a->mask; p.order = a->order;
   p.raw = out->raw_reward; p.shaped = out->shaped_reward; p.done = out->done;
   p.pre_masks = out->pre_masks; p.obs = out->obs; p.dbg_cycles = h->dbg_cycles; p.bl_env = h->bl_env; p.bl_stride = (h->bl_env && h->bl_rows > 1) ? h->B : 0;
-  p.B = h->B; p.env_id0 = h->env_id0; p.G = a->n_groups; p.order_stride = a->order_stride;
+  p.G = a->n_groups; p.order_stride = a->order_stride;
   p.obs_mode = out->obs ? out->obs_mode : 0;
   p.flags = step_flags;
   p.T = n_steps;
-  p.row_base = 0; p.envs_per_row = 0; p.n_rows = h->B; p.ret_acc = nullptr; p.id_run = 0; p.id_stride = 0; p.block_order = nullptr;
-  p.logs = logs_of(h); p.det_slots = h->det_slots; p.det_of_env = h->det_of_env;
-  p.block_envs = h->NB;
-  const bool plain = !(step_flags & CYG_STEP_GROUPED) && a->order == nullptr; /* the hot form: see cyg_step_kernel */
-  int blocks = (h->B + h->NB - 1) / h->NB;
-  int threads = ((2 * h->NB + 31) / 32) * 32;
-  if (threads > CYG_MAX_BLOCK_THREADS) threads = CYG_MAX_BLOCK_THREADS;
-  if (threads < h->NB) threads = ((h->NB + 31) / 32) * 32;
-  if (h->W > CYG_MAX_W) {
-    wops(h->W)->step(false, (h->B + h->NB - 1) / h->NB, 256, h->smem_bytes, (cudaStream_t)stream, p);
-    if (out->obs) { /* post-evolve observation rows: a second launch on the generic path */
-      h->launches++;
-      CU(cudaGetLastError());
-      return cyg_observe(h, out->obs_mode, out->obs, stream);
-    }
-  } else {
-    wops(h->W)->step(plain, blocks, threads, h->smem_bytes, (cudaStream_t)stream, p);
-  }
+  p.n_rows = h->B;
+  const bool plain = !(step_flags & CYG_STEP_GROUPED) && a->order == nullptr; /* cyg_step_kernel; else cyg_step_seq_kernel */
+  const StepGrid grid = step_grid(h);
+  wops(h->W)->step(plain, grid.blocks, grid.threads, h->smem_bytes, (cudaStream_t)stream, p);
   h->launches++;
   CU(cudaGetLastError());
+  /* large networks: the post-evolve observation rows are a second launch */
+  if (h->W > CYG_MAX_W && out->obs) return cyg_observe(h, out->obs_mode, out->obs, stream);
   return CYG_OK;
 }
 
@@ -1445,22 +1526,14 @@ int cyg_rollout(cyg_handle h, const cyg_rollout_args* a, uint32_t step_flags, vo
   if (step_flags & CYG_STEP_GROUPED) return fail(CYG_E_INVAL, "cyg_rollout: plain steps only");
   if (((uintptr_t)a->hdr) & 15) return fail(CYG_E_INVAL, "hdr must be 16-byte aligned");
   DeviceGuard g(h->device);
-  StepParams p;
-  p.net = h->net;
-  p.recs = h->state; p.ckpt = ckpt_of(h); p.xtra = xtra_of(h);
-  p.hdr = a->hdr; p.mask = a->mask; p.order = nullptr;
-  p.raw = nullptr; p.shaped = nullptr; p.done = nullptr; p.pre_masks = nullptr; p.obs = nullptr; p.dbg_cycles = nullptr;
+  StepParams p = step_params(h);
+  p.hdr = a->hdr; p.mask = a->mask;
   p.bl_env = a->base_line; p.bl_stride = a->base_line ? a->n_rows : 0;
-  p.B = h->B; p.env_id0 = h->env_id0; p.G = 1; p.order_stride = 0; p.obs_mode = 0; p.flags = step_flags; p.T = a->n_steps;
+  p.G = 1; p.flags = step_flags; p.T = a->n_steps;
   p.row_base = a->row_base; p.envs_per_row = a->envs_per_row; p.n_rows = a->n_rows; p.ret_acc = a->returns;
   p.id_run = h->id_run; p.id_stride = h->id_stride; p.block_order = a->block_order;
-  p.logs = logs_of(h); p.det_slots = h->det_slots; p.det_of_env = h->det_of_env;
-  p.block_envs = h->NB;
-  int blocks = (h->B + h->NB - 1) / h->NB;
-  int threads = ((2 * h->NB + 31) / 32) * 32;
-  if (threads > CYG_MAX_BLOCK_THREADS) threads = CYG_MAX_BLOCK_THREADS;
-  if (threads < h->NB) threads = ((h->NB + 31) / 32) * 32;
-  wops(h->W)->rollout(blocks, threads, h->smem_bytes, (cudaStream_t)stream, p);
+  const StepGrid grid = step_grid(h);
+  wops(h->W)->rollout(grid.blocks, grid.threads, h->smem_bytes, (cudaStream_t)stream, p);
   h->launches++;
   CU(cudaGetLastError());
   return CYG_OK;

@@ -8,4 +8,4 @@ from cygym_b200 import _capi  # noqa: E402
 
 out = os.path.abspath(sys.argv[1])
 log = _capi.compile_units(out, widths=(4,), extra=["-DCYG_FAST_BUILD"] + sys.argv[2:], obj_dir=os.path.join(os.path.dirname(out), "obj"))
-print(out, "cyg_step_kernel<4, plain> spill bytes:", _capi._step_kernel_spill(log))
+print(out, "cyg_step_kernel<4, false, false> spill bytes:", _capi._step_kernel_spill(log))

@@ -33,9 +33,9 @@ cp gpurun_out/${R}_launches.csv profiles/${R}_launches.csv
 [ -f gpurun_out/${R}_exclude_sweep.txt ] && cp gpurun_out/${R}_exclude_sweep.txt profiles/${R}_exclude_sweep.txt
 [ -f gpurun_out/${R}_cta_phases.txt ] && cp gpurun_out/${R}_cta_phases.txt profiles/${R}_cta_phases.txt
 # SASS evidence: bulk (TMA) copies + mbarrier waits in the step kernel, instruction count of the plain instantiation
-cuobjdump -sass -fun '_Z15cyg_step_kernelILi4ELb1ELb0ELb0EEv10StepParams' cygym_b200/libcygym_b200.so > gpurun_out/${R}_step_kernel.sass 2>/dev/null || true
-{ echo "# cuobjdump -sass of cyg_step_kernel<4, PLAIN, no ROLL, no LOG> in cygym_b200/libcygym_b200.so (sm_100a)";
-  echo "# SASS instructions: $(grep -cE '^\s+/\*[0-9a-f]{4,}\*/' gpurun_out/${R}_step_kernel.sass)";
-  echo "# bulk-copy / mbarrier / cluster instructions:"; grep -nE 'UBLKCP|UBLKPF|SYNCS|UTMA|FENCE|ELECT' gpurun_out/${R}_step_kernel.sass | sed 's/  */ /g' | head -40;
-  echo "# opcode histogram (top 25):"; grep -oE '^\s+/\*[0-9a-f]{4,}\*/\s+(@!?U?P[0-9T] )?[A-Z0-9_.]+' gpurun_out/${R}_step_kernel.sass | awk '{print $NF}' | cut -d. -f1 | sort | uniq -c | sort -rn | head -25; } > profiles/${R}_step_kernel_sass.txt
+SASS=$(cuobjdump -sass -fun '_Z15cyg_step_kernelILi4ELb0ELb0EEv10StepParams' cygym_b200/libcygym_b200.so 2>/dev/null || true)
+{ echo "# cuobjdump -sass of cyg_step_kernel<4, no ROLL, no LOG> in cygym_b200/libcygym_b200.so (sm_100a)";
+  echo "# SASS instructions: $(grep -cE '^\s+/\*[0-9a-f]{4,}\*/' <<< "$SASS")";
+  echo "# bulk-copy / mbarrier / cluster instructions:"; grep -nE 'UBLKCP|UBLKPF|SYNCS|UTMA|FENCE|ELECT' <<< "$SASS" | sed 's/  */ /g' | head -40;
+  echo "# opcode histogram (top 25):"; grep -oE '^\s+/\*[0-9a-f]{4,}\*/\s+(@!?U?P[0-9T] )?[A-Z0-9_.]+' <<< "$SASS" | awk '{print $NF}' | cut -d. -f1 | sort | uniq -c | sort -rn | head -25; } > profiles/${R}_step_kernel_sass.txt
 ls -la profiles/${R}_*

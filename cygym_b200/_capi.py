@@ -10,7 +10,7 @@ import subprocess
 from . import draw_tables as DT
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("CYGYM_B200_LIB") or os.path.join(_HERE, "libcygym_b200.so")  # override: profiling builds only
+LIB_PATH = os.path.join(_HERE, "libcygym_b200.so")
 _SRC = os.path.join(_HERE, "csrc", "cyg_kernels.cu")
 _DEPS = [_SRC, os.path.join(_HERE, "csrc", "cyg_core.cuh"), os.path.join(_HERE, "csrc", "cyg_coop.cuh"),
          os.path.join(_HERE, "csrc", "cyg_tables.h"), os.path.join(_HERE, "csrc", "cyg_iforest.cuh"),
@@ -20,7 +20,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 PLANE_WIDTHS = (1, 2, 3, 4, 64)  # one translation unit of cyg_kernels.cu per plane width W (+ one for the C-ABI)
 
 # The constants of include/cygym_b200.h, named as there without the CYG_ prefix (tests/test_abi_formats.py checks them).
-ABI_VERSION = 2
+ABI_VERSION = 3
 NSCAL = 16
 ATYPE_NONE = 0x80
 MODE_DEFENDER, MODE_ATTACKER = 0, 1
@@ -129,7 +129,7 @@ class CygRolloutArgs(C.Structure):
 
 EXPORTS = ["cyg_version", "cyg_last_error", "cyg_create", "cyg_destroy", "cyg_set_base_line", "cyg_set_base_line_per_env", "cyg_set_base_line_per_env_steps", "cyg_internal_words",
            "cyg_bind", "cyg_set_detectors", "cyg_fit_detectors", "cyg_import_state", "cyg_export_state", "cyg_step", "cyg_step_multi", "cyg_rollout", "cyg_unpack_actions", "cyg_pack_done", "cyg_block_envs", "cyg_set_env_id_stride", "cyg_randomize", "cyg_rebuild_graph_cache", "cyg_sample_actions", "cyg_sample_actions_ordered",
-           "cyg_observe", "cyg_group_actions", "cyg_launch_count", "cyg_set_debug_cycles"]
+           "cyg_observe", "cyg_group_actions", "cyg_launch_count"]
 
 
 class CygError(RuntimeError):
@@ -249,7 +249,6 @@ def lib():
                                         C.c_void_p, C.c_void_p, C.c_void_p]
         L.cyg_launch_count.argtypes = [C.c_void_p]
         L.cyg_launch_count.restype = C.c_int64
-        L.cyg_set_debug_cycles.argtypes = [C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 

@@ -159,9 +159,6 @@ struct Coop {
       int pos = 0;
       uint32_t kbase = 0;
       while (pos < na) { /* uniform */
-#ifdef CYG_COUNT_ROUNDS
-        e.dbg_rounds++;
-#endif
         const int idx = pos + lane;
         const bool valid0 = idx < na;
         const int d = valid0 ? e.select_nth(act, idx) : 0;
@@ -257,9 +254,6 @@ struct Coop {
         auto passes = [&](auto has_x) {
         constexpr bool HX = decltype(has_x)::value;
         for (;;) {
-#ifdef CYG_COUNT_ROUNDS
-          e.dbg_rounds += 0x10000;
-#endif
           const int c0 = popc(x[0]), c1 = popc(x[1]), c2 = popc(x[2]), c3 = popc(x[3]);
           const int tot = c0 + c1 + c2 + c3 + (HX ? popc(imo) + popc(imi) : 0);
           nem = __ballot_sync(CYG_FULL, tot > 0);

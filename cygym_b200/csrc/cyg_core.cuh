@@ -48,13 +48,6 @@
 
 namespace cyg {
 
-/* optional phase timestamps inside step() (profiling builds only: -DCYG_PHASE_TIMING) */
-#if defined(CYG_PHASE_TIMING) && defined(__CUDA_ARCH__)
-#define CYG_MARK(i) do { if (phase_t) phase_t[i] = clock64(); } while (0)
-#else
-#define CYG_MARK(i) do { } while (0)
-#endif
-
 /* draw sites: oracle/draws.py (each is one RNG call site of the reference) */
 enum {
   SITE_STALL = 1, SITE_BLOCK = 2, SITE_UNBLOCK = 3, SITE_ZDAY = 4, SITE_PROBE = 5, SITE_WL_SAMPLE = 6,
@@ -249,8 +242,6 @@ struct Env {
   Stream stall;    /* SITE_STALL is shared by every group of a grouped step */
   int bl;          /* base_line in effect for this env (CYG_BL_*): cfg.base_line unless the caller set one per env */
   double defcost, cleancost;
-  long long* phase_t = nullptr; /* profiling builds only */
-  int dbg_rounds = 0;           /* profiling builds only */
 
   CYG_HD Env(const Net* net, uint32_t* record, uint32_t* ck, uint32_t* xt, uint32_t env_id, uint32_t rec_off = 0,
              uint32_t tab_off = 0)
@@ -1590,11 +1581,9 @@ struct Env {
    * step_post: work, arrivals, reward, counters, evolve_network (volt:1207-1333) */
   CYG_HD int step_pre(const uint32_t* hdr, uint32_t flags) {
     begin_epoch();
-    CYG_MARK(0);
     if (flags & CYG_STEP_GROUPED) return 0;
     int atype = exec_type(n->cfg, hdr[0], bl);
     tick_busyset(); /* volt:904-908 */
-    CYG_MARK(1);
     return atype;
   }
   CYG_HD void load_costs() {
@@ -1669,7 +1658,6 @@ struct Env {
       }
       tick_all(); /* _tick_busy_time_once (volt:607-610) */
     }
-    CYG_MARK(2);
     store_costs();
     return atype;
   }
@@ -1682,13 +1670,11 @@ struct Env {
     int cur_work = 0;
     if (!skip_work || grouped) {
       cur_work = workload_advance();
-      CYG_MARK(3);
       arrivals_if_due();
     }
     double def_work = (double)c.work_scale * cur_work;
     int n_comp, n_comp_dc;
     count_comp(n_comp, n_comp_dc);
-    CYG_MARK(4);
     if (!grouped) scal(CYG_S_COMPCNT) += (uint32_t)n_comp; /* volt:1267-1270; absent from step_grouped */
     double raw, shaped;
     if (mode == CYG_MODE_DEFENDER) {
@@ -1704,7 +1690,6 @@ struct Env {
       scal(CYG_S_PREV_X) = (scal(CYG_S_PREV_X) & 0xFFFF0000u) | (uint32_t)n_comp;
       shaped = raw + bonus;
     }
-    CYG_MARK(5);
     if (pre_masks) { /* the `state` step() returns is the pre-evolve view (volt:1306) */
       const int Wm = n->Wm;
       for (int w = 0; w < W; w++) {
@@ -1721,11 +1706,9 @@ struct Env {
     int done = scal(CYG_S_STEP) > 1000u; /* _check_done (CyberDefenseEnv.py:547-552) */
     bool periodic = (scal(CYG_S_STEP) % (uint32_t)c.evolve_period) == 0;
     if (dirty || periodic) evolve_network();
-    CYG_MARK(6);
     if (!grouped) { /* volt:1330 */
       for (int w = 0; w < W; w++) pl(P_BUSYSET, w) = busy_nz(w);
     }
-    CYG_MARK(7);
     *raw_out = (float)raw; *shaped_out = (float)shaped; *done_out = done;
   }
 

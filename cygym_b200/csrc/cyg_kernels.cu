@@ -81,7 +81,6 @@ struct StepParams {
   int32_t* done;
   uint32_t* pre_masks;
   float* obs;
-  unsigned long long* dbg_cycles; /* optional [B]: SM cycles each env's step took (diagnostics) */
   uint32_t* logs;                 /* [B][log_cap] hop-log rings (NULL when log_cap == 0) */
   const uint32_t* det_slots;      /* uploaded detectors (cyg_set_detectors) */
   const int32_t* det_of_env;      /* [B] slot of env, -1 none */
@@ -285,16 +284,6 @@ __host__ __device__ inline SmemPlan smem_plan(uint32_t hot_words, int S, int NB)
   return p;
 }
 
-/* CTA-level phase timestamps (profiling build -DCYG_CTA_TIMING: thread 0 writes clock64 at the phase boundaries) */
-#ifdef CYG_CTA_TIMING
-#define CYG_CTA_MARK(i) do { if (p.dbg_cycles && threadIdx.x == 0) p.dbg_cycles[(size_t)blockIdx.x * 8 + (i)] = (unsigned long long)clock64(); } while (0)
-/* per-warp timestamps inside phase B (after the block/unblock, deposit and attack task loops): slots of 4 behind the CTA marks */
-#define CYG_WARP_MARK(i) do { if (p.dbg_cycles && (threadIdx.x & 31) == 0) p.dbg_cycles[2048 + ((size_t)blockIdx.x * 32 + (threadIdx.x >> 5)) * 4 + (i)] = (unsigned long long)clock64(); } while (0)
-#else
-#define CYG_CTA_MARK(i) do { } while (0)
-#define CYG_WARP_MARK(i) do { } while (0)
-#endif
-
 /* The plain step: one ungrouped action per env, device lists as sets (no order array) -- the hot form: thread-per-env
  * phases A / C plus the warp-per-env phase B, T steps fused per launch.  Grouped steps and explicit order lists run in
  * cyg_step_seq_kernel (the sequential forms of every action live only there). */
@@ -308,7 +297,6 @@ template <int W, bool ROLL, bool LOG>
 __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(const __grid_constant__ StepParams p) {
   unsigned char* smem = reinterpret_cast<unsigned char*>(cyg_smem);
   const int NB = p.block_envs, NT = blockDim.x, tid = threadIdx.x; /* NB envs, NT >= NB threads */
-  CYG_CTA_MARK(0);
   const int S = p.net.S, M = p.net.M;
   int blk_i = (int)blockIdx.x;
   if constexpr (ROLL) { if (p.block_order) blk_i = p.block_order[blockIdx.x]; }
@@ -353,11 +341,9 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
   }
   for (int i = tid; i < CYG_NKEYS + 7; i += NT) s_cnt[i] = 0; /* ... + one "past pass 0" flag per owning warp */
   __syncthreads(); /* mbarrier initialised, counters zeroed (t > 0: the previous step is complete) */
-  CYG_CTA_MARK(1);
   sort_block<W, true>(p.net, hdr_t, bl_t, true, arow, env0, nb, s_cnt, s_perm, tid);
   if (t == 0) load_block_finish(bulk_ok, s_rec, g_rec, nb * S, bar, tid, NT);
   __syncthreads();
-  CYG_CTA_MARK(2);
 
   /* ---- the step in two passes over ONE copy of the thread-per-env code (the loop is not unrolled: step_post alone
    *      is ~10k SASS instructions, and the kernel's instruction footprint is what its warps miss on):
@@ -380,11 +366,6 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
     }
   };
   if (tid < nb) bind_aux(e, env);
-  long long t_begin = 0;
-#ifdef CYG_PHASE_TIMING
-  long long ph[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  e.phase_t = ph;
-#endif
   int mode = 0;
   uint32_t home_mask = 0; /* lanes of this warp whose env's record is finished and not yet sent home (uniform) */
   auto send_some = [&](int k) {
@@ -407,7 +388,6 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
         act[0] = hv.x; act[1] = hv.y; act[2] = hv.z; act[3] = hv.w;
 #pragma unroll
         for (int w = 0; w < W; w++) act[4 + w] = mask_t[my_row * W + w];
-        t_begin = p.dbg_cycles ? clock64() : 0;
         mode = (int)((act[0] >> 8) & 1u);
         if (bl_t) e.bl = (int)bl_t[my_row];
         atype = e.step_pre(act, p.flags);
@@ -427,7 +407,6 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
         do_post = true;
       }
     } else {
-  CYG_CTA_MARK(3);
       if (lane == 0) while (atomicAdd(&s_cnt[CYG_NKEYS + 6], 0u) < (uint32_t)((nb + 31) >> 5)) __nanosleep(32);
       __syncwarp();
       auto load_action = [&](size_t row_b, uint32_t* act) {
@@ -468,7 +447,6 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
           Env<W, 1>::decode(act, act + 4, nullptr, a);
           double tcost = 0.0;
           bool tdirty = false;
-          long long tb0 = p.dbg_cycles ? clock64() : 0;
           if (lane == 0) eb.load_costs();
           if (kind == 0) {
             Coop<W>::template flip<32>(eb, a, (int)(act[0] & 0xFFu), tcost, tdirty); /* flip keys only hold executed types 6 / 9 == the header's */
@@ -479,22 +457,14 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
             Coop<W>::defender(eb, a, atype_b, tcost, tdirty);
           }
           if (lane == 0) {
-#if !defined(CYG_PHASE_TIMING) && !defined(CYG_CTA_TIMING)
-            if (p.dbg_cycles) p.dbg_cycles[env_b] = (unsigned long long)(clock64() - tb0); /* heavy envs: phase-B cycles */
-#endif
-#ifdef CYG_COUNT_ROUNDS
-            if (p.dbg_cycles && kind == 0) p.dbg_cycles[env_b] = (unsigned long long)eb.dbg_rounds;
-#endif
             eb.store_costs();
             s_out[el_b] = (float)tcost;
             s_out[NB + el_b] = __int_as_float(tdirty ? 1 : 0);
           }
           __syncwarp();
         }
-        CYG_WARP_MARK(kind);
       }
       __syncthreads();
-  CYG_CTA_MARK(4);
       /* ---- phase C, thread per env again: the rest of the step for the envs phase B handled ---- */
       if (deferred) {
         e = Env<W, 1>(&p.net, nullptr, p.ckpt + (size_t)env * M, p.xtra + (size_t)env * p.net.cfg.xcap, (uint32_t)p.env_id0 + idx_of(env),
@@ -514,13 +484,6 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
       if constexpr (ROLL) p.ret_acc[(size_t)mode * p.B + env] += (double)raw;
       else { raw_t[env] = raw; shaped_t[env] = shaped; done_t[env] = done; }
     }
-    if (pass == 0 && tid < nb) {
-#ifdef CYG_PHASE_TIMING
-      if (p.dbg_cycles) for (int i = 0; i < 8; i++) p.dbg_cycles[(size_t)env * 8 + i] = (unsigned long long)(ph[i] - t_begin);
-#elif !defined(CYG_CTA_TIMING)
-      if (p.dbg_cycles && !deferred) p.dbg_cycles[env] = (unsigned long long)(clock64() - t_begin);
-#endif
-    }
     if (last && lower) {
       /* The records this warp's threads just finished go home by warp-wide copies, right away.  Measured alternatives:
        * 4 records after each phase-B task of the warp (38.3 / 50.5 us fused / single against 37.8 / 48.1), a shared
@@ -532,15 +495,14 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
     }
   }
   __syncthreads();
-  CYG_CTA_MARK(5);
   } /* fused steps */
 
-  /* ---- optional fused observation rows (post-evolve view, CyberDefenseEnv.py:146-257) ---- */
+  /* ---- optional fused observation rows (post-evolve view, CyberDefenseEnv.py:146-257); every warp sent its records
+   *      home already ---- */
   if (p.obs && p.obs_mode) {
     const int dim = p.obs_mode == 2 ? 4 * M + p.net.cfg.X : 6 * M;
     observe_rows<W>(p.net, s_rec, S, nb, p.obs_mode, p.obs + (size_t)env0 * dim, tid >> 5, NT >> 5, lane);
   }
-  CYG_CTA_MARK(6); /* every warp sent its records home already */
 }
 
 /* Grouped steps (CYG_STEP_GROUPED: G action groups per env) and explicit order lists: one step per launch, thread per env
@@ -550,7 +512,6 @@ template <int W>
 __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_seq_kernel(const __grid_constant__ StepParams p) {
   unsigned char* smem = reinterpret_cast<unsigned char*>(cyg_smem);
   const int NB = p.block_envs, NT = blockDim.x, tid = threadIdx.x;
-  CYG_CTA_MARK(0);
   const int S = p.net.S, M = p.net.M;
   const int env0 = (int)blockIdx.x * NB;
   const int nb = min(NB, p.B - env0);
@@ -568,11 +529,9 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_seq_kernel(
   const int lane = tid & 31;
   for (int i = tid; i < CYG_NKEYS + 7; i += NT) s_cnt[i] = 0;
   __syncthreads(); /* mbarrier initialised, counters zeroed */
-  CYG_CTA_MARK(1);
   sort_block<W, false>(p.net, p.hdr, p.bl_env, !grouped, [](int env_i) { return (size_t)env_i; }, env0, nb, s_cnt, s_perm, tid);
   load_block_finish(bulk_ok, s_rec, g_rec, nb * S, bar, tid, NT);
   __syncthreads();
-  CYG_CTA_MARK(2);
 
   const int el = tid < nb ? (int)s_perm[tid] : 0, env = env0 + el;
   Env<W, 1> e(&p.net, nullptr, p.ckpt + (size_t)env * M, p.xtra + (size_t)env * p.net.cfg.xcap, (uint32_t)p.env_id0 + (uint32_t)env,
@@ -581,11 +540,6 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_seq_kernel(
     e.logs = p.logs ? p.logs + (size_t)env * p.net.cfg.log_cap : nullptr;
     e.det = (p.det_slots && p.det_of_env[env] >= 0) ? p.det_slots + (size_t)p.det_of_env[env] * CYG_DET_WORDS : nullptr;
   }
-  long long t_begin = 0;
-#ifdef CYG_PHASE_TIMING
-  long long ph[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  e.phase_t = ph;
-#endif
   double cost = 0.0;
   bool dirty = false;
   uint32_t act[4 + W]; /* this env's action (group 0), in registers */
@@ -595,7 +549,6 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_seq_kernel(
     act[0] = hv.x; act[1] = hv.y; act[2] = hv.z; act[3] = hv.w;
 #pragma unroll
     for (int w = 0; w < W; w++) act[4 + w] = p.mask[(size_t)env * W + w];
-    t_begin = p.dbg_cycles ? clock64() : 0;
     const int mode = (int)((act[0] >> 8) & 1u);
     if (p.bl_env) e.bl = (int)p.bl_env[env];
     const int atype = e.step_pre(act, p.flags);
@@ -606,14 +559,8 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_seq_kernel(
     int32_t done;
     e.step_post(mode, cost, dirty, p.flags, &raw, &shaped, &done, p.pre_masks ? p.pre_masks + (size_t)env * 3 * W : nullptr);
     p.raw[env] = raw; p.shaped[env] = shaped; p.done[env] = done;
-#ifdef CYG_PHASE_TIMING
-    if (p.dbg_cycles) for (int i = 0; i < 8; i++) p.dbg_cycles[(size_t)env * 8 + i] = (unsigned long long)(ph[i] - t_begin);
-#elif !defined(CYG_CTA_TIMING)
-    if (p.dbg_cycles) p.dbg_cycles[env] = (unsigned long long)(clock64() - t_begin);
-#endif
   }
   __syncthreads();
-  CYG_CTA_MARK(5);
 
   /* ---- optional fused observation rows (post-evolve view, CyberDefenseEnv.py:146-257) ---- */
   if (p.obs && p.obs_mode) {
@@ -627,14 +574,12 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_seq_kernel(
   if (bulk_ok) {
     fence_proxy_async();
     __syncthreads();
-    CYG_CTA_MARK(6);
     if (tid == 0) {
       bulk_s2g(g_rec, s_rec, rec_bytes);
       bulk_commit_wait_read();
     }
   } else {
     for (int i = tid; i < nb * S; i += NT) g_rec[i] = s_rec[i];
-    CYG_CTA_MARK(6);
   }
 }
 
@@ -1183,25 +1128,19 @@ void cyg_group_launch(int blocks, int threads, cudaStream_t st, const GroupParam
 void cyg_unpack_launch(int blocks, int threads, cudaStream_t st, const UnpackParams& p);
 void cyg_pack_done_launch(int blocks, int threads, cudaStream_t st, const int32_t* done, uint32_t* bits, int B);
 int cyg_fit_launch(int n_sms, cudaStream_t st, const FitParams& p);
-const WOps* cyg_wops_4(void);
-#ifndef CYG_FAST_BUILD /* profiling builds link the W = 4 unit only (config C3) */
 const WOps* cyg_wops_1(void);
 const WOps* cyg_wops_2(void);
 const WOps* cyg_wops_3(void);
+const WOps* cyg_wops_4(void);
 const WOps* cyg_wops_64(void);
-#endif
 }
 static const WOps* wops(int W) {
   switch (W) {
-    case 4: return cyg_wops_4();
-#ifndef CYG_FAST_BUILD
     case 1: return cyg_wops_1();
     case 2: return cyg_wops_2();
     case 3: return cyg_wops_3();
+    case 4: return cyg_wops_4();
     default: return cyg_wops_64();
-#else
-    default: return nullptr;
-#endif
   }
 }
 
@@ -1214,7 +1153,6 @@ struct cyg_env_s {
   uint32_t* d_blob;
   uint32_t* state;   /* bound internal buffer: [B][S] records then [B][M] checkpoint words */
   int B, env_id0, device, W, NB, n_sms;
-  unsigned long long* dbg_cycles;
   const uint32_t* det_slots; /* uploaded detectors (device memory of the caller) */
   const int32_t* det_of_env;
   int n_det_slots;
@@ -1247,10 +1185,9 @@ struct DeviceGuard {
   ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
-static int pick_block_envs(const cyg_env_s* h, int requested) {
+static int pick_block_envs(const cyg_env_s* h) {
   /* envs (= threads) per CTA.  One CTA per SM: the bigger the block, the purer the per-warp action types after
    * the in-CTA sort.  Spread B over the SMs in one wave, bounded by shared memory and 512 threads. */
-  if (requested > 0) return requested;
   const size_t budget = 226 * 1024;
   int per_sm = (h->B + h->n_sms - 1) / h->n_sms;
   int nb = ((per_sm + 3) / 4) * 4; /* a multiple of 4 records keeps every CTA's span 16-byte sized (bulk copies) whatever S is;
@@ -1262,7 +1199,6 @@ static int pick_block_envs(const cyg_env_s* h, int requested) {
 }
 
 static int configure_step(cyg_env_s* h) {
-  if (!wops(h->W)) return fail(CYG_E_INVAL, "this build has no kernels for the network's plane width");
   if (h->W > CYG_MAX_W) { /* large networks: a few envs per CTA so that every SM gets some, records staged in shared memory */
     int per_sm = (h->B + h->n_sms - 1) / h->n_sms;
     const size_t rec_bytes = (size_t)h->net.S * 4;
@@ -1304,7 +1240,7 @@ int cyg_create(cyg_handle* out, const cyg_config* cfg, const cyg_network* host_n
   if (!h) return fail(CYG_E_NOMEM, "out of host memory");
   std::string err = build_tables(*cfg, *host_net, h->blob);
   if (!err.empty()) { delete h; return fail(CYG_E_INVAL, err); }
-  h->B = B; h->env_id0 = env_id0; h->device = device; h->state = nullptr; h->launches = 0; h->dbg_cycles = nullptr; h->bl_env = nullptr; h->bl_rows = 1; h->id_run = 0; h->id_stride = 0;
+  h->B = B; h->env_id0 = env_id0; h->device = device; h->state = nullptr; h->launches = 0; h->bl_env = nullptr; h->bl_rows = 1; h->id_run = 0; h->id_stride = 0;
   h->det_slots = nullptr; h->det_of_env = nullptr; h->n_det_slots = 0; h->fit_work = nullptr;
   h->W = h->blob.net.W;
   DeviceGuard g(device);
@@ -1317,9 +1253,7 @@ int cyg_create(cyg_handle* out, const cyg_config* cfg, const cyg_network* host_n
   relocate(h->blob, h->d_blob, h->net);
   cudaDeviceGetAttribute(&h->n_sms, cudaDevAttrMultiProcessorCount, device);
   if (h->n_sms < 1) h->n_sms = 148;
-  const char* nb_env = getenv("CYG_BLOCK_ENVS");
-  h->NB = pick_block_envs(h, nb_env ? atoi(nb_env) : 0);
-  if (h->NB < 1 || h->NB > CYG_MAX_BLOCK_ENVS) { cudaFree(h->d_blob); delete h; return fail(CYG_E_INVAL, "CYG_BLOCK_ENVS must be in 1..512"); }
+  h->NB = pick_block_envs(h);
   int rc = CYG_OK;
   rc = configure_step(h);
   if (rc != CYG_OK) { cudaFree(h->d_blob); delete h; return rc; }
@@ -1499,7 +1433,7 @@ static int step_impl(cyg_handle h, const cyg_actions* a, int n_steps, uint32_t s
   StepParams p = step_params(h);
   p.hdr = a->hdr; p.mask = a->mask; p.order = a->order;
   p.raw = out->raw_reward; p.shaped = out->shaped_reward; p.done = out->done;
-  p.pre_masks = out->pre_masks; p.obs = out->obs; p.dbg_cycles = h->dbg_cycles; p.bl_env = h->bl_env; p.bl_stride = (h->bl_env && h->bl_rows > 1) ? h->B : 0;
+  p.pre_masks = out->pre_masks; p.obs = out->obs; p.bl_env = h->bl_env; p.bl_stride = (h->bl_env && h->bl_rows > 1) ? h->B : 0;
   p.G = a->n_groups; p.order_stride = a->order_stride;
   p.obs_mode = out->obs ? out->obs_mode : 0;
   p.flags = step_flags;
@@ -1638,12 +1572,6 @@ int cyg_group_actions(cyg_handle h, int32_t mode, int32_t role, const int32_t* p
 }
 
 int64_t cyg_launch_count(cyg_handle h) { return h ? h->launches : 0; }
-
-int cyg_set_debug_cycles(cyg_handle h, uint64_t* per_env_cycles) {
-  if (!h) return fail(CYG_E_INVAL, "null handle");
-  h->dbg_cycles = (unsigned long long*)per_env_cycles;
-  return CYG_OK;
-}
 
 } /* extern "C" */
 #endif /* CYG_TU_W */

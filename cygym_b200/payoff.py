@@ -177,8 +177,9 @@ def _cached_env(network, nloc, lo, device, seed, xcap):
     return env
 
 
-# rough SM cycles per env of one turn by executed action type (profiles/type_cycles.py: warp-per-env tasks shared by
-# the 20 warps of a CTA, thread-per-env types by 14 warps of 32 lanes); only the ORDER of the blocks depends on them
+# rough SM cycles per env of one turn by executed action type (measured on a B200 with a per-env cycle counter the step
+# kernel no longer has, see git history: warp-per-env tasks shared by the 20 warps of a CTA, thread-per-env types by
+# 14 warps of 32 lanes); only the ORDER of the blocks depends on them
 _DEF_PER_DEVICE = {6: 11.0, 9: 9.0, 1: 3.75, 3: 2.75, 4: 2.25}
 _TURN_BASE, _ATTACK_COST, _BASELINE_COST = 25.0, 185.0, 60.0
 

@@ -215,7 +215,7 @@ class VectorCyberDefenseEnv:
 
     def _drop_graphs(self):
         """A captured step_host() graph holds the kernel parameters BY VALUE (base_line, the per-env base_line
-        pointer and stride, the debug buffer): whatever changes one of them must drop the captures."""
+        pointer and stride): whatever changes one of them must drop the captures."""
         if self._graphs:
             torch.cuda.synchronize(self.device)
             self._graphs = {}

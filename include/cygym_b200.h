@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define CYG_ABI_VERSION 2
+#define CYG_ABI_VERSION 3
 
 /* ---- error codes ------------------------------------------------------- */
 #define CYG_OK 0
@@ -374,10 +374,6 @@ int cyg_group_actions(cyg_handle h, int32_t mode, int32_t role, const int32_t* p
 
 /* Number of kernels this handle has launched so far (bench.py's gpu_launches). */
 int64_t cyg_launch_count(cyg_handle h);
-
-/* Diagnostics: when a device buffer [B] is set, every cyg_step writes the SM cycles each env's transition
- * took (profiles/type_cycles.py groups them by action type).  NULL switches it off (the default). */
-int cyg_set_debug_cycles(cyg_handle h, uint64_t* per_env_cycles);
 
 #ifdef __cplusplus
 }

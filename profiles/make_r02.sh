@@ -2,7 +2,7 @@
 # Round-2 measurement recipe (run on the B200 box through gpurun from the repo root):
 #   the default bench line, the launch list of a short bench command (ncu gpu__time_duration: cold-cache, serialised --
 #   compare shares), one full capture of single-step launches (defender + attacker turn), one of a fused launch, the
-#   per-type exclusion sweep and the CTA phase cycles (profiling build)
+#   per-type exclusion sweep
 mkdir -p gpurun_out
 python bench.py > gpurun_out/r02_bench.json 2> gpurun_out/r02_bench.err
 python bench.py --steps 24 --warmup 4 --no-cpu-baseline --no-e2e --no-legs > gpurun_out/r02_plain.log 2>&1 && \
@@ -14,5 +14,4 @@ ncu --set full --clock-control none --import-source on -k regex:cyg_step_kernel 
 ncu --set full --clock-control none -k regex:cyg_step_kernel -s 4 -c 2 -o gpurun_out/r02_step_kernel_fused \
     python bench.py --steps 24 --warmup 4 --no-cpu-baseline --no-e2e --no-legs > gpurun_out/r02_ncu_full_fused.log 2>&1
 bash profiles/exclude_sweep.sh gpurun_out/r02_exclude_sweep.txt > /dev/null 2>&1
-if [ -f profiles/_build/cta.so ]; then CYGYM_B200_LIB=profiles/_build/cta.so python profiles/cta_phases.py > gpurun_out/r02_cta_phases.txt 2>&1; fi
 tail -1 gpurun_out/r02_bench.json | cut -c1-300

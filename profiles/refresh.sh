@@ -31,7 +31,6 @@ python profiles/ncu_lines.py gpurun_out/src_${R}_2.csv 25 > profiles/${R}_step_k
 tail -1 gpurun_out/${R}_bench.json > profiles/${R}_bench_line.json
 cp gpurun_out/${R}_launches.csv profiles/${R}_launches.csv
 [ -f gpurun_out/${R}_exclude_sweep.txt ] && cp gpurun_out/${R}_exclude_sweep.txt profiles/${R}_exclude_sweep.txt
-[ -f gpurun_out/${R}_cta_phases.txt ] && cp gpurun_out/${R}_cta_phases.txt profiles/${R}_cta_phases.txt
 # SASS evidence: bulk (TMA) copies + mbarrier waits in the step kernel, instruction count of the plain instantiation
 SASS=$(cuobjdump -sass -fun '_Z15cyg_step_kernelILi4ELb0ELb0EEv10StepParams' cygym_b200/libcygym_b200.so 2>/dev/null || true)
 { echo "# cuobjdump -sass of cyg_step_kernel<4, no ROLL, no LOG> in cygym_b200/libcygym_b200.so (sm_100a)";

@@ -25,7 +25,7 @@ def test_library_loaded_is_the_cuda_one():
     import torch
     from cygym_b200 import _capi
     assert torch.cuda.is_available()
-    assert _capi.lib().cyg_version() == 2
+    assert _capi.lib().cyg_version() == 3
     assert "sm_100" in " ".join(torch.cuda.get_arch_list()) or torch.cuda.get_device_capability()[0] >= 10
 
 

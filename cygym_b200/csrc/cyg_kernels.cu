@@ -14,6 +14,8 @@
  * cyg_step_generic_kernel<W>: networks beyond 128 device slots (tables too large for shared memory).
  * cyg_fit_assign_kernel + cyg_fit_kernel: the detector fit of defender action 10 (cyg_iforest.cuh), one warp per
  *   pending env.
+ * Host side: each plane width's translation unit exports the handles of its kernels in one table (Kernels); the C-ABI
+ *   unit holds the kernels that do not depend on the width, and every entry point launches through launch().
  * No tensor cores: the path has no dense contraction.  No CPU fallback anywhere in this file.
  */
 #include <cuda_runtime.h>
@@ -818,6 +820,7 @@ __global__ void cyg_export_kernel(const __grid_constant__ ConvParams p) {
     for (int i = lane; i < n.cfg.log_cap; i += 32) p.logs[(size_t)warp * n.cfg.log_cap + i] = p.logs_int[(size_t)warp * n.cfg.log_cap + i];
 }
 
+#ifndef CYG_TU_W /* the kernels that do not depend on the plane width: one copy, in the C-ABI unit */
 /* ---- IPPO / MAPPO glue: per-device action types -> the per-type action groups of one grouped step (IPPO.py:559-570),
  *      with the role's visibility mask (build_visibility_mask, IPPO.py:74-96) read straight from the bit-planes.
  *      One warp per env, lanes on 32 devices; group g = the g-th action type other than the no-op. ---- */
@@ -833,7 +836,6 @@ struct GroupParams {
   uint32_t* mask;         /* [n_types - 1][B][Wm] */
   int B, mode, role, n_types, noop;
 };
-#if defined(CYG_TU_W) && CYG_TU_W == 4 /* one copy: the kernel is not templated on the plane width */
 /* the groups of ONE env by one warp: lane g < G ends up with group g's device words (handed to `put` word by word) and its
  * header (returned through h4) */
 template <typename Put>
@@ -902,8 +904,6 @@ __global__ void cyg_group_kernel(const __grid_constant__ GroupParams p) {
   if (lane < G) *reinterpret_cast<uint4*>(p.hdr + ((size_t)lane * p.B + b) * 4) = make_uint4(h4[0], h4[1], h4[2], h4[3]);
 }
 
-#endif
-
 /* cyg_unpack_actions: compact action rows [B][2 + Wm] (include/cygym_b200.h) -> hdr [B][4] + mask [B][Wm].  One thread
  * per env; the rows are what a host-buffer step moves over PCIe (24 bytes per env at M <= 128 instead of 32). */
 struct UnpackParams {
@@ -912,7 +912,6 @@ struct UnpackParams {
   uint32_t* mask;
   int B, Wm;
 };
-#if defined(CYG_TU_W) && CYG_TU_W == 4
 __global__ void cyg_unpack_kernel(const __grid_constant__ UnpackParams p) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env >= p.B) return;
@@ -933,17 +932,12 @@ __global__ void cyg_unpack_kernel(const __grid_constant__ UnpackParams p) {
   *reinterpret_cast<uint4*>(p.hdr + (size_t)env * 4) = h;
   for (int w = 0; w < p.Wm; w++) p.mask[(size_t)env * p.Wm + w] = r[2 + w];
 }
-extern "C" void cyg_unpack_launch(int blocks, int threads, cudaStream_t st, const UnpackParams& p) { cyg_unpack_kernel<<<blocks, threads, 0, st>>>(p); }
 /* cyg_pack_done: done flags [B] (int32) -> one bit per env (bit b % 32 of word b / 32) */
 __global__ void cyg_pack_done_kernel(const int32_t* done, uint32_t* bits, int B) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   const uint32_t m = __ballot_sync(0xFFFFFFFFu, env < B && done[env] != 0);
   if ((threadIdx.x & 31) == 0 && env < B) bits[env >> 5] = m;
 }
-extern "C" void cyg_pack_done_launch(int blocks, int threads, cudaStream_t st, const int32_t* done, uint32_t* bits, int B) {
-  cyg_pack_done_kernel<<<blocks, threads, 0, st>>>(done, bits, B);
-}
-#endif
 
 /* ---- detector fits (cyg_fit_detectors; cyg_iforest.cuh) ---- */
 struct FitParams {
@@ -957,7 +951,6 @@ struct FitParams {
   int S, B, log_cap, n_slots;
 };
 #define CYG_FIT_WARPS 4 /* fitting warps per CTA (cyg_iforest::Scratch each, in shared memory) */
-#if defined(CYG_TU_W) && CYG_TU_W == 4
 /* Block-wide exclusive count of `v` over the threads below this one; *total = count over the block. */
 __device__ __forceinline__ int block_rank(bool v, int* warp_tot, int* total) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = (blockDim.x + 31) >> 5;
@@ -1037,15 +1030,7 @@ __global__ void __launch_bounds__(32 * CYG_FIT_WARPS) cyg_fit_kernel(const __gri
     __syncwarp();
   }
 }
-extern "C" int cyg_fit_launch(int n_sms, cudaStream_t st, const FitParams& p) {
-  const size_t smem = sizeof(iforest::Scratch) * CYG_FIT_WARPS;
-  cudaError_t e = cudaFuncSetAttribute(cyg_fit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  cyg_fit_assign_kernel<<<1, 1024, 0, st>>>(p);
-  cyg_fit_kernel<<<3 * n_sms, 32 * CYG_FIT_WARPS, smem, st>>>(p); /* 3 CTAs of 4 Scratch each fit one SM's shared memory */
-  return (int)cudaGetLastError();
-}
-#endif
+#endif /* !CYG_TU_W */
 
 struct ObsParams {
   Net net;
@@ -1060,87 +1045,38 @@ __global__ void cyg_observe_kernel(const __grid_constant__ ObsParams p) {
 }
 
 /* ===========================================================================
- * Per-W launch table.  The library is built from several translation units of THIS file: one per plane width W
- * (-DCYG_TU_W=1|2|3|4|64: the kernels of that width and their launchers, compiled without --split-compile so that the
- * register allocation of the hot kernels does not depend on what else is in the module) and one with the C-ABI
- * (no CYG_TU_W: no kernel is instantiated there).
+ * Per-W kernel table.  The library is built from several translation units of THIS file: one per plane width W
+ * (-DCYG_TU_W=1|2|3|4|64: the kernels of that width, in a module of their own so that the register allocation of the
+ * hot kernels does not depend on what else is compiled), each exporting the handles of its kernels in one table, and
+ * one with the C-ABI (no CYG_TU_W: the width-independent kernels above and the entry points, which launch every kernel
+ * through launch() below).
  * ======================================================================== */
-struct WOps {
-  cudaError_t (*set_smem_optin)(int max_optin);
-  void (*step)(bool plain, int blocks, int threads, size_t smem, cudaStream_t st, const StepParams& p);
-  void (*rollout)(int blocks, int threads, size_t smem, cudaStream_t st, const StepParams& p);
-  void (*import_state)(int blocks, int threads, cudaStream_t st, const ConvParams& p);
-  void (*export_state)(int blocks, int threads, cudaStream_t st, const ConvParams& p);
-  void (*randomize)(int blocks, int threads, cudaStream_t st, const SimpleParams& p);
-  void (*rebuild)(int blocks, int threads, cudaStream_t st, const SimpleParams& p);
-  void (*sample)(int blocks, int threads, cudaStream_t st, const SimpleParams& p);
-  void (*observe)(int blocks, int threads, cudaStream_t st, const ObsParams& p);
+struct Kernels {
+  const void *step, *step_log, *step_seq, *rollout; /* W = 64: cyg_step_generic_kernel in `step`, the other forms null */
+  const void *import_state, *export_state, *randomize, *rebuild, *sample, *observe;
 };
-#define CYG_WOPS_NAME2(w) cyg_wops_##w
-#define CYG_WOPS_NAME(w) CYG_WOPS_NAME2(w)
+#define CYG_KERNELS_NAME2(w) cyg_kernels_w##w
+#define CYG_KERNELS_NAME(w) CYG_KERNELS_NAME2(w)
 
 #ifdef CYG_TU_W
-#if CYG_TU_W == 4
-extern "C" void cyg_group_launch(int blocks, int threads, cudaStream_t st, const GroupParams& p) { cyg_group_kernel<<<blocks, threads, 0, st>>>(p); }
+extern "C" const Kernels CYG_KERNELS_NAME(CYG_TU_W) = {
+#if CYG_TU_W <= CYG_MAX_W
+    (const void*)cyg_step_kernel<CYG_TU_W, false, false>, (const void*)cyg_step_kernel<CYG_TU_W, false, true>,
+    (const void*)cyg_step_seq_kernel<CYG_TU_W>, (const void*)cyg_step_kernel<CYG_TU_W, true, false>,
+#else
+    (const void*)cyg_step_generic_kernel<CYG_TU_W>, nullptr, nullptr, nullptr,
 #endif
-template <int KW>
-struct WImpl {
-  static cudaError_t set_smem_optin(int max_optin) {
-    if constexpr (KW <= CYG_MAX_W) {
-      cudaError_t e = cudaFuncSetAttribute(cyg_step_kernel<KW, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
-      if (e != cudaSuccess) return e;
-      e = cudaFuncSetAttribute(cyg_step_kernel<KW, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
-      if (e != cudaSuccess) return e;
-      e = cudaFuncSetAttribute(cyg_step_kernel<KW, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
-      if (e != cudaSuccess) return e;
-      return cudaFuncSetAttribute(cyg_step_seq_kernel<KW>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
-    } else {
-      return cudaFuncSetAttribute(cyg_step_generic_kernel<KW>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
-    }
-  }
-  static void step(bool plain, int blocks, int threads, size_t smem, cudaStream_t st, const StepParams& p) {
-    if constexpr (KW <= CYG_MAX_W) {
-      if (!plain) cyg_step_seq_kernel<KW><<<blocks, threads, smem, st>>>(p);
-      else if (!p.logs) cyg_step_kernel<KW, false, false><<<blocks, threads, smem, st>>>(p);
-      else cyg_step_kernel<KW, false, true><<<blocks, threads, smem, st>>>(p);
-    } else {
-      cyg_step_generic_kernel<KW><<<blocks, threads, smem, st>>>(p);
-    }
-  }
-  static void rollout(int blocks, int threads, size_t smem, cudaStream_t st, const StepParams& p) {
-    if constexpr (KW <= CYG_MAX_W) cyg_step_kernel<KW, true, false><<<blocks, threads, smem, st>>>(p);
-  }
-  static void import_state(int blocks, int threads, cudaStream_t st, const ConvParams& p) { cyg_import_kernel<KW><<<blocks, threads, 0, st>>>(p); }
-  static void export_state(int blocks, int threads, cudaStream_t st, const ConvParams& p) { cyg_export_kernel<KW><<<blocks, threads, 0, st>>>(p); }
-  static void randomize(int blocks, int threads, cudaStream_t st, const SimpleParams& p) { cyg_randomize_kernel<KW><<<blocks, threads, 0, st>>>(p); }
-  static void rebuild(int blocks, int threads, cudaStream_t st, const SimpleParams& p) { cyg_rebuild_kernel<KW><<<blocks, threads, 0, st>>>(p); }
-  static void sample(int blocks, int threads, cudaStream_t st, const SimpleParams& p) { cyg_sample_kernel<KW><<<blocks, threads, 0, st>>>(p); }
-  static void observe(int blocks, int threads, cudaStream_t st, const ObsParams& p) { cyg_observe_kernel<KW><<<blocks, threads, 0, st>>>(p); }
-};
-extern "C" const WOps* CYG_WOPS_NAME(CYG_TU_W)(void) {
-  typedef WImpl<CYG_TU_W> I;
-  static const WOps ops = {I::set_smem_optin, I::step, I::rollout, I::import_state, I::export_state, I::randomize, I::rebuild, I::sample, I::observe};
-  return &ops;
-}
+    (const void*)cyg_import_kernel<CYG_TU_W>, (const void*)cyg_export_kernel<CYG_TU_W>, (const void*)cyg_randomize_kernel<CYG_TU_W>,
+    (const void*)cyg_rebuild_kernel<CYG_TU_W>, (const void*)cyg_sample_kernel<CYG_TU_W>, (const void*)cyg_observe_kernel<CYG_TU_W>};
 #else /* ---- the C-ABI translation unit ---- */
-extern "C" {
-void cyg_group_launch(int blocks, int threads, cudaStream_t st, const GroupParams& p);
-void cyg_unpack_launch(int blocks, int threads, cudaStream_t st, const UnpackParams& p);
-void cyg_pack_done_launch(int blocks, int threads, cudaStream_t st, const int32_t* done, uint32_t* bits, int B);
-int cyg_fit_launch(int n_sms, cudaStream_t st, const FitParams& p);
-const WOps* cyg_wops_1(void);
-const WOps* cyg_wops_2(void);
-const WOps* cyg_wops_3(void);
-const WOps* cyg_wops_4(void);
-const WOps* cyg_wops_64(void);
-}
-static const WOps* wops(int W) {
+extern "C" const Kernels cyg_kernels_w1, cyg_kernels_w2, cyg_kernels_w3, cyg_kernels_w4, cyg_kernels_w64;
+static const Kernels& kernels(int W) {
   switch (W) {
-    case 1: return cyg_wops_1();
-    case 2: return cyg_wops_2();
-    case 3: return cyg_wops_3();
-    case 4: return cyg_wops_4();
-    default: return cyg_wops_64();
+    case 1: return cyg_kernels_w1;
+    case 2: return cyg_kernels_w2;
+    case 3: return cyg_kernels_w3;
+    case 4: return cyg_kernels_w4;
+    default: return cyg_kernels_w64;
   }
 }
 
@@ -1175,6 +1111,17 @@ static int cuda_fail(cudaError_t e, const char* what) {
     if (_e != cudaSuccess) return cuda_fail(_e, #call);  \
   } while (0)
 
+/* one kernel launch of an entry point, counted by cyg_launch_count.  It also clears the runtime's last error, so that
+ * a failed launch is reported here and not again by the next caller of cudaGetLastError (torch checks it after its
+ * own launches). */
+static int launch(cyg_env_s* h, const void* kernel, int blocks, int threads, size_t smem, void* stream, void** args) {
+  cudaError_t e = cudaLaunchKernel(kernel, dim3(blocks), dim3(threads), args, smem, (cudaStream_t)stream);
+  h->launches++;
+  const cudaError_t last = cudaGetLastError();
+  if (e == cudaSuccess) e = last;
+  return e == cudaSuccess ? CYG_OK : cuda_fail(e, "cudaLaunchKernel");
+}
+
 struct DeviceGuard {
   int prev;
   bool ok;
@@ -1199,6 +1146,8 @@ static int pick_block_envs(const cyg_env_s* h) {
 }
 
 static int configure_step(cyg_env_s* h) {
+  int max_optin = 0;
+  CU(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
   if (h->W > CYG_MAX_W) { /* large networks: a few envs per CTA so that every SM gets some, records staged in shared memory */
     int per_sm = (h->B + h->n_sms - 1) / h->n_sms;
     const size_t rec_bytes = (size_t)h->net.S * 4;
@@ -1209,19 +1158,34 @@ static int configure_step(cyg_env_s* h) {
     h->NB = per_sm < 1 ? 1 : (per_sm > cap ? cap : per_sm);
     if (h->NB > 128) h->NB = 128;
     h->smem_bytes = (size_t)h->NB * rec_bytes + 16 + (size_t)h->NB * 16 + tab_bytes; /* records, pad, 4 words of phase hand-over per env, hot tables */
-    int max_optin = 0;
-    CU(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
-    CU(wops(h->W)->set_smem_optin(max_optin));
-    return CYG_OK;
+  } else {
+    h->smem_bytes = smem_plan(h->net.hot_words, h->net.S, h->NB).total;
+    if ((int)h->smem_bytes > max_optin) return fail(CYG_E_INVAL, "record block does not fit in shared memory");
   }
-  SmemPlan sp = smem_plan(h->net.hot_words, h->net.S, h->NB);
-  h->smem_bytes = sp.total;
   /* opt in to the device maximum once (handles with different block sizes share the kernel) */
-  int max_optin = 0;
-  CU(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
-  if ((int)sp.total > max_optin) return fail(CYG_E_INVAL, "record block does not fit in shared memory");
-  CU(wops(h->W)->set_smem_optin(max_optin));
+  const Kernels& k = kernels(h->W);
+  for (const void* f : {k.step, k.step_log, k.step_seq, k.rollout})
+    if (f) CU(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin));
   return CYG_OK;
+}
+
+/* cyg_create past its argument checks: the tables, their device copy and the step configuration */
+static int init_handle(cyg_env_s* h, const cyg_config& cfg, const cyg_network& host_net) {
+  std::string err = build_tables(cfg, host_net, h->blob);
+  if (!err.empty()) return fail(CYG_E_INVAL, err);
+  h->W = h->blob.net.W;
+  DeviceGuard g(h->device);
+  if (!g.ok) return fail(CYG_E_CUDA, "cudaSetDevice failed");
+  size_t bytes = h->blob.words.size() * 4;
+  cudaError_t e = cudaMalloc((void**)&h->d_blob, bytes);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(tables)");
+  e = cudaMemcpy(h->d_blob, h->blob.words.data(), bytes, cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpy(tables)");
+  relocate(h->blob, h->d_blob, h->net);
+  cudaDeviceGetAttribute(&h->n_sms, cudaDevAttrMultiProcessorCount, h->device);
+  if (h->n_sms < 1) h->n_sms = 148;
+  h->NB = pick_block_envs(h);
+  return configure_step(h);
 }
 
 extern "C" {
@@ -1236,36 +1200,22 @@ int cyg_create(cyg_handle* out, const cyg_config* cfg, const cyg_network* host_n
   int ndev = 0;
   CU(cudaGetDeviceCount(&ndev));
   if (device < 0 || device >= ndev) return fail(CYG_E_INVAL, "bad CUDA device ordinal");
-  cyg_env_s* h = new (std::nothrow) cyg_env_s();
+  cyg_env_s* h = new (std::nothrow) cyg_env_s(); /* value-initialised: every pointer null, every count 0 */
   if (!h) return fail(CYG_E_NOMEM, "out of host memory");
-  std::string err = build_tables(*cfg, *host_net, h->blob);
-  if (!err.empty()) { delete h; return fail(CYG_E_INVAL, err); }
-  h->B = B; h->env_id0 = env_id0; h->device = device; h->state = nullptr; h->launches = 0; h->bl_env = nullptr; h->bl_rows = 1; h->id_run = 0; h->id_stride = 0;
-  h->det_slots = nullptr; h->det_of_env = nullptr; h->n_det_slots = 0; h->fit_work = nullptr;
-  h->W = h->blob.net.W;
-  DeviceGuard g(device);
-  if (!g.ok) { delete h; return fail(CYG_E_CUDA, "cudaSetDevice failed"); }
-  size_t bytes = h->blob.words.size() * 4;
-  cudaError_t e = cudaMalloc((void**)&h->d_blob, bytes);
-  if (e != cudaSuccess) { delete h; return cuda_fail(e, "cudaMalloc(tables)"); }
-  e = cudaMemcpy(h->d_blob, h->blob.words.data(), bytes, cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) { cudaFree(h->d_blob); delete h; return cuda_fail(e, "cudaMemcpy(tables)"); }
-  relocate(h->blob, h->d_blob, h->net);
-  cudaDeviceGetAttribute(&h->n_sms, cudaDevAttrMultiProcessorCount, device);
-  if (h->n_sms < 1) h->n_sms = 148;
-  h->NB = pick_block_envs(h);
-  int rc = CYG_OK;
-  rc = configure_step(h);
-  if (rc != CYG_OK) { cudaFree(h->d_blob); delete h; return rc; }
+  h->B = B; h->env_id0 = env_id0; h->device = device; h->bl_rows = 1;
+  const int rc = init_handle(h, *cfg, *host_net);
+  if (rc != CYG_OK) { cyg_destroy(h); return rc; }
   *out = h;
   return CYG_OK;
 }
 
 int cyg_destroy(cyg_handle h) {
   if (!h) return CYG_OK;
-  DeviceGuard g(h->device);
-  cudaFree(h->d_blob);
-  if (h->fit_work) cudaFree(h->fit_work);
+  if (h->d_blob) { /* else cyg_create gave up before the handle had device memory */
+    DeviceGuard g(h->device);
+    cudaFree(h->d_blob);
+    if (h->fit_work) cudaFree(h->fit_work);
+  }
   delete h;
   return CYG_OK;
 }
@@ -1331,10 +1281,12 @@ int cyg_fit_detectors(cyg_handle h, const uint32_t* seeds, int32_t* next_slot, v
   DeviceGuard g(h->device);
   FitParams p = {h->state, logs_of(h), const_cast<uint32_t*>(h->det_slots), const_cast<int32_t*>(h->det_of_env), seeds, next_slot,
                  h->fit_work, (int)h->net.S, h->B, h->net.cfg.log_cap, h->n_det_slots};
-  const int e = cyg_fit_launch(h->n_sms, (cudaStream_t)stream, p);
-  h->launches += 2;
-  if (e != 0) return cuda_fail((cudaError_t)e, "cyg_fit_detectors");
-  return CYG_OK;
+  const size_t smem = sizeof(iforest::Scratch) * CYG_FIT_WARPS;
+  CU(cudaFuncSetAttribute(cyg_fit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  void* args[] = {&p};
+  const int rc = launch(h, (const void*)cyg_fit_assign_kernel, 1, 1024, 0, stream, args);
+  if (rc != CYG_OK) return rc;
+  return launch(h, (const void*)cyg_fit_kernel, 3 * h->n_sms, 32 * CYG_FIT_WARPS, smem, stream, args); /* 3 CTAs of 4 Scratch each fit one SM's shared memory */
 }
 
 int cyg_internal_words(cyg_handle h, int64_t* words_per_env) {
@@ -1354,28 +1306,29 @@ static uint32_t* ckpt_of(cyg_handle h) { return h->state + (size_t)h->B * h->net
 static uint32_t* xtra_of(cyg_handle h) { return ckpt_of(h) + (size_t)h->B * h->net.M; }
 static uint32_t* logs_of(cyg_handle h) { return h->net.cfg.log_cap > 0 ? xtra_of(h) + (size_t)h->B * h->net.cfg.xcap : nullptr; }
 
+/* the conversion kernels' parameters: the handle's internal buffers and the caller's canonical state */
+static ConvParams conv_params(cyg_handle h, const cyg_state* c) {
+  return {h->net, h->state, ckpt_of(h), xtra_of(h), c->dev, c->ckpt, c->blocked, c->extra, c->scal, h->B, logs_of(h), c->logs};
+}
+
 int cyg_import_state(cyg_handle h, const cyg_state* c, void* stream) {
   if (!h || !c || !c->dev || !c->blocked || !c->extra || !c->scal) return fail(CYG_E_INVAL, "null argument");
   if (!h->state) return fail(CYG_E_INVAL, "cyg_bind() first");
   DeviceGuard g(h->device);
-  ConvParams p = {h->net, h->state, ckpt_of(h), xtra_of(h), c->dev, c->ckpt, c->blocked, c->extra, c->scal, h->B, logs_of(h), c->logs};
+  ConvParams p = conv_params(h, c);
+  void* args[] = {&p};
   int threads = 128, blocks = (int)(((size_t)h->B * 32 + threads - 1) / threads);
-  wops(h->W)->import_state(blocks, threads, (cudaStream_t)stream, p);
-  h->launches++;
-  CU(cudaGetLastError());
-  return CYG_OK;
+  return launch(h, kernels(h->W).import_state, blocks, threads, 0, stream, args);
 }
 
 int cyg_export_state(cyg_handle h, const cyg_state* c, void* stream) {
   if (!h || !c || !c->dev || !c->blocked || !c->extra || !c->scal) return fail(CYG_E_INVAL, "null argument");
   if (!h->state) return fail(CYG_E_INVAL, "cyg_bind() first");
   DeviceGuard g(h->device);
-  ConvParams p = {h->net, h->state, ckpt_of(h), xtra_of(h), c->dev, c->ckpt, c->blocked, c->extra, c->scal, h->B, logs_of(h), c->logs};
+  ConvParams p = conv_params(h, c);
+  void* args[] = {&p};
   int threads = 128, blocks = (int)(((size_t)h->B * 32 + threads - 1) / threads);
-  wops(h->W)->export_state(blocks, threads, (cudaStream_t)stream, p);
-  h->launches++;
-  CU(cudaGetLastError());
-  return CYG_OK;
+  return launch(h, kernels(h->W).export_state, blocks, threads, 0, stream, args);
 }
 
 /* the fields of a step launch that come from the handle alone; every other field is zero */
@@ -1401,27 +1354,15 @@ static StepGrid step_grid(cyg_handle h) {
   return g;
 }
 
-static int step_impl(cyg_handle h, const cyg_actions* a, int n_steps, uint32_t step_flags, const cyg_step_out* out, void* stream);
-
-int cyg_step(cyg_handle h, const cyg_actions* a, uint32_t step_flags, const cyg_step_out* out, void* stream) {
-  return step_impl(h, a, 1, step_flags, out, stream);
-}
-
-int cyg_step_multi(cyg_handle h, const cyg_actions* a, int32_t n_steps, uint32_t step_flags, const cyg_step_out* out, void* stream) {
-  if (n_steps < 1) return fail(CYG_E_INVAL, "n_steps must be >= 1");
+static int step_impl(cyg_handle h, const cyg_actions* a, int n_steps, uint32_t step_flags, const cyg_step_out* out, void* stream) {
+  if (!h || !a || !out || !a->hdr || !a->mask || !out->raw_reward || !out->shaped_reward || !out->done)
+    return fail(CYG_E_INVAL, "null argument");
   if (n_steps > 1) {
-    if (!h || !a || !out) return fail(CYG_E_INVAL, "null argument");
     if (h->bl_env && h->bl_rows > 1 && h->bl_rows < n_steps) return fail(CYG_E_INVAL, "cyg_step_multi: fewer base_line rows than steps");
     if ((step_flags & CYG_STEP_GROUPED) || a->order || a->n_groups != 1) return fail(CYG_E_INVAL, "cyg_step_multi: plain steps only (no groups, no order array)");
     if (out->obs || out->pre_masks) return fail(CYG_E_INVAL, "cyg_step_multi: no obs / pre_masks outputs");
     if (h->W > CYG_MAX_W) return fail(CYG_E_INVAL, "cyg_step_multi: networks of at most 128 device slots");
   }
-  return step_impl(h, a, n_steps, step_flags, out, stream);
-}
-
-static int step_impl(cyg_handle h, const cyg_actions* a, int n_steps, uint32_t step_flags, const cyg_step_out* out, void* stream) {
-  if (!h || !a || !out || !a->hdr || !a->mask || !out->raw_reward || !out->shaped_reward || !out->done)
-    return fail(CYG_E_INVAL, "null argument");
   if (!h->state) return fail(CYG_E_INVAL, "cyg_bind() first");
   if (h->id_run > 0) return fail(CYG_E_INVAL, "strided env ids (cyg_set_env_id_stride): cyg_rollout only");
   const bool grouped = (step_flags & CYG_STEP_GROUPED) != 0;
@@ -1439,14 +1380,24 @@ static int step_impl(cyg_handle h, const cyg_actions* a, int n_steps, uint32_t s
   p.flags = step_flags;
   p.T = n_steps;
   p.n_rows = h->B;
-  const bool plain = !(step_flags & CYG_STEP_GROUPED) && a->order == nullptr; /* cyg_step_kernel; else cyg_step_seq_kernel */
+  const bool plain = !grouped && a->order == nullptr; /* cyg_step_kernel; else cyg_step_seq_kernel */
+  const Kernels& k = kernels(h->W);
+  const void* kernel = h->W > CYG_MAX_W ? k.step : !plain ? k.step_seq : p.logs ? k.step_log : k.step;
+  void* args[] = {&p};
   const StepGrid grid = step_grid(h);
-  wops(h->W)->step(plain, grid.blocks, grid.threads, h->smem_bytes, (cudaStream_t)stream, p);
-  h->launches++;
-  CU(cudaGetLastError());
+  const int rc = launch(h, kernel, grid.blocks, grid.threads, h->smem_bytes, stream, args);
   /* large networks: the post-evolve observation rows are a second launch */
-  if (h->W > CYG_MAX_W && out->obs) return cyg_observe(h, out->obs_mode, out->obs, stream);
-  return CYG_OK;
+  if (rc == CYG_OK && h->W > CYG_MAX_W && out->obs) return cyg_observe(h, out->obs_mode, out->obs, stream);
+  return rc;
+}
+
+int cyg_step(cyg_handle h, const cyg_actions* a, uint32_t step_flags, const cyg_step_out* out, void* stream) {
+  return step_impl(h, a, 1, step_flags, out, stream);
+}
+
+int cyg_step_multi(cyg_handle h, const cyg_actions* a, int32_t n_steps, uint32_t step_flags, const cyg_step_out* out, void* stream) {
+  if (n_steps < 1) return fail(CYG_E_INVAL, "n_steps must be >= 1");
+  return step_impl(h, a, n_steps, step_flags, out, stream);
 }
 
 int cyg_rollout(cyg_handle h, const cyg_rollout_args* a, uint32_t step_flags, void* stream) {
@@ -1466,35 +1417,39 @@ int cyg_rollout(cyg_handle h, const cyg_rollout_args* a, uint32_t step_flags, vo
   p.G = 1; p.flags = step_flags; p.T = a->n_steps;
   p.row_base = a->row_base; p.envs_per_row = a->envs_per_row; p.n_rows = a->n_rows; p.ret_acc = a->returns;
   p.id_run = h->id_run; p.id_stride = h->id_stride; p.block_order = a->block_order;
+  void* args[] = {&p};
   const StepGrid grid = step_grid(h);
-  wops(h->W)->rollout(grid.blocks, grid.threads, h->smem_bytes, (cudaStream_t)stream, p);
-  h->launches++;
-  CU(cudaGetLastError());
-  return CYG_OK;
+  return launch(h, kernels(h->W).rollout, grid.blocks, grid.threads, h->smem_bytes, stream, args);
+}
+
+/* the fields of a randomize / rebuild / sample launch that come from the handle alone; every other field is zero */
+static SimpleParams simple_params(cyg_handle h) {
+  SimpleParams p{};
+  p.net = h->net; p.recs = h->state; p.xtra = xtra_of(h);
+  p.B = h->B; p.env_id0 = h->env_id0; p.id_run = h->id_run; p.id_stride = h->id_stride;
+  return p;
 }
 
 int cyg_randomize(cyg_handle h, const uint8_t* env_mask, void* stream) {
   if (!h) return fail(CYG_E_INVAL, "null handle");
   if (!h->state) return fail(CYG_E_INVAL, "cyg_bind() first");
   DeviceGuard g(h->device);
-  SimpleParams p = {h->net, h->state, xtra_of(h), env_mask, nullptr, nullptr, h->B, h->env_id0, 0, nullptr, 0, h->id_run, h->id_stride};
+  SimpleParams p = simple_params(h);
+  p.env_mask = env_mask;
+  void* args[] = {&p};
   int threads = 128, blocks = (h->B + threads - 1) / threads;
-  wops(h->W)->randomize(blocks, threads, (cudaStream_t)stream, p);
-  h->launches++;
-  CU(cudaGetLastError());
-  return CYG_OK;
+  return launch(h, kernels(h->W).randomize, blocks, threads, 0, stream, args);
 }
 
 int cyg_rebuild_graph_cache(cyg_handle h, const uint8_t* env_mask, void* stream) {
   if (!h) return fail(CYG_E_INVAL, "null handle");
   if (!h->state) return fail(CYG_E_INVAL, "cyg_bind() first");
   DeviceGuard g(h->device);
-  SimpleParams p = {h->net, h->state, xtra_of(h), env_mask, nullptr, nullptr, h->B, h->env_id0, 0, nullptr, 0, h->id_run, h->id_stride};
+  SimpleParams p = simple_params(h);
+  p.env_mask = env_mask;
+  void* args[] = {&p};
   int threads = 128, blocks = (h->B + threads - 1) / threads;
-  wops(h->W)->rebuild(blocks, threads, (cudaStream_t)stream, p);
-  h->launches++;
-  CU(cudaGetLastError());
-  return CYG_OK;
+  return launch(h, kernels(h->W).rebuild, blocks, threads, 0, stream, args);
 }
 
 int cyg_sample_actions(cyg_handle h, int32_t mode, uint32_t* hdr, uint32_t* mask, void* stream) {
@@ -1508,12 +1463,11 @@ int cyg_sample_actions_ordered(cyg_handle h, int32_t mode, uint32_t* hdr, uint32
   if (!h->state) return fail(CYG_E_INVAL, "cyg_bind() first");
   if (mode != CYG_MODE_DEFENDER && mode != CYG_MODE_ATTACKER) return fail(CYG_E_INVAL, "mode must be 0 or 1");
   DeviceGuard g(h->device);
-  SimpleParams p = {h->net, h->state, xtra_of(h), nullptr, hdr, mask, h->B, h->env_id0, mode, order, order_stride, h->id_run, h->id_stride};
+  SimpleParams p = simple_params(h);
+  p.hdr = hdr; p.mask = mask; p.mode = mode; p.order = order; p.order_stride = order_stride;
+  void* args[] = {&p};
   int threads = 128, blocks = (h->B + threads - 1) / threads;
-  wops(h->W)->sample(blocks, threads, (cudaStream_t)stream, p);
-  h->launches++;
-  CU(cudaGetLastError());
-  return CYG_OK;
+  return launch(h, kernels(h->W).sample, blocks, threads, 0, stream, args);
 }
 
 int cyg_observe(cyg_handle h, int32_t obs_mode, float* obs, void* stream) {
@@ -1522,14 +1476,12 @@ int cyg_observe(cyg_handle h, int32_t obs_mode, float* obs, void* stream) {
   if (obs_mode < 1 || obs_mode > 3) return fail(CYG_E_INVAL, "obs_mode must be 1..3");
   DeviceGuard g(h->device);
   ObsParams p = {h->net, h->state, obs, h->B, obs_mode};
+  void* args[] = {&p};
   int threads = 256;
   size_t total = (size_t)h->B * (obs_mode == 2 ? 4 * h->net.M + h->net.cfg.X : 6 * h->net.M);
   int blocks = (int)((total + threads - 1) / threads);
   if (blocks > 148 * 16) blocks = 148 * 16;
-  wops(h->W)->observe(blocks, threads, (cudaStream_t)stream, p);
-  h->launches++;
-  CU(cudaGetLastError());
-  return CYG_OK;
+  return launch(h, kernels(h->W).observe, blocks, threads, 0, stream, args);
 }
 
 int cyg_unpack_actions(cyg_handle h, const uint32_t* rows, uint32_t* hdr, uint32_t* mask, void* stream) {
@@ -1538,21 +1490,17 @@ int cyg_unpack_actions(cyg_handle h, const uint32_t* rows, uint32_t* hdr, uint32
   if (h->net.M > 254) return fail(CYG_E_INVAL, "compact action rows: networks of at most 254 device slots");
   DeviceGuard g(h->device);
   UnpackParams p = {rows, hdr, mask, h->B, h->net.Wm};
+  void* args[] = {&p};
   const int threads = 256, blocks = (h->B + threads - 1) / threads;
-  cyg_unpack_launch(blocks, threads, (cudaStream_t)stream, p);
-  h->launches++;
-  CU(cudaGetLastError());
-  return CYG_OK;
+  return launch(h, (const void*)cyg_unpack_kernel, blocks, threads, 0, stream, args);
 }
 
 int cyg_pack_done(cyg_handle h, const int32_t* done, uint32_t* bits, void* stream) {
   if (!h || !done || !bits) return fail(CYG_E_INVAL, "null argument");
   DeviceGuard g(h->device);
+  void* args[] = {&done, &bits, &h->B};
   const int threads = 256, blocks = (h->B + threads - 1) / threads;
-  cyg_pack_done_launch(blocks, threads, (cudaStream_t)stream, done, bits, h->B);
-  h->launches++;
-  CU(cudaGetLastError());
-  return CYG_OK;
+  return launch(h, (const void*)cyg_pack_done_kernel, blocks, threads, 0, stream, args);
 }
 
 int cyg_group_actions(cyg_handle h, int32_t mode, int32_t role, const int32_t* per_dev_types, const uint8_t* visible, const int32_t* exp_idx,
@@ -1564,11 +1512,9 @@ int cyg_group_actions(cyg_handle h, int32_t mode, int32_t role, const int32_t* p
   if (((uintptr_t)hdr) & 15) return fail(CYG_E_INVAL, "hdr must be 16-byte aligned");
   DeviceGuard g(h->device);
   GroupParams p = {h->net, h->state, per_dev_types, exp_idx, app_idx, visible, single_choice, hdr, mask, h->B, mode, role, n_types, noop};
+  void* args[] = {&p};
   const int threads = 128, blocks = (int)(((size_t)h->B * 32 + threads - 1) / threads);
-  cyg_group_launch(blocks, threads, (cudaStream_t)stream, p);
-  h->launches++;
-  CU(cudaGetLastError());
-  return CYG_OK;
+  return launch(h, (const void*)cyg_group_kernel, blocks, threads, 0, stream, args);
 }
 
 int64_t cyg_launch_count(cyg_handle h) { return h ? h->launches : 0; }

@@ -707,7 +707,7 @@ struct Env {
         }
       }
       cost += -1.0 * ds;
-      if (scal(CYG_S_LOGS) > 0) /* detector.train(last <= 2000 logs): the fit is scikit-learn's, on the host (cygym_b200/detector.py) */
+      if (scal(CYG_S_LOGS) > 0) /* detector.train(last <= 2000 logs): pending until a fit between launches (cyg_fit_detectors, or detector.py on the host) */
         scal(CYG_S_FLAGS) |= CYG_FL_DET_TRAINED | (n->cfg.turbo ? 0u : CYG_FL_DET_PENDING);
     } else if (atype == 11) {
       int d = first_dev(a); /* the host raises ValueError when n_dev == 0 (volt:965-966) */

@@ -12,8 +12,8 @@
  *   home by warp-wide copies.
  * cyg_step_seq_kernel<W>: grouped steps and explicit order lists, one thread-per-env pass, one bulk store of the block.
  * cyg_step_generic_kernel<W>: networks beyond 128 device slots (tables too large for shared memory).
- * cyg_fit_assign_kernel + cyg_fit_kernel: the detector fit of defender action 10 (cyg_iforest.cuh), one warp per
- *   pending env.
+ * cyg_fit_count_kernel + cyg_fit_assign_kernel + cyg_fit_kernel: the detector fit of defender action 10
+ *   (cyg_iforest.cuh): slot assignment in env order over the whole grid, then one warp per pending env.
  * Host side: each plane width's translation unit exports the handles of its kernels in one table (Kernels); the C-ABI
  *   unit holds the kernels that do not depend on the width, and every entry point launches through launch().
  * No tensor cores: the path has no dense contraction.  No CPU fallback anywhere in this file.
@@ -294,7 +294,8 @@ __host__ __device__ inline SmemPlan smem_plan(uint32_t hot_words, int S, int NB)
  * step (registers) although no step ever takes those branches. */
 /* LOG: the env keeps a hop-log ring and may hold a trained detector (cfg.log_cap > 0): the lateral-movement scan writes
  * its hops, scans consult the detector.  Also its own instantiation (the handles that keep only the log's length --
- * every throughput run -- take the kernel without that code: ~1 us per step). */
+ * every throughput run -- take the kernel without that code: ~1 us per step).  ROLL and LOG together: cyg_rollout on a
+ * handle with a ring.  The ring and det_of_env are indexed by slot, the draw streams and action rows by env id. */
 template <int W, bool ROLL, bool LOG>
 __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(const __grid_constant__ StepParams p) {
   unsigned char* smem = reinterpret_cast<unsigned char*>(cyg_smem);
@@ -947,15 +948,27 @@ struct FitParams {
   int32_t* det_of_env;     /* [B] */
   const uint32_t* seeds;   /* [B] */
   int32_t* next_slot;      /* first free slot */
-  int32_t* work;           /* [2 + B]: envs to fit, the fit kernel's cursor, their list */
+  int32_t* work;           /* fit_work_words(B): envs to fit, the fit kernel's cursor, their list, the assignment's counts */
   int S, B, log_cap, n_slots;
 };
 #define CYG_FIT_WARPS 4 /* fitting warps per CTA (cyg_iforest::Scratch each, in shared memory) */
-/* Block-wide exclusive count of `v` over the threads below this one; *total = count over the block. */
-__device__ __forceinline__ int block_rank(bool v, int* warp_tot, int* total) {
+/* slot assignment: a CTA walks a chunk of CYG_ASSIGN_CHUNK consecutive envs, CYG_ASSIGN_ENVS consecutive ones per thread */
+#define CYG_ASSIGN_THREADS 256
+#define CYG_ASSIGN_ENVS 8
+#define CYG_ASSIGN_CHUNK (CYG_ASSIGN_THREADS * CYG_ASSIGN_ENVS)
+/* work words of cyg_fit_detectors for B envs: [0] listed envs, [1] the fit kernel's cursor, [2, 2 + B) the list, then
+ * the count of envs that need a new slot in every assignment chunk, then the first free slot as the call found it */
+static inline size_t fit_work_words(int B) { return 2 + (size_t)B + (size_t)(B + CYG_ASSIGN_CHUNK - 1) / CYG_ASSIGN_CHUNK + 1; }
+/* Block-wide exclusive sum of `v` over the threads below this one; *total = the sum over the block. */
+__device__ __forceinline__ int block_excl_sum(int v, int* warp_tot, int* total) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = (blockDim.x + 31) >> 5;
-  const uint32_t m = __ballot_sync(0xFFFFFFFFu, v);
-  if (lane == 0) warp_tot[warp] = __popc(m);
+  int x = v;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const int y = __shfl_up_sync(0xFFFFFFFFu, x, d);
+    if (lane >= d) x += y;
+  }
+  if (lane == 31) warp_tot[warp] = x;
   __syncthreads();
   int before = 0, all = 0;
   for (int w = 0; w < nwarps; w++) {
@@ -964,46 +977,95 @@ __device__ __forceinline__ int block_rank(bool v, int* warp_tot, int* total) {
   }
   __syncthreads();
   *total = all;
-  return before + __popc(m & ((1u << lane) - 1u));
+  return before + x - v;
 }
-/* One CTA walks the envs in order: slots go to pending envs without one in env order (deterministic, and the same
- * order service_detectors() uses); the envs that can be fitted are listed for cyg_fit_kernel. */
-__global__ void __launch_bounds__(1024) cyg_fit_assign_kernel(const __grid_constant__ FitParams p) {
-  __shared__ int warp_tot[32];
-  const int first = *p.next_slot;
-  int taken = 0, listed = 0;
-  for (int c = 0; c < p.B; c += blockDim.x) {
-    const int b = c + (int)threadIdx.x;
-    bool pend = false, fits_ring = false;
-    int cur = -1;
-    uint32_t flags = 0;
-    if (b < p.B) {
-      const uint32_t* sc = p.recs + (size_t)b * p.S;
-      flags = sc[CYG_S_FLAGS];
-      pend = (flags & CYG_FL_DET_PENDING) != 0;
-      if (pend) {
-        const uint32_t nl = sc[CYG_S_LOGS];
-        const uint32_t win = nl < (uint32_t)CYG_DET_WINDOW ? nl : (uint32_t)CYG_DET_WINDOW;
-        fits_ring = p.logs != nullptr && win >= 1u && win <= (uint32_t)p.log_cap;
-        cur = p.det_of_env[b];
-      }
-    }
-    const bool need = pend && fits_ring && cur < 0;
-    int n_need, n_ok;
-    const int slot = first + taken + block_rank(need, warp_tot, &n_need);
-    const bool ok = pend && fits_ring && (cur >= 0 || slot < p.n_slots);
-    const int at = listed + block_rank(ok, warp_tot, &n_ok);
-    if (need && slot < p.n_slots) p.det_of_env[b] = slot;
-    if (pend && !ok) p.recs[(size_t)b * p.S + CYG_S_FLAGS] = flags | CYG_FL_ERR_DETECTOR;
-    if (ok) p.work[2 + at] = b;
-    taken += n_need;
-    listed += n_ok;
+/* what the assignment reads of env b: its flags, whether it is pending, whether its ring holds the records the fit
+ * reads, and (pending envs only) its slot */
+struct FitEnv {
+  uint32_t flags;
+  int cur;
+  bool pend, fits_ring;
+  __device__ __forceinline__ bool need() const { return pend && fits_ring && cur < 0; } /* takes a new slot */
+};
+__device__ __forceinline__ FitEnv fit_env(const FitParams& p, int b) {
+  FitEnv e{0u, -1, false, false};
+  if (b >= p.B) return e;
+  const uint32_t* sc = p.recs + (size_t)b * p.S;
+  e.flags = sc[CYG_S_FLAGS];
+  e.pend = (e.flags & CYG_FL_DET_PENDING) != 0;
+  if (e.pend) {
+    const uint32_t nl = sc[CYG_S_LOGS];
+    const uint32_t win = nl < (uint32_t)CYG_DET_WINDOW ? nl : (uint32_t)CYG_DET_WINDOW;
+    e.fits_ring = p.logs != nullptr && win >= 1u && win <= (uint32_t)p.log_cap;
+    e.cur = p.det_of_env[b];
   }
+  return e;
+}
+/* Slots go to pending envs without one in env order (deterministic, and the same order service_detectors() uses); the
+ * envs that can be fitted are listed for cyg_fit_kernel.  Two passes over the whole grid, so that a batch of 2^20 envs
+ * is walked by every SM: (1) each CTA counts the envs of its chunk that need a slot; (2) each CTA adds up the counts of
+ * the chunks before it, ranks its own envs and assigns. */
+__global__ void __launch_bounds__(CYG_ASSIGN_THREADS) cyg_fit_count_kernel(const __grid_constant__ FitParams p) {
+  __shared__ int warp_tot[32];
+  const int b0 = (int)blockIdx.x * CYG_ASSIGN_CHUNK + (int)threadIdx.x * CYG_ASSIGN_ENVS;
+  int n = 0;
+#pragma unroll
+  for (int k = 0; k < CYG_ASSIGN_ENVS; k++) n += fit_env(p, b0 + k).need() ? 1 : 0;
+  int total;
+  block_excl_sum(n, warp_tot, &total);
   if (threadIdx.x == 0) {
-    const int next = first + taken;
+    int32_t* chunk_need = p.work + 2 + p.B;
+    chunk_need[blockIdx.x] = total;
+    if (blockIdx.x == 0) {
+      chunk_need[gridDim.x] = *p.next_slot; /* pass 2 reads the first free slot from here while its last CTA moves *next_slot */
+      p.work[0] = 0;
+      p.work[1] = 0;
+    }
+  }
+}
+__global__ void __launch_bounds__(CYG_ASSIGN_THREADS) cyg_fit_assign_kernel(const __grid_constant__ FitParams p) {
+  __shared__ int warp_tot[32];
+  const int32_t* chunk_need = p.work + 2 + p.B;
+  const int first = chunk_need[gridDim.x];
+  int before = 0, in_chunk = 0;
+  for (int c = (int)threadIdx.x; c < (int)blockIdx.x; c += blockDim.x) before += chunk_need[c];
+  block_excl_sum(before, warp_tot, &before); /* slots taken by the chunks before this one */
+  const int b0 = (int)blockIdx.x * CYG_ASSIGN_CHUNK + (int)threadIdx.x * CYG_ASSIGN_ENVS;
+  FitEnv e[CYG_ASSIGN_ENVS];
+  int n = 0;
+#pragma unroll
+  for (int k = 0; k < CYG_ASSIGN_ENVS; k++) {
+    e[k] = fit_env(p, b0 + k);
+    n += e[k].need() ? 1 : 0;
+  }
+  int slot = first + before + block_excl_sum(n, warp_tot, &in_chunk);
+  uint32_t ok_bits = 0;
+#pragma unroll
+  for (int k = 0; k < CYG_ASSIGN_ENVS; k++) {
+    const int b = b0 + k;
+    const bool ok = e[k].pend && e[k].fits_ring && (e[k].cur >= 0 || slot < p.n_slots);
+    if (e[k].need()) {
+      if (slot < p.n_slots) p.det_of_env[b] = slot;
+      slot++;
+    }
+    if (e[k].pend && !ok) p.recs[(size_t)b * p.S + CYG_S_FLAGS] = e[k].flags | CYG_FL_ERR_DETECTOR;
+    ok_bits |= (ok ? 1u : 0u) << k;
+  }
+  /* the order of the list does not matter (every fit is independent): one atomic per warp that lists any env */
+  const int lane = threadIdx.x & 31, n_ok = __popc(ok_bits);
+  int x = n_ok;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const int y = __shfl_up_sync(0xFFFFFFFFu, x, d);
+    if (lane >= d) x += y;
+  }
+  int base = 0;
+  if (lane == 31 && x > 0) base = atomicAdd(&p.work[0], x);
+  int at = __shfl_sync(0xFFFFFFFFu, base, 31) + x - n_ok;
+  for (uint32_t m = ok_bits; m; m &= m - 1u) p.work[2 + at++] = b0 + __ffs((int)m) - 1;
+  if (blockIdx.x == gridDim.x - 1 && threadIdx.x == 0) {
+    const int next = first + before + in_chunk;
     *p.next_slot = next <= p.n_slots ? next : (first > p.n_slots ? first : p.n_slots);
-    p.work[0] = listed;
-    p.work[1] = 0;
   }
 }
 /* Persistent warps take the listed envs one by one: lane 0 runs the serial fit (streams, row sampling, tree builds)
@@ -1052,7 +1114,7 @@ __global__ void cyg_observe_kernel(const __grid_constant__ ObsParams p) {
  * through launch() below).
  * ======================================================================== */
 struct Kernels {
-  const void *step, *step_log, *step_seq, *rollout; /* W = 64: cyg_step_generic_kernel in `step`, the other forms null */
+  const void *step, *step_log, *step_seq, *rollout, *rollout_log; /* W = 64: cyg_step_generic_kernel in `step`, the other forms null */
   const void *import_state, *export_state, *randomize, *rebuild, *sample, *observe;
 };
 #define CYG_KERNELS_NAME2(w) cyg_kernels_w##w
@@ -1063,8 +1125,9 @@ extern "C" const Kernels CYG_KERNELS_NAME(CYG_TU_W) = {
 #if CYG_TU_W <= CYG_MAX_W
     (const void*)cyg_step_kernel<CYG_TU_W, false, false>, (const void*)cyg_step_kernel<CYG_TU_W, false, true>,
     (const void*)cyg_step_seq_kernel<CYG_TU_W>, (const void*)cyg_step_kernel<CYG_TU_W, true, false>,
+    (const void*)cyg_step_kernel<CYG_TU_W, true, true>,
 #else
-    (const void*)cyg_step_generic_kernel<CYG_TU_W>, nullptr, nullptr, nullptr,
+    (const void*)cyg_step_generic_kernel<CYG_TU_W>, nullptr, nullptr, nullptr, nullptr,
 #endif
     (const void*)cyg_import_kernel<CYG_TU_W>, (const void*)cyg_export_kernel<CYG_TU_W>, (const void*)cyg_randomize_kernel<CYG_TU_W>,
     (const void*)cyg_rebuild_kernel<CYG_TU_W>, (const void*)cyg_sample_kernel<CYG_TU_W>, (const void*)cyg_observe_kernel<CYG_TU_W>};
@@ -1092,7 +1155,7 @@ struct cyg_env_s {
   const uint32_t* det_slots; /* uploaded detectors (device memory of the caller) */
   const int32_t* det_of_env;
   int n_det_slots;
-  int32_t* fit_work; /* [2 + B] device words of cyg_fit_detectors (allocated with the detector slots) */
+  int32_t* fit_work; /* fit_work_words(B) device words of cyg_fit_detectors (allocated with the detector slots) */
   const uint8_t* bl_env;
   int bl_rows;       /* rows of [B] codes behind bl_env (cyg_set_base_line_per_env_steps; 1 otherwise) */
   int id_run, id_stride; /* cyg_set_env_id_stride (0: env id = env_id0 + slot) */
@@ -1164,7 +1227,7 @@ static int configure_step(cyg_env_s* h) {
   }
   /* opt in to the device maximum once (handles with different block sizes share the kernel) */
   const Kernels& k = kernels(h->W);
-  for (const void* f : {k.step, k.step_log, k.step_seq, k.rollout})
+  for (const void* f : {k.step, k.step_log, k.step_seq, k.rollout, k.rollout_log})
     if (f) CU(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin));
   return CYG_OK;
 }
@@ -1262,7 +1325,7 @@ int cyg_set_detectors(cyg_handle h, const uint32_t* slots, int32_t n_slots, cons
   if ((slots == nullptr) != (det_of_env == nullptr) || (slots && n_slots < 1)) return fail(CYG_E_INVAL, "slots and det_of_env go together");
   if (slots && !h->fit_work) {
     DeviceGuard g(h->device);
-    CU(cudaMalloc((void**)&h->fit_work, sizeof(int32_t) * (2 + (size_t)h->B)));
+    CU(cudaMalloc((void**)&h->fit_work, sizeof(int32_t) * fit_work_words(h->B)));
   }
   h->det_slots = slots;
   h->det_of_env = det_of_env;
@@ -1284,7 +1347,9 @@ int cyg_fit_detectors(cyg_handle h, const uint32_t* seeds, int32_t* next_slot, v
   const size_t smem = sizeof(iforest::Scratch) * CYG_FIT_WARPS;
   CU(cudaFuncSetAttribute(cyg_fit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   void* args[] = {&p};
-  const int rc = launch(h, (const void*)cyg_fit_assign_kernel, 1, 1024, 0, stream, args);
+  const int chunks = (h->B + CYG_ASSIGN_CHUNK - 1) / CYG_ASSIGN_CHUNK;
+  int rc = launch(h, (const void*)cyg_fit_count_kernel, chunks, CYG_ASSIGN_THREADS, 0, stream, args);
+  if (rc == CYG_OK) rc = launch(h, (const void*)cyg_fit_assign_kernel, chunks, CYG_ASSIGN_THREADS, 0, stream, args);
   if (rc != CYG_OK) return rc;
   return launch(h, (const void*)cyg_fit_kernel, 3 * h->n_sms, 32 * CYG_FIT_WARPS, smem, stream, args); /* 3 CTAs of 4 Scratch each fit one SM's shared memory */
 }
@@ -1404,7 +1469,6 @@ int cyg_rollout(cyg_handle h, const cyg_rollout_args* a, uint32_t step_flags, vo
   if (!h || !a || !a->hdr || !a->mask || !a->returns) return fail(CYG_E_INVAL, "null argument");
   if (!h->state) return fail(CYG_E_INVAL, "cyg_bind() first");
   if (h->W > CYG_MAX_W) return fail(CYG_E_INVAL, "cyg_rollout: networks of at most 128 device slots");
-  if (h->net.cfg.log_cap > 0) return fail(CYG_E_INVAL, "cyg_rollout: handles with a hop-log ring (log_cap > 0) step through cyg_step");
   if (a->n_steps < 1 || a->n_rows < 1 || a->envs_per_row < 1 || a->row_base < 0 || a->row_base + h->B > 0x7FFFFFFFll) return fail(CYG_E_INVAL, "cyg_rollout: bad sizes");
   const int64_t last_idx = h->id_run > 0 ? (int64_t)strided_index((uint32_t)(h->B - 1), (uint32_t)h->id_run, (uint32_t)h->id_stride) : (int64_t)h->B - 1;
   if (a->row_base + last_idx > 0x7FFFFFFFll || (a->row_base + last_idx) / a->envs_per_row >= a->n_rows) return fail(CYG_E_INVAL, "cyg_rollout: an env's action row is beyond n_rows");
@@ -1419,7 +1483,8 @@ int cyg_rollout(cyg_handle h, const cyg_rollout_args* a, uint32_t step_flags, vo
   p.id_run = h->id_run; p.id_stride = h->id_stride; p.block_order = a->block_order;
   void* args[] = {&p};
   const StepGrid grid = step_grid(h);
-  return launch(h, kernels(h->W).rollout, grid.blocks, grid.threads, h->smem_bytes, stream, args);
+  const Kernels& k = kernels(h->W);
+  return launch(h, p.logs ? k.rollout_log : k.rollout, grid.blocks, grid.threads, h->smem_bytes, stream, args);
 }
 
 /* the fields of a randomize / rebuild / sample launch that come from the handle alone; every other field is zero */

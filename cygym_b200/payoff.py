@@ -8,6 +8,12 @@ independent, so they shard over ranks with no per-step collective: rank r runs r
 [r*N/world, (r+1)*N/world) of every pair and holds a partial [n_def, n_att, 10] sum; ONE
 all-reduce(sum) of that tensor (NCCL over NVLink on GPUs, gloo in the CPU tests) finishes the
 evaluation.  The 10 columns are simulate_game's return tuple (do_agent.py:2078-2089).
+
+Defender action 10 trains the env's IsolationForest and a later action 5 scans with it (volt:945-962, :1020-1069).  Both
+evaluators serve strategies that train only with train_detectors=True: the envs then keep a hop-log ring and detector
+slots, and every pending env is fitted on the device between turns (VectorCyberDefenseEnv.fit_detectors, seeded by
+detector_fit_seeds()).  Without it, a strategy that trains gets the stub scan -- no un-compromise, no stall -- and a
+sticky CYG_FL_ERR_DETECTOR bit on the env, which the default path does not read.
 """
 import numpy as np
 
@@ -19,6 +25,9 @@ _INFO_OF_COLUMN = ("Compromised_devices", "work_done", "Scan_count", "defensive_
                    "Edges Blocked", "Edges Added")  # env.info() keys of COLUMNS[2:]
 # the counters the reference zeroes before a rollout (do_agent.py:2038-2045)
 _ROLLOUT_RESET = (K.S_STEP, K.S_DEF_STEP, K.S_ATT_STEP, K.S_WORK, K.S_CKPT, K.S_DEFCOST, K.S_CLEANCOST, K.S_REVERT, K.S_SCAN)
+DETECTOR_LOG_CAP = K.DET_WINDOW  # hop-log records per env with train_detectors=True: the most a fit or a scan reads
+_ERR_NAMES = ((K.FL_ERR_BUSY, "CYG_FL_ERR_BUSY"), (K.FL_ERR_XCAP, "CYG_FL_ERR_XCAP"), (K.FL_ERR_DETECTOR, "CYG_FL_ERR_DETECTOR"),
+              (0x80, "error bit 0x80"))
 
 
 def _columns(def_r, att_r, info):
@@ -29,12 +38,20 @@ def _columns(def_r, att_r, info):
 class Strategy:
     """The flavours of strategy.Strategy the evaluators serve: baseline_name | actions (fixed sequence) | actor (a torch
     module: the parametric DDPG best responses, Actor of do_agent.py:357-371; evaluate_payoff_matrix_batched only) |
-    none of them (no-op)."""
+    none of them (no-op).  A defender sequence with a type-10 action, and any defender actor (its type slice may pick
+    10), trains the detector: evaluate such strategies with train_detectors=True, or their scans run the stub and leave
+    CYG_FL_ERR_DETECTOR on the env."""
 
     def __init__(self, baseline_name=None, actions=None, actor=None):
         self.baseline_name = baseline_name
         self.actions = list(actions) if actions is not None else None
         self.actor = actor
+
+    def can_train(self):
+        """Whether this strategy, as the defender, may execute action 10 (train the detector).  A baseline never does."""
+        if self.actor is not None:
+            return True
+        return self.baseline_name is None and any(a is not None and int(a[0]) == 10 for a in (self.actions or ()))
 
     def decide(self, t_step):
         """(action, base_line to set or None) -- _strategy_decide_action (do_agent.py:707-764)."""
@@ -54,6 +71,43 @@ def shard_range(total, rank, world):
     return lo, lo + base + (1 if rank < extra else 0)
 
 
+def detector_fit_seeds(seed, env_ids, turn):
+    """The seed of the detector fit of every env after turn `turn`: int64 tensor [n] of uint32 values (what
+    fit_detectors() takes), on env_ids' device.  env_ids: int64 tensor of evaluation env ids g = pair * n_rollouts +
+    rollout.  The reference fits with random_state=None, i.e. from numpy's global stream as it stands, so any fixed rule
+    is a valid sample of its behaviour; this one depends on (seed, g, turn) alone -- not on the rank, the number of
+    ranks, steps_per_launch or the evaluator -- so that every layout of an evaluation gives the same result."""
+    import torch
+    M = 0xFFFFFFFF
+
+    def mul32(h, c):  # (h * c) mod 2^32 with every product below 2^48 (no int64 overflow)
+        return ((h & 0xFFFF) * c + ((((h >> 16) * c) & 0xFFFF) << 16)) & M
+
+    def fmix(h):  # MurmurHash3's 32-bit finaliser
+        h = h ^ (h >> 16)
+        h = mul32(h, 0x85EBCA6B)
+        h = h ^ (h >> 13)
+        h = mul32(h, 0xC2B2AE35)
+        return h ^ (h >> 16)
+
+    g = torch.as_tensor(env_ids).to(torch.int64)
+    h = fmix(torch.full_like(g, (int(seed) + 0x9E3779B9) & M))
+    h = fmix(h ^ (g & M))
+    h = fmix(h ^ ((g >> 32) & M))
+    return fmix(h ^ ((int(turn) + 0x7F4A7C15) & M))
+
+
+def _check_error_bits(flags_of_envs):
+    """train_detectors=True: raise when an env ended with a sticky CYG_FL_ERR_* bit (a scan without a fitted detector,
+    a full busy set or extra-edge list), naming the bits and how many envs carry each."""
+    import torch
+    err = torch.cat([f.reshape(-1) & K.FL_ERR_MASK for f in flags_of_envs]) if flags_of_envs else None
+    if err is None or not bool(err.any()):
+        return
+    found = [f"{name} on {int(((err & bit) != 0).sum())} envs" for bit, name in _ERR_NAMES if bool(((err & bit) != 0).any())]
+    raise RuntimeError("payoff evaluation with train_detectors=True: envs ended with sticky error bits: " + ", ".join(found))
+
+
 def reduce_payoff(partial_sums, n_rollouts, steps_per_episode, group=None):
     """All-reduce the per-rank [n_def, n_att, 10] sums and turn them into simulate_game's averages."""
     import torch
@@ -67,21 +121,31 @@ def reduce_payoff(partial_sums, n_rollouts, steps_per_episode, group=None):
 
 
 def evaluate_payoff_matrix(network, def_strategies, att_strategies, n_rollouts, steps_per_episode=100, seed=0,
-                           device="cuda:0", rank=0, world=1, xcap=16, group=None, reduce=True):
-    """Returns a float64 tensor [n_def, n_att, 10] (averages) on `device`."""
+                           device="cuda:0", rank=0, world=1, xcap=16, group=None, reduce=True, train_detectors=False):
+    """Returns a float64 tensor [n_def, n_att, 10] (averages) on `device`.
+
+    train_detectors=True: every env keeps a hop-log ring of DETECTOR_LOG_CAP records (8 KB per env) and, where the
+    defender strategy can train (Strategy.can_train), a detector slot (24.6 KB per env); after every defender turn the
+    pending envs are fitted on the device with detector_fit_seeds(seed, env ids, turn), and the call raises RuntimeError
+    when an env ends with a sticky CYG_FL_ERR_* bit.  Without it, a strategy that trains gets the stub scan and a sticky
+    CYG_FL_ERR_DETECTOR bit, and the result does not say so."""
     import torch
     from .vector_env import ActionBatch, VectorCyberDefenseEnv
     lo, hi = shard_range(n_rollouts, rank, world)
     nloc = hi - lo
     nd, na = len(def_strategies), len(att_strategies)
     sums = torch.zeros(nd, na, len(COLUMNS), dtype=torch.float64, device=device)
+    flags = []
     if nloc > 0:
         M = network.M
         for i, ds in enumerate(def_strategies):
+            fits = train_detectors and ds.can_train()
             for j, as_ in enumerate(att_strategies):
                 # env ids are unique per (pair, rollout) so that every rollout has its own draw stream
-                env = VectorCyberDefenseEnv(network, nloc, device=device, seed=seed,
-                                            env_id0=(i * na + j) * n_rollouts + lo, xcap=xcap)
+                id0 = (i * na + j) * n_rollouts + lo
+                env = VectorCyberDefenseEnv(network, nloc, device=device, seed=seed, env_id0=id0, xcap=xcap,
+                                            log_cap=DETECTOR_LOG_CAP if train_detectors else 0, detector_slots=nloc if fits else 0)
+                g = id0 + torch.arange(nloc, device=env.device) if fits else None
                 env.randomize_compromise_and_ownership()
                 for slot in _ROLLOUT_RESET:
                     env.scalars[:, slot] = 0
@@ -99,10 +163,16 @@ def evaluate_payoff_matrix(network, def_strategies, att_strategies, n_rollouts, 
                     raw, _, _ = env.step(ab)
                     if mode == 0:
                         def_r += raw.double()
+                        if fits and t < steps_per_episode - 1:
+                            env.fit_detectors(detector_fit_seeds(seed, g, t))
                     else:
                         att_r += raw.double()
                 sums[i, j] = torch.stack([c.sum() for c in _columns(def_r, att_r, env.info())])
+                if train_detectors:
+                    flags.append(env.scalars[:, K.S_FLAGS].clone())
                 env.close()
+    if train_detectors:
+        _check_error_bits(flags)
     if not reduce:
         return sums
     return reduce_payoff(sums, n_rollouts, steps_per_episode, group=group)
@@ -160,20 +230,23 @@ def _strategy_rows(def_strategies, att_strategies, T, M):
 _ENV_CACHE = {}
 
 
-def _cached_env(network, nloc, lo, device, seed, xcap):
+def _cached_env(network, nloc, lo, device, seed, xcap, log_cap=0, detector_slots=0):
     """The evaluation's env batch, kept between calls (a Double-Oracle run evaluates the same network again and again:
     build_payoff_matrices, do_agent.py:1666-1870): re-creating 1 M envs costs ~15 ms of allocation and table upload per
-    call, a reset() of the kept ones ~2 ms."""
+    call, a reset() of the kept ones ~2 ms.  The hop-log ring and the detector slots are part of the key (a kept handle
+    without a ring never serves an evaluation that trains); a kept handle's envs give their slots back."""
     from .vector_env import VectorCyberDefenseEnv
-    key = (id(network), int(nloc), int(lo), str(device), int(seed), int(xcap))
+    key = (id(network), int(nloc), int(lo), str(device), int(seed), int(xcap), int(log_cap), int(detector_slots))
     env = _ENV_CACHE.get(key)
     if env is None:
         for k in list(_ENV_CACHE):
             _ENV_CACHE.pop(k).close()
-        env = _ENV_CACHE[key] = VectorCyberDefenseEnv(network, nloc, device=device, seed=seed, env_id0=lo, xcap=xcap)
+        env = _ENV_CACHE[key] = VectorCyberDefenseEnv(network, nloc, device=device, seed=seed, env_id0=lo, xcap=xcap,
+                                                      log_cap=log_cap, detector_slots=detector_slots)
     else:
         env.reset()
         env.set_base_line_per_env(None)
+        env.release_detectors()
     return env
 
 
@@ -216,7 +289,8 @@ def _block_order(env, sides, i_of_pair, j_of_pair, pair_of_env, T):
 
 
 def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_rollouts, steps_per_episode=100, seed=0,
-                                   device="cuda:0", rank=0, world=1, xcap=16, group=None, reduce=True, steps_per_launch=None):
+                                   device="cuda:0", rank=0, world=1, xcap=16, group=None, reduce=True, steps_per_launch=None,
+                                   train_detectors=False):
     """Same result as evaluate_payoff_matrix(), with ALL (pair, rollout) combinations in one batch: the flattened
     index g = pair * n_rollouts + rollout is split over the ranks (env id == g, so the draw streams do not depend on the
     number of ranks): every rank takes the same slice of rollouts of every pair when n_rollouts divides evenly (balanced
@@ -230,7 +304,18 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
     With a parametric strategy (Strategy(actor=...): the DDPG best responses) on either side the rollout is closed
     loop: per turn one observation launch, one batched actor forward per parametric strategy on the rows of its envs,
     decode_actions() on the device, one step launch.  Strategies with unsorted / repeated device lists are not handled
-    here (use the per-pair evaluator)."""
+    here (use the per-pair evaluator).
+
+    train_detectors=True serves defender strategies that train the detector (action 10; Strategy.can_train): the envs
+    keep a hop-log ring of DETECTOR_LOG_CAP records, and this rank's envs whose defender can train get a detector slot
+    each.  Memory at C5 shape (2^20 envs on one GPU): the ring is handle-wide, 2000 x 4 B x 2^20 = 8.4 GB; a slot is
+    24.6 KB per env that can train.  A detector cannot be fitted inside a launch, so the table-driven path also ends a
+    launch after every turn t < T - 1 at which some pair's defender row executes type 10 (its base_line is Nash), and
+    fits every pending env on the device (fit_detectors, seeds detector_fit_seeds(seed, g, t)) before the next launch;
+    the closed-loop path fits after every defender turn.  The result equals the same rollouts with those host fits, for
+    any steps_per_launch and sharding.  After the last turn the call raises RuntimeError when an env carries a sticky
+    CYG_FL_ERR_* bit.  Without the flag, a strategy that trains gets the stub scan and a sticky CYG_FL_ERR_DETECTOR bit,
+    and the result does not say so."""
     import torch
     from .vector_env import ActionBatch, VectorCyberDefenseEnv
     nd, na = len(def_strategies), len(att_strategies)
@@ -249,11 +334,19 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
         nloc = hi - lo
     sums = torch.zeros(P, len(COLUMNS), dtype=torch.float64, device=device)
     if nloc > 0:
-        env = _cached_env(network, nloc, lo, device, seed, xcap)
-        env.set_env_id_stride(run if strided else 0, n_rollouts)
-        pair_of_env = (lo + env.env_index_of_slot()) // n_rollouts
         i_of_pair = np.arange(P) // na
         j_of_pair = np.arange(P) % na
+        n_slots = 0
+        if train_detectors:  # this rank's envs whose defender strategy can train
+            trains = np.array([st.can_train() for st in def_strategies], bool)[i_of_pair]
+            if strided:
+                n_slots = run * int(trains.sum())
+            else:
+                n_slots = int(np.bincount(np.arange(lo, lo + nloc) // n_rollouts, minlength=P)[trains].sum())
+        env = _cached_env(network, nloc, lo, device, seed, xcap, DETECTOR_LOG_CAP if train_detectors else 0, n_slots)
+        env.set_env_id_stride(run if strided else 0, n_rollouts)
+        g_of_env = lo + env.env_index_of_slot()
+        pair_of_env = g_of_env // n_rollouts
         env.randomize_compromise_and_ownership()
         for slot in _ROLLOUT_RESET:
             env.scalars[:, slot] = 0
@@ -286,9 +379,18 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
         if not any_nn and W <= 4:
             spl = T if not steps_per_launch else max(1, int(steps_per_launch))
             order = _block_order(env, sides, i_of_pair, j_of_pair, pair_of_env, T)
-            for t0 in range(0, T, spl):
-                t1 = min(T, t0 + spl)
+            cuts = set(range(spl, T, spl))
+            fit_after = set()
+            if n_slots:  # the turns after which a fit must run: some pair's defender row executes type 10 (one read of [T, P])
+                h0 = hdr_d[:, :, 0]
+                trains_t = (((h0 & 0xFF) == 10) & (((h0 >> 8) & 1) == K.MODE_DEFENDER) & (bl_d == K.BASE_LINES["Nash"])).any(1)
+                fit_after = {int(t) for t in torch.nonzero(trains_t).flatten().tolist() if t < T - 1}
+                cuts |= {t + 1 for t in fit_after}
+            bounds = [0] + sorted(cuts) + [T]
+            for t0, t1 in zip(bounds[:-1], bounds[1:]):
                 env.rollout(hdr_d[t0:t1], mask_d[t0:t1], bl_d[t0:t1], n_rollouts, lo, returns=ret, block_order=order)  # the mode of a turn is in its headers
+                if t1 - 1 in fit_after:
+                    env.fit_detectors(detector_fit_seeds(seed, g_of_env, t1 - 1))
         else:
             X, n_app = network.X, int(network.cfg.get("n_app_ids", 0))
             side_of_env = [torch.from_numpy(i_of_pair).to(device)[pair_of_env], torch.from_numpy(j_of_pair).to(device)[pair_of_env]]
@@ -312,7 +414,11 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
                 env.set_base_line_per_env(bl_d[t][pair_of_env])
                 raw, _, _ = env.step(ActionBatch(hdr_e, mask_e))
                 ret[mode] += raw.double()
+                if n_slots and mode == 0 and t < T - 1:
+                    env.fit_detectors(detector_fit_seeds(seed, g_of_env, t))
         sums.index_add_(0, pair_of_env, torch.stack(_columns(ret[0], ret[1], env.info()), dim=1))
+        if train_detectors:
+            _check_error_bits([env.scalars[:, K.S_FLAGS]])
     sums = sums.view(nd, na, len(COLUMNS))
     if not reduce:
         return sums

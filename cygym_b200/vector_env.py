@@ -570,6 +570,13 @@ class VectorCyberDefenseEnv:
         self._hold_seeds = s
         K.check(self.L.cyg_fit_detectors(self.h, _ptr(s), _ptr(self._next_slot), self._s()))
 
+    def release_detectors(self):
+        """Every env gives its detector slot back (the next fits take slots from 0 again); a no-op without detector
+        slots.  For a batch that is reset() and reused."""
+        if self._det_slots is not None:
+            self._det_of_env.fill_(-1)
+            self._next_slot.zero_()
+
     def rebuild_graph_cache(self, env_mask=None):
         """_rebuild_graph_cache() from outside a step (volt_typhoon_env.py:456-483): every blocked edge is forgotten (:476)."""
         if env_mask is not None:

@@ -270,7 +270,12 @@ int cyg_step_multi(cyg_handle h, const cyg_actions* actions, int32_t n_steps, ui
  * the per-pair tables are uploaded once per evaluation and gathered inside the kernel.  base_line (optional) has the
  * same row layout: what the two players' baselines set env.base_line to on their turns (do_agent.py:716-719).
  * returns[2][B] (float64) receives += the raw reward of every step, row 0 on defender turns, row 1 on attacker turns
- * (def_r / att_r of do_agent.py:2060-2062); the counters of the info dict are read from the scalars afterwards. */
+ * (def_r / att_r of do_agent.py:2060-2062); the counters of the info dict are read from the scalars afterwards.
+ * A handle with a hop-log ring (log_cap > 0) and detector slots keeps its rings and consults its detectors here as in
+ * cyg_step.  No detector is fitted inside a launch: an env whose defender trains (action 10) stays CYG_FL_DET_PENDING
+ * until cyg_fit_detectors runs, and a trained scan (action 5) of that env later in the SAME launch sets
+ * CYG_FL_ERR_DETECTOR, exactly as in cyg_step_multi.  A caller whose strategies may train ends the launch after every
+ * turn that may train and calls cyg_fit_detectors before the next one (cygym_b200/payoff.py, train_detectors=True). */
 typedef struct cyg_rollout_args {
   const uint32_t* hdr;      /* [n_steps][n_rows][4] */
   const uint32_t* mask;     /* [n_steps][n_rows][W] */
@@ -346,8 +351,9 @@ int cyg_set_detectors(cyg_handle h, const uint32_t* slots, int32_t n_slots, cons
  * An env without a slot (det_of_env[b] < 0) takes slot *next_slot, in env order, and *next_slot advances: next_slot is a
  * device int32 owned by the caller and shared with whatever assigns slots on the host.  A fitted env keeps
  * CYG_FL_DET_TRAINED and loses CYG_FL_DET_PENDING.  An env that cannot be fitted -- no slot left, or
- * min(CYG_S_LOGS, CYG_DET_WINDOW) > log_cap -- stays pending and gets CYG_FL_ERR_DETECTOR.  Two launches on `stream` (slot
- * assignment, then the fits), no host synchronisation.  CYG_E_INVAL when the handle has no detector slots. */
+ * min(CYG_S_LOGS, CYG_DET_WINDOW) > log_cap -- stays pending and gets CYG_FL_ERR_DETECTOR.  Three launches on `stream`
+ * (slot assignment in two passes over the whole batch, then the fits), no host synchronisation.  CYG_E_INVAL when the
+ * handle has no detector slots. */
 int cyg_fit_detectors(cyg_handle h, const uint32_t* seeds, int32_t* next_slot, void* stream);
 
 /* Replaces sample_action() (CyberDefenseEnv.py:555-578) for every env; writes hdr[B][4], mask[B][W]. */

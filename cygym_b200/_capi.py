@@ -23,6 +23,7 @@ PLANE_WIDTHS = (1, 2, 3, 4, 64)  # one translation unit of cyg_kernels.cu per pl
 ABI_VERSION = 3
 NSCAL = 16
 ATYPE_NONE = 0x80
+ORDER_NONE = 0xFFFF  # first entry of a set-form row of a cyg_rollout_ordered order table
 MODE_DEFENDER, MODE_ATTACKER = 0, 1
 STEP_GROUPED, STEP_SKIP_WORK = 1, 2
 BL_NASH, BL_NO_DEFENSE, BL_PRESET, BL_NO_ATTACK, BL_OTHER = range(5)
@@ -128,7 +129,7 @@ class CygRolloutArgs(C.Structure):
 
 
 EXPORTS = ["cyg_version", "cyg_last_error", "cyg_create", "cyg_destroy", "cyg_set_base_line", "cyg_set_base_line_per_env", "cyg_set_base_line_per_env_steps", "cyg_internal_words",
-           "cyg_bind", "cyg_set_detectors", "cyg_fit_detectors", "cyg_import_state", "cyg_export_state", "cyg_step", "cyg_step_multi", "cyg_rollout", "cyg_unpack_actions", "cyg_pack_done", "cyg_block_envs", "cyg_set_env_id_stride", "cyg_randomize", "cyg_rebuild_graph_cache", "cyg_sample_actions", "cyg_sample_actions_ordered",
+           "cyg_bind", "cyg_set_detectors", "cyg_fit_detectors", "cyg_import_state", "cyg_export_state", "cyg_step", "cyg_step_multi", "cyg_rollout", "cyg_rollout_ordered", "cyg_unpack_actions", "cyg_pack_done", "cyg_block_envs", "cyg_set_env_id_stride", "cyg_randomize", "cyg_rebuild_graph_cache", "cyg_sample_actions", "cyg_sample_actions_ordered",
            "cyg_observe", "cyg_group_actions", "cyg_launch_count"]
 
 
@@ -142,7 +143,7 @@ SPILL_LIMIT = 256   # bytes of spill stores tolerated in the config-C3 step kern
 THREAD_CAPS = (640, 512)  # threads per CTA -> 93 / 127 registers per thread at one CTA per SM (640 measured fastest)
 
 
-STEP_KERNEL = "_Z15cyg_step_kernelILi4ELb0ELb0EEv10StepParams"  # cyg_step_kernel<4, false, false>: plain steps, no ROLL, no LOG
+STEP_KERNEL = "_Z15cyg_step_kernelILi4ELb0ELb0ELb0EEv10StepParams"  # cyg_step_kernel<4, false, false, false>: plain steps, no ROLL, no LOG, no ORD
 
 
 def _step_kernel_spill(ptxas_log, mangled=STEP_KERNEL):
@@ -236,6 +237,7 @@ def lib():
         L.cyg_step.argtypes = [C.c_void_p, C.POINTER(CygActions), C.c_uint32, C.POINTER(CygStepOut), C.c_void_p]
         L.cyg_step_multi.argtypes = [C.c_void_p, C.POINTER(CygActions), C.c_int32, C.c_uint32, C.POINTER(CygStepOut), C.c_void_p]
         L.cyg_rollout.argtypes = [C.c_void_p, C.POINTER(CygRolloutArgs), C.c_uint32, C.c_void_p]
+        L.cyg_rollout_ordered.argtypes = [C.c_void_p, C.POINTER(CygRolloutArgs), C.c_void_p, C.c_int32, C.c_uint32, C.c_void_p]
         L.cyg_set_env_id_stride.argtypes = [C.c_void_p, C.c_int32, C.c_int32]
         L.cyg_block_envs.argtypes = [C.c_void_p, C.POINTER(C.c_int32)]
         L.cyg_unpack_actions.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]

@@ -10,6 +10,8 @@
  * cyg_step_kernel<W, ROLL, LOG>: plain steps (one set-form action per env), T fused per launch: phase A thread per
  *   env, phase B warp per env for the draw-heavy actions, phase C thread per env; each warp sends its finished records
  *   home by warp-wide copies.
+ * cyg_step_kernel<W, true, LOG, true>: rollouts with an order table (cyg_rollout_ordered): an ordered row's env runs
+ *   its action thread per env in phase A with the sequential forms, set-form rows as above.
  * cyg_step_seq_kernel<W>: grouped steps and explicit order lists, one thread-per-env pass, one bulk store of the block.
  * cyg_step_generic_kernel<W>: networks beyond 128 device slots (tables too large for shared memory).
  * cyg_fit_count_kernel + cyg_fit_assign_kernel + cyg_fit_kernel: the detector fit of defender action 10
@@ -224,10 +226,13 @@ __device__ __forceinline__ void load_block_finish(bool bulk_ok, uint32_t* s_rec,
  *    copies): a warp then runs ONE branch of the 14 defender / 3+X attacker actions.  s_perm[pos] = the env (0..nb-1)
  *    thread pos steps; s_cnt[k + 1] ends as the end of key k's run.  keyed == false: every env has key 0 (grouped steps).
  *    FLIP_KEYS: block / unblock envs go to keys 32..47 by listed-device count, longest first (phase B of the plain kernel
- *    runs them in that order).  row_of(env) = the env's row of hdr_t / bl_t.  s_cnt[0..CYG_NKEYS] must be zero. */
-template <int W, bool FLIP_KEYS, class RowOf>
+ *    runs them in that order).  row_of(env) = the env's row of hdr_t / bl_t.  s_cnt[0..CYG_NKEYS] must be zero.
+ *    ORD_KEYS: rows whose order entry ord_t[row * ord_stride] is not CYG_ORDER_NONE keep their type key (6 / 9 stay out
+ *    of the block / unblock buckets: their own thread walks the list in pass 0, so they need no phase-B task). */
+template <int W, bool FLIP_KEYS, class RowOf, bool ORD_KEYS = false>
 __device__ __forceinline__ void sort_block(const Net& net, const uint32_t* hdr_t, const uint8_t* bl_t, bool keyed, RowOf row_of,
-                                           int env0, int nb, uint32_t* s_cnt, uint16_t* s_perm, int tid) {
+                                           int env0, int nb, uint32_t* s_cnt, uint16_t* s_perm, int tid,
+                                           const uint16_t* ord_t = nullptr, int ord_stride = 0) {
   int key = 0;
   if (tid < nb) {
     if (keyed) {
@@ -237,7 +242,9 @@ __device__ __forceinline__ void sort_block(const Net& net, const uint32_t* hdr_t
       const int blk = bl_t ? (int)bl_t[r0] : net.cfg.base_line;
       const int xt = Env<W, 1>::exec_type(net.cfg, h0, blk) & 15;
       key = (int)(((h0 >> 8) & 1u) << 4) | xt;
-      if (FLIP_KEYS && (key == 6 || key == 9)) { /* longest-processing-time first: 8 buckets of 16 listed devices */
+      bool flip_key = FLIP_KEYS && (key == 6 || key == 9);
+      if constexpr (ORD_KEYS) flip_key = flip_key && ord_t[r0 * (size_t)ord_stride] == CYG_ORDER_NONE;
+      if (flip_key) { /* longest-processing-time first: 8 buckets of 16 listed devices */
         int nd = (int)(hv.z & 0xFFFFu);
         nd = nd < 0 ? 0 : (nd > 127 ? 127 : nd);
         key = CYG_KEY_FLIP0 + 2 * (7 - (nd >> 4)) + (key == 9 ? 1 : 0);
@@ -296,8 +303,14 @@ __host__ __device__ inline SmemPlan smem_plan(uint32_t hot_words, int S, int NB)
  * its hops, scans consult the detector.  Also its own instantiation (the handles that keep only the log's length --
  * every throughput run -- take the kernel without that code: ~1 us per step).  ROLL and LOG together: cyg_rollout on a
  * handle with a ring.  The ring and det_of_env are indexed by slot, the draw streams and action rows by env id. */
-template <int W, bool ROLL, bool LOG>
+/* ORD (with ROLL only: cyg_rollout_ordered): the rollout carries an order table p.order [T][n_rows][order_stride].  A row
+ * whose first entry is CYG_ORDER_NONE is a set-form row and runs as without ORD; any other row lists device_indices in
+ * order, and its env's own thread runs the whole action in pass 0 with the sequential forms cyg_step_seq_kernel runs for
+ * order arrays (never deferred to phase B).  Its own instantiation: the sequential forms are code the other forms never
+ * run. */
+template <int W, bool ROLL, bool LOG, bool ORD = false>
 __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(const __grid_constant__ StepParams p) {
+  static_assert(ROLL || !ORD, "order tables are a rollout form");
   unsigned char* smem = reinterpret_cast<unsigned char*>(cyg_smem);
   const int NB = p.block_envs, NT = blockDim.x, tid = threadIdx.x; /* NB envs, NT >= NB threads */
   const int S = p.net.S, M = p.net.M;
@@ -342,9 +355,10 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
     asm volatile("prefetch.global.L2 [%0];" ::"l"(hdr_t + ((size_t)p.B + env0 + tid) * 4));
     asm volatile("prefetch.global.L2 [%0];" ::"l"(mask_t + ((size_t)p.B + env0 + tid) * W));
   }
+  const uint16_t* ord_t = ORD ? p.order + (size_t)t * p.n_rows * p.order_stride : nullptr; /* this step's order rows */
   for (int i = tid; i < CYG_NKEYS + 7; i += NT) s_cnt[i] = 0; /* ... + one "past pass 0" flag per owning warp */
   __syncthreads(); /* mbarrier initialised, counters zeroed (t > 0: the previous step is complete) */
-  sort_block<W, true>(p.net, hdr_t, bl_t, true, arow, env0, nb, s_cnt, s_perm, tid);
+  sort_block<W, true, decltype(arow), ORD>(p.net, hdr_t, bl_t, true, arow, env0, nb, s_cnt, s_perm, tid, ord_t, p.order_stride);
   if (t == 0) load_block_finish(bulk_ok, s_rec, g_rec, nb * S, bar, tid, NT);
   __syncthreads();
 
@@ -386,15 +400,24 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
     if (pass == 0) {
       uint32_t act[4 + W]; /* this env's action (group 0), in registers */
       int atype = 0;
+      const uint16_t* my_ord = nullptr; /* ORD: this env's order row when it is ordered */
       if (tid < nb) {
         uint4 hv = *reinterpret_cast<const uint4*>(hdr_t + my_row * 4);
         act[0] = hv.x; act[1] = hv.y; act[2] = hv.z; act[3] = hv.w;
 #pragma unroll
         for (int w = 0; w < W; w++) act[4 + w] = mask_t[my_row * W + w];
+        if constexpr (ORD) {
+          const uint16_t* o = ord_t + my_row * p.order_stride;
+          if (o[0] != CYG_ORDER_NONE) {
+            my_ord = o;
+            if ((act[2] & 0xFFFFu) > (uint32_t)p.order_stride) act[2] = (act[2] & 0xFFFF0000u) | (uint32_t)p.order_stride; /* the row holds no more */
+          }
+        }
         mode = (int)((act[0] >> 8) & 1u);
         if (bl_t) e.bl = (int)bl_t[my_row];
         atype = e.step_pre(act, p.flags);
         deferred = Coop<W>::is_heavy(e, mode, atype) && !(mode == CYG_MODE_ATTACKER && e.bl == CYG_BL_NO_ATTACK);
+        if constexpr (ORD) deferred = deferred && !my_ord;
       }
       /* once every env has its epoch open and its busy tick done (s_cnt[CYG_NKEYS + 6] counts the owning warps that
        * got there) phase B may touch any deferred env: the warps that own no env start it right away, the owning
@@ -406,7 +429,8 @@ __global__ void __launch_bounds__(CYG_MAX_BLOCK_THREADS, 1) cyg_step_kernel(cons
         if (lane == 0) { s_def[tid >> 5] = dmask; __threadfence_block(); atomicAdd(&s_cnt[CYG_NKEYS + 6], 1u); }
       }
       if (tid < nb && !deferred) {
-        e.template step_act<true>(act, act + 4, nullptr, 0, 0, 0, 1, p.flags, atype, cost, dirty);
+        if (ORD && my_ord) e.step_act(act, act + 4, my_ord, 0, 0, 0, 1, p.flags, atype, cost, dirty); /* as cyg_step_seq_kernel */
+        else e.template step_act<true>(act, act + 4, nullptr, 0, 0, 0, 1, p.flags, atype, cost, dirty);
         do_post = true;
       }
     } else {
@@ -1115,6 +1139,7 @@ __global__ void cyg_observe_kernel(const __grid_constant__ ObsParams p) {
  * ======================================================================== */
 struct Kernels {
   const void *step, *step_log, *step_seq, *rollout, *rollout_log; /* W = 64: cyg_step_generic_kernel in `step`, the other forms null */
+  const void *rollout_ord, *rollout_ord_log; /* cyg_rollout_ordered */
   const void *import_state, *export_state, *randomize, *rebuild, *sample, *observe;
 };
 #define CYG_KERNELS_NAME2(w) cyg_kernels_w##w
@@ -1126,8 +1151,9 @@ extern "C" const Kernels CYG_KERNELS_NAME(CYG_TU_W) = {
     (const void*)cyg_step_kernel<CYG_TU_W, false, false>, (const void*)cyg_step_kernel<CYG_TU_W, false, true>,
     (const void*)cyg_step_seq_kernel<CYG_TU_W>, (const void*)cyg_step_kernel<CYG_TU_W, true, false>,
     (const void*)cyg_step_kernel<CYG_TU_W, true, true>,
+    (const void*)cyg_step_kernel<CYG_TU_W, true, false, true>, (const void*)cyg_step_kernel<CYG_TU_W, true, true, true>,
 #else
-    (const void*)cyg_step_generic_kernel<CYG_TU_W>, nullptr, nullptr, nullptr, nullptr,
+    (const void*)cyg_step_generic_kernel<CYG_TU_W>, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
 #endif
     (const void*)cyg_import_kernel<CYG_TU_W>, (const void*)cyg_export_kernel<CYG_TU_W>, (const void*)cyg_randomize_kernel<CYG_TU_W>,
     (const void*)cyg_rebuild_kernel<CYG_TU_W>, (const void*)cyg_sample_kernel<CYG_TU_W>, (const void*)cyg_observe_kernel<CYG_TU_W>};
@@ -1227,7 +1253,7 @@ static int configure_step(cyg_env_s* h) {
   }
   /* opt in to the device maximum once (handles with different block sizes share the kernel) */
   const Kernels& k = kernels(h->W);
-  for (const void* f : {k.step, k.step_log, k.step_seq, k.rollout, k.rollout_log})
+  for (const void* f : {k.step, k.step_log, k.step_seq, k.rollout, k.rollout_log, k.rollout_ord, k.rollout_ord_log})
     if (f) CU(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin));
   return CYG_OK;
 }
@@ -1465,7 +1491,9 @@ int cyg_step_multi(cyg_handle h, const cyg_actions* a, int32_t n_steps, uint32_t
   return step_impl(h, a, n_steps, step_flags, out, stream);
 }
 
-int cyg_rollout(cyg_handle h, const cyg_rollout_args* a, uint32_t step_flags, void* stream) {
+/* cyg_rollout and cyg_rollout_ordered: the argument checks they share, then the launch (order NULL: the set-form kernel) */
+static int rollout_impl(cyg_handle h, const cyg_rollout_args* a, const uint16_t* order, int32_t order_stride, uint32_t step_flags,
+                        void* stream) {
   if (!h || !a || !a->hdr || !a->mask || !a->returns) return fail(CYG_E_INVAL, "null argument");
   if (!h->state) return fail(CYG_E_INVAL, "cyg_bind() first");
   if (h->W > CYG_MAX_W) return fail(CYG_E_INVAL, "cyg_rollout: networks of at most 128 device slots");
@@ -1476,7 +1504,7 @@ int cyg_rollout(cyg_handle h, const cyg_rollout_args* a, uint32_t step_flags, vo
   if (((uintptr_t)a->hdr) & 15) return fail(CYG_E_INVAL, "hdr must be 16-byte aligned");
   DeviceGuard g(h->device);
   StepParams p = step_params(h);
-  p.hdr = a->hdr; p.mask = a->mask;
+  p.hdr = a->hdr; p.mask = a->mask; p.order = order; p.order_stride = order ? order_stride : 0;
   p.bl_env = a->base_line; p.bl_stride = a->base_line ? a->n_rows : 0;
   p.G = 1; p.flags = step_flags; p.T = a->n_steps;
   p.row_base = a->row_base; p.envs_per_row = a->envs_per_row; p.n_rows = a->n_rows; p.ret_acc = a->returns;
@@ -1484,7 +1512,19 @@ int cyg_rollout(cyg_handle h, const cyg_rollout_args* a, uint32_t step_flags, vo
   void* args[] = {&p};
   const StepGrid grid = step_grid(h);
   const Kernels& k = kernels(h->W);
-  return launch(h, p.logs ? k.rollout_log : k.rollout, grid.blocks, grid.threads, h->smem_bytes, stream, args);
+  const void* kernel = order ? (p.logs ? k.rollout_ord_log : k.rollout_ord) : (p.logs ? k.rollout_log : k.rollout);
+  return launch(h, kernel, grid.blocks, grid.threads, h->smem_bytes, stream, args);
+}
+
+int cyg_rollout(cyg_handle h, const cyg_rollout_args* a, uint32_t step_flags, void* stream) {
+  return rollout_impl(h, a, nullptr, 0, step_flags, stream);
+}
+
+int cyg_rollout_ordered(cyg_handle h, const cyg_rollout_args* a, const uint16_t* order, int32_t order_stride, uint32_t step_flags,
+                        void* stream) {
+  if (!order) return fail(CYG_E_INVAL, "cyg_rollout_ordered: null order table");
+  if (h && order_stride < h->net.M) return fail(CYG_E_INVAL, "cyg_rollout_ordered: order_stride must hold M entries");
+  return rollout_impl(h, a, order, order_stride, step_flags, stream);
 }
 
 /* the fields of a randomize / rebuild / sample launch that come from the handle alone; every other field is zero */

@@ -192,14 +192,24 @@ def decode_actions(raw, mode, n_types, M, X, n_app, W):
     return header_rows(at, m, ex, dev.sum(1), app), pack_device_mask(dev, W).contiguous()
 
 
+def _is_set_form(action):
+    """Whether an action's device_indices can travel as a set: None, or an ascending duplicate-free list."""
+    return action is None or [int(d) for d in action[2]] == sorted(set(int(d) for d in action[2]))
+
+
 def _strategy_rows(def_strategies, att_strategies, T, M):
     """The distinct action rows of every strategy, packed once on the host, and which row each strategy plays on each
     turn: per side (hdr rows [R, 4], mask rows [R, W], row index [T, S], base_line code [S] (255 = the strategy does not
-    touch env.base_line)).  A fixed sequence of L actions is L rows indexed by t % L."""
+    touch env.base_line), order rows [R, M] uint16).  A fixed sequence of L actions is L rows indexed by t % L.
+
+    A defender row whose list is not ascending and duplicate-free (the draw order of the sequences DoubleOracle samples,
+    do_agent.py:1001-1013) is ORDERED: its order row holds the list, and the kernel visits the devices in that order.
+    Every other row is a set: its order row starts with ORDER_NONE.  Attacker rows are sets whatever their list
+    (attacker_act reads the exploits and the sources, never device_indices)."""
     from .vector_env import ActionBatch
     out = []
     for mode, sts in ((0, def_strategies), (1, att_strategies)):
-        hs, ms, first, length, bls, n_rows = [], [], [], [], [], 0
+        hs, ms, os_, first, length, bls, n_rows = [], [], [], [], [], [], 0
         for st in sts:
             key = (mode, M)
             cached = st.__dict__.setdefault("_packed_rows", {}).get(key)  # a strategy is evaluated again and again as the matrices grow
@@ -212,19 +222,36 @@ def _strategy_rows(def_strategies, att_strategies, T, M):
                     acts, bl = list(st.actions), 255
                 else:
                     acts, bl = [None], K.BASE_LINES["Nash"]
-                for a in acts:
-                    if a is not None and list(a[2]) != sorted(set(int(d) for d in a[2])):
-                        raise NotImplementedError("unsorted device_indices: use evaluate_payoff_matrix()")
-                h, m, _ = ActionBatch.pack(acts, mode, M)
-                cached = st._packed_rows[key] = (h.view(np.int32), m.view(np.int32), bl)
-            h, m, bl = cached
+                h, m, o = ActionBatch.pack(acts, mode, M, order_form=True)  # the mask holds the set of any list
+                ordered = np.array([mode == K.MODE_DEFENDER and not _is_set_form(a) for a in acts], bool)
+                o[~ordered] = K.ORDER_NONE
+                cached = st._packed_rows[key] = (h.view(np.int32), m.view(np.int32), bl, o)
+            h, m, bl, o = cached
             first.append(n_rows); length.append(len(h)); bls.append(bl)
             n_rows += len(h)
-            hs.append(h); ms.append(m)
+            hs.append(h); ms.append(m); os_.append(o)
         t = np.arange(T)[:, None]
         ridx = np.asarray(first)[None, :] + t % np.asarray(length)[None, :]
-        out.append((np.concatenate(hs), np.concatenate(ms), ridx.astype(np.int64), np.asarray(bls, np.uint8)))
+        out.append((np.concatenate(hs), np.concatenate(ms), ridx.astype(np.int64), np.asarray(bls, np.uint8), np.concatenate(os_)))
     return out
+
+
+_ORDER_NONE_I16 = K.ORDER_NONE - 0x10000  # ORDER_NONE as the int16 the device tables hold
+
+
+def _order_arrays(hdr, mask, ord_rows):
+    """The order array of a closed-loop step whose batch has ordered rows (cyg_step applies an order array to every env):
+    ord_rows [N, M] int16 where the env's row is ordered, the ascending list of its mask where the row is a set (the
+    set read in order).  Width = the longest list of the batch.  int16 [N, width] on the device."""
+    import torch
+    N, M = ord_rows.shape
+    width = max(1, int((hdr[:, 2] & 0xFFFF).max()))
+    bits = (mask.to(torch.int32)[:, :, None] >> torch.arange(32, device=mask.device, dtype=torch.int32)) & 1  # [N, W, 32]
+    ids = torch.arange(bits.shape[1] * 32, device=mask.device, dtype=torch.int32)
+    asc = torch.where(bits.view(N, -1).bool(), ids, 0x7FFF).sort(dim=1).values[:, :M]  # set devices first, ascending
+    out = torch.where((ord_rows[:, :1] != _ORDER_NONE_I16), ord_rows.to(torch.int32), asc)
+    pad = max(0, width - M)
+    return torch.nn.functional.pad(out, (0, pad))[:, :width].to(torch.int16).contiguous()
 
 
 _ENV_CACHE = {}
@@ -265,7 +292,7 @@ def _block_order(env, sides, i_of_pair, j_of_pair, pair_of_env, T):
     import torch
     from .vector_env import decode_header
     cost_side = []
-    for mode, (h, _, ridx, bls) in enumerate(sides):
+    for mode, (h, _, ridx, bls, _) in enumerate(sides):
         f = decode_header(h)
         t = (f.atype & 0xFF).astype(np.int64)
         n = f.n_dev.astype(np.float64)
@@ -303,8 +330,13 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
 
     With a parametric strategy (Strategy(actor=...): the DDPG best responses) on either side the rollout is closed
     loop: per turn one observation launch, one batched actor forward per parametric strategy on the rows of its envs,
-    decode_actions() on the device, one step launch.  Strategies with unsorted / repeated device lists are not handled
-    here (use the per-pair evaluator).
+    decode_actions() on the device, one step launch.
+
+    Fixed sequences whose defender actions list their devices in draw order (DoubleOracle's sampled strategies,
+    do_agent.py:1001-1013) are evaluated as they are: those rows carry their list in an order table (_strategy_rows),
+    the table-driven path launches cyg_rollout_ordered (an ordered row's env runs its action with one thread, in list
+    order), and the closed-loop path passes an order array to the defender turns that have ordered rows.  An evaluation
+    without such a row takes exactly the launches it took before.
 
     train_detectors=True serves defender strategies that train the detector (action 10; Strategy.can_train): the envs
     keep a hop-log ring of DETECTOR_LOG_CAP records, and this rank's envs whose defender can train get a detector slot
@@ -356,11 +388,15 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
         sides = _strategy_rows(def_strategies, att_strategies, T, M)
         tt = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(device)
         of_pair = (tt(i_of_pair), tt(j_of_pair))
-        hdr_side = [tt(h)[tt(r)][:, of_pair[m_]] for m_, (h, _, r, _) in enumerate(sides)]    # [T, P, 4] per side
-        mask_side = [tt(m)[tt(r)][:, of_pair[m_]] for m_, (_, m, r, _) in enumerate(sides)]  # [T, P, W]
+        hdr_side = [tt(h)[tt(r)][:, of_pair[m_]] for m_, (h, _, r, _, _) in enumerate(sides)]    # [T, P, 4] per side
+        mask_side = [tt(m)[tt(r)][:, of_pair[m_]] for m_, (_, m, r, _, _) in enumerate(sides)]  # [T, P, W]
         even = (torch.arange(T, device=device) % 2 == 0)[:, None, None]
         hdr_d = torch.where(even, hdr_side[0], hdr_side[1]).contiguous()
         mask_d = torch.where(even, mask_side[0], mask_side[1]).contiguous()
+        ord_d = None  # [T, P, M] int16 order rows, only when some defender row is ordered (attacker rows are sets)
+        if (sides[0][4][:, 0] != K.ORDER_NONE).any():
+            o_def = tt(sides[0][4].view(np.int16))[tt(sides[0][2])][:, of_pair[0]]
+            ord_d = torch.where(even, o_def, o_def.new_full((), _ORDER_NONE_I16)).contiguous()
         bl_def, bl_att = tt(sides[0][3])[of_pair[0]], tt(sides[1][3])[of_pair[1]]                # [P] code each side sets (255: none)
         nash = torch.full((P,), K.BASE_LINES["Nash"], dtype=torch.uint8, device=device)
         # base_line after the defender's turn / after the attacker's turn, in the steady state of the alternation
@@ -388,7 +424,8 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
                 cuts |= {t + 1 for t in fit_after}
             bounds = [0] + sorted(cuts) + [T]
             for t0, t1 in zip(bounds[:-1], bounds[1:]):
-                env.rollout(hdr_d[t0:t1], mask_d[t0:t1], bl_d[t0:t1], n_rollouts, lo, returns=ret, block_order=order)  # the mode of a turn is in its headers
+                env.rollout(hdr_d[t0:t1], mask_d[t0:t1], bl_d[t0:t1], n_rollouts, lo, returns=ret, block_order=order,
+                            order=None if ord_d is None else ord_d[t0:t1])  # the mode of a turn is in its headers
                 if t1 - 1 in fit_after:
                     env.fit_detectors(detector_fit_seeds(seed, g_of_env, t1 - 1))
         else:
@@ -411,8 +448,11 @@ def evaluate_payoff_matrix_batched(network, def_strategies, att_strategies, n_ro
                         h_k, m_k = decode_actions(raw_a, mode, n_types, M, X, n_app, W)
                         hdr_e[idx] = h_k
                         mask_e[idx] = m_k
+                order_e = None
+                if ord_d is not None and bool((ord_d[t, :, 0] != _ORDER_NONE_I16).any()):  # a defender turn with ordered rows
+                    order_e = _order_arrays(hdr_e, mask_e, ord_d[t][pair_of_env])
                 env.set_base_line_per_env(bl_d[t][pair_of_env])
-                raw, _, _ = env.step(ActionBatch(hdr_e, mask_e))
+                raw, _, _ = env.step(ActionBatch(hdr_e, mask_e, order_e))
                 ret[mode] += raw.double()
                 if n_slots and mode == 0 and t < T - 1:
                     env.fit_detectors(detector_fit_seeds(seed, g_of_env, t))

@@ -353,13 +353,18 @@ class VectorCyberDefenseEnv:
         K.check(self.L.cyg_block_envs(self.h, C.byref(nb)))
         return int(nb.value)
 
-    def rollout(self, hdr, mask, base_line, envs_per_row, row_base, returns=None, flags=0, block_order=None):
+    def rollout(self, hdr, mask, base_line, envs_per_row, row_base, returns=None, flags=0, block_order=None, order=None):
         """n_steps plain steps of every env in ONE launch from per-ROW action tables (cyg_rollout): hdr [T, R, 4],
         mask [T, R, W] int32, base_line [T, R] uint8 or None; slot b reads row (row_base + env_index_of_slot()[b]) // envs_per_row.
         `returns` [2, B] float64 accumulates the raw rewards of defender / attacker turns.  The loop body of
-        DoubleOracle.simulate_game (do_agent.py:1875-2089) for the strategies that need no observation."""
+        DoubleOracle.simulate_game (do_agent.py:1875-2089) for the strategies that need no observation.
+        order: optional [T, R, order_stride] int16 / uint16 device tensor (order_stride >= M), device_indices in list
+        order for the rows whose first entry is not ORDER_NONE (cyg_rollout_ordered); None: every row is a set."""
         T, R = int(hdr.shape[0]), int(hdr.shape[1])
         assert hdr.shape == (T, R, 4) and mask.shape == (T, R, self.W) and hdr.is_contiguous() and mask.is_contiguous()
+        if order is not None:
+            assert order.dim() == 3 and tuple(order.shape[:2]) == (T, R) and order.dtype in (torch.int16, torch.uint16)
+            assert order.device == hdr.device and order.is_contiguous()
         if returns is None:
             returns = torch.zeros(2, self.B, dtype=torch.float64, device=self.device)
         if base_line is not None:
@@ -370,8 +375,11 @@ class VectorCyberDefenseEnv:
             assert block_order.numel() == (self.B + self.block_envs() - 1) // self.block_envs()
         a = K.CygRolloutArgs(hdr.data_ptr(), mask.data_ptr(), None if base_line is None else base_line.data_ptr(), T, R,
                              int(row_base), int(envs_per_row), 0, returns.data_ptr(), None if block_order is None else block_order.data_ptr())
-        K.check(self.L.cyg_rollout(self.h, C.byref(a), flags, self._s()))
-        self._hold = (hdr, mask, base_line, returns, block_order)
+        if order is None:
+            K.check(self.L.cyg_rollout(self.h, C.byref(a), flags, self._s()))
+        else:
+            K.check(self.L.cyg_rollout_ordered(self.h, C.byref(a), order.data_ptr(), int(order.shape[2]), flags, self._s()))
+        self._hold = (hdr, mask, base_line, returns, block_order, order)
         return returns
 
     def set_env_id_stride(self, run, stride):

@@ -294,6 +294,22 @@ typedef struct cyg_rollout_args {
 int cyg_block_envs(cyg_handle h, int32_t* block_envs);
 int cyg_rollout(cyg_handle h, const cyg_rollout_args* a, uint32_t step_flags, void* stream);
 
+/* cyg_rollout with device_indices in a given ORDER: the sequences DoubleOracle draws with sample_action (do_agent.py:
+ * 1001-1013) list their devices in random.sample draw order (CyberDefenseEnv.py:565), and for defender types 1, 4, 5, 6,
+ * 9, 12 and 13 that order changes the result (the _stall draws are taken per listed device in list order; block /
+ * unblock pick one edge per listed device, each pick seeing the flips before it, volt:485-511).
+ * order[n_steps][n_rows][order_stride] (uint16) has the row layout of a->hdr.  A row whose first entry is
+ * CYG_ORDER_NONE is a set-form row and steps exactly as in cyg_rollout; any other row lists its n_dev devices in order
+ * in its first n_dev entries (as cyg_actions.order does for cyg_step; the mask still holds their set) and its env runs
+ * the action with one thread, as cyg_step does with an order array.  A header whose n_dev exceeds order_stride is read
+ * as order_stride: the kernel never reads past order_stride entries of a row.  Everything else -- base_line rows,
+ * returns, block_order, strided env ids, hop-log rings and detectors -- is as in cyg_rollout, and the result of every
+ * env is bit-identical to n_steps cyg_step() calls with the same order rows.  CYG_E_INVAL on a NULL order,
+ * order_stride < M, networks beyond 128 device slots and CYG_STEP_GROUPED. */
+#define CYG_ORDER_NONE 0xFFFFu
+int cyg_rollout_ordered(cyg_handle h, const cyg_rollout_args* a, const uint16_t* order, int32_t order_stride,
+                        uint32_t step_flags, void* stream);
+
 /* Which env a slot of the handle holds.  Default: slot s is env env_id0 + s.  With run > 0 (run divides B, stride >= run)
  * slot s is env env_id0 + (s / run) * stride + s % run: runs of `run` consecutive env ids, `stride` ids apart.  The payoff
  * evaluation numbers its envs (strategy pair, rollout) row-major; a rank that takes rollouts [r * run, (r + 1) * run) of

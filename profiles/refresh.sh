@@ -32,7 +32,7 @@ tail -1 gpurun_out/${R}_bench.json > profiles/${R}_bench_line.json
 cp gpurun_out/${R}_launches.csv profiles/${R}_launches.csv
 [ -f gpurun_out/${R}_exclude_sweep.txt ] && cp gpurun_out/${R}_exclude_sweep.txt profiles/${R}_exclude_sweep.txt
 # SASS evidence: bulk (TMA) copies + mbarrier waits in the step kernel, instruction count of the plain instantiation
-SASS=$(cuobjdump -sass -fun '_Z15cyg_step_kernelILi4ELb0ELb0EEv10StepParams' cygym_b200/libcygym_b200.so 2>/dev/null || true)
+SASS=$(cuobjdump -sass -fun '_Z15cyg_step_kernelILi4ELb0ELb0ELb0EEv10StepParams' cygym_b200/libcygym_b200.so 2>/dev/null || true)
 { echo "# cuobjdump -sass of cyg_step_kernel<4, no ROLL, no LOG> in cygym_b200/libcygym_b200.so (sm_100a)";
   echo "# SASS instructions: $(grep -cE '^\s+/\*[0-9a-f]{4,}\*/' <<< "$SASS")";
   echo "# bulk-copy / mbarrier / cluster instructions:"; grep -nE 'UBLKCP|UBLKPF|SYNCS|UTMA|FENCE|ELECT' <<< "$SASS" | sed 's/  */ /g' | head -40;
